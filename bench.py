@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- D8 flow direction + flow accumulation throughput on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--size S]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--size S] [--dump-outputs DIR]
 
 One step = one pass of the hot path (flow direction, then flow accumulation) over one synthetic
 float32 DEM.  N=1: the S x S raster (default 65536, BASELINE.json configs[2]) is resident in HBM
@@ -16,6 +16,10 @@ recurrence on every cell (across strip boundaries too), 64-bit position-weighted
 against the same rows of a single-GPU run of the whole raster (N>1), and oracle-checked direction windows
 that touch the strip boundaries.  `other_workloads` repeats step + checks on the flat-heavy and the
 adversarial long-path DEMs (BASELINE.json configs[3], configs[4]).
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step -- codes and counts at a fixed,
+seeded sample of cells (every cell of a small raster) -- so that two builds, or two GPU counts, can be compared output
+for output on identical inputs.
 """
 import argparse
 import json
@@ -37,6 +41,9 @@ HBM_NOMINAL_GBS = 8000.0   # nominal HBM3e bandwidth of a B200 (SURVEY 8d: repor
 PHASE_BYTES = {"direction": 5.0, "acc_tile_a": 1.0, "acc_tile_b": 8.0}
 KINDS = {0: "fractal value-noise", 1: "terraced fractal", 2: "tilted plane", 3: "walled serpentine (one channel, east-west runs)",
          4: "walled serpentine (one channel, north-south runs)"}
+# --dump-outputs: cells written per raster, 40 MB in all (codes float32, counts and cell indices float64), under 64 MB
+DUMP_CELLS = 1 << 21
+DUMP_SEED = 0
 
 
 def measured_hbm_peak():
@@ -98,6 +105,47 @@ class ClockSampler:
         s = sorted(self.samples)
         return {"sm_mhz": (s[len(s) // 2] if s else None), "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons),
                 "samples": len(s)}
+
+
+# ---------------------------------------------------------------- --dump-outputs
+def dump_cells(rows, cols):
+    """Row-major indices of the cells --dump-outputs writes, ascending: every cell of a raster of at most DUMP_CELLS
+    cells, else DUMP_CELLS distinct cells drawn with a fixed seed (the same for every run, build and GPU count)."""
+    import numpy as np
+
+    n = rows * cols
+    if n <= DUMP_CELLS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_CELLS, replace=False))
+
+
+def dump_outputs(out_dir, fdr, fac, row0, rows, cols, sum_ranks=None):
+    """Writes DIR/fdr.npy (codes, float32), DIR/fac.npy (counts, float64) and DIR/cells.npy (their row-major indices,
+    float64) for the cells dump_cells(rows, cols) names.  `fdr` / `fac` (numpy arrays or device tensors) hold rows
+    row0 .. row0 + len(fdr) of the raster; with several ranks each contributes zeros outside its rows, `sum_ranks`
+    adds the ranks' arrays and only the caller passing out_dir writes.  Both conversions are exact."""
+    import numpy as np
+
+    cells = dump_cells(rows, cols)
+    lo = row0 * cols
+    mine = (cells >= lo) & (cells < lo + fdr.shape[0] * cols)
+    r, c = np.divmod(cells[mine] - lo, cols)
+    if not isinstance(fdr, np.ndarray):  # gather on the device; only the sample is copied to the host
+        import torch
+
+        r, c = torch.from_numpy(r).to(fdr.device), torch.from_numpy(c).to(fdr.device)
+    out = {"fdr": np.zeros(len(cells), np.float32), "fac": np.zeros(len(cells), np.float64)}
+    for name, full in (("fdr", fdr), ("fac", fac)):
+        got = full[r, c]
+        out[name][mine] = got if isinstance(got, np.ndarray) else got.cpu().numpy()
+        if sum_ranks is not None:
+            out[name] = sum_ranks(out[name])
+    if out_dir is None:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    out["cells"] = cells.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 # ---------------------------------------------------------------- reference arm (CPU, no CUDA library in the process)
@@ -184,10 +232,12 @@ def run_reference(args):
     t0 = time.perf_counter()
     td = ta = 0.0
     for _ in range(args.steps):
-        _, _, a, b = cpu_pass(oracle, dem_pad, numba_dir)
+        fdr, fac, a, b = cpu_pass(oracle, dem_pad, numba_dir)
         td += a
         ta += b
     el = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, fdr, fac, 0, sample, sample)
     value = cells * args.steps / el / 1e9
     dir_how = ("the reference's own numba flow_direction_for_tile (oracle/_ref)" if numba_dir is not None
                else "C port (oracle/d8_oracle.c, OpenMP)")
@@ -461,6 +511,15 @@ def run_native(args):
     load(args.seed, args.kind, args.holes)
     ms_per_step, per_step, launches, clocks = timed(args.steps, args.warmup)
     value = cells_total / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs:  # before anything below overwrites the step's buffers
+
+        def sum_ranks(a):
+            t = torch.from_numpy(a).cuda()
+            dist.all_reduce(t, op=dist.ReduceOp.SUM)
+            return t.cpu().numpy()
+
+        dump_outputs(args.dump_outputs if rank == 0 else None, my_fdr(), my_fac(), r0, S, S,
+                     sum_ranks if world > 1 else None)
 
     # ---- roofline (live CUDA-event times from the timed region, this rank).  SURVEY 8(d) states the algorithmic
     #      bytes per stage: direction 5 B/cell, accumulation 9 B/cell (1 B code read + 8 B count write).  The
@@ -820,7 +879,12 @@ def main():
     ap.add_argument("--no-flats", action="store_true", help="skip the fix_flats / pit breaching legs (next_rows)")
     ap.add_argument("--no-numa", action="store_true", help="N > 1: do not bind the rank to its GPU's NUMA node")
     ap.add_argument("--no-numba", action="store_true", help="reference arm: C port for direction even if oracle/_ref exists")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the codes and counts of the last timed step (a fixed sample of cells of a large raster) "
+                         "as DIR/fdr.npy, DIR/fac.npy and their cell indices as DIR/cells.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     if args.impl == "reference":
         run_reference(args)
     else:
