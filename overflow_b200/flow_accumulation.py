@@ -141,29 +141,26 @@ def check_flow_accumulation(flow_direction: np.ndarray, flow_accumulation_raster
     return int(n_bad.value)
 
 
-def flow_accumulation(input_path, output_path, chunk_size=2000, streamed=True):
+def flow_accumulation(input_path, output_path, chunk_size=2000):
     """Flow-accumulation GeoTIFF from a flow-direction GeoTIFF.
 
     Absent from the reference snapshot (SURVEY.md fact 1); follows the house pattern of
     flow_direction() (flow_direction.py:99-124): band 1 in, 1-band Int64 GeoTIFF out with the
     same projection / geotransform and nodata FLOW_ACCUMULATION_NODATA.  The whole raster is
     accumulated on the device; `chunk_size` is the I/O granularity: the codes go up and the counts come down in
-    bands of rows while the files are read and written (streaming.py; `streamed=False`: read everything,
-    one library call, write everything).  NODATA cells hold -9998 in the output, as in the reference's array
+    bands of rows while the files are read and written (streaming.py; an empty raster is read whole, one library
+    call, written whole).  NODATA cells hold -9998 in the output, as in the reference's array
     result (SURVEY fact 2), although the band's nodata value is -9999: see INTEGRATION.md section 3.
     """
     from .util import raster as _raster
 
-    if streamed:
+    src = _raster.open_raster(input_path)
+    if src.RasterXSize * src.RasterYSize > 0:
         from .streaming import stream_accumulation
 
-        ds = _raster.open_raster(input_path)
-        empty = ds.RasterXSize * ds.RasterYSize == 0
-        ds = None
-        if not empty:
-            stream_accumulation(input_path, output_path, band_rows=chunk_size)
-            return
-    src = _raster.open_raster(input_path)
+        src = None
+        stream_accumulation(input_path, output_path, band_rows=chunk_size)
+        return
     band = src.GetRasterBand(1)
     fdr = _raster.read_band(band, chunk_size)
     fac = flow_accumulation_for_raster(fdr)

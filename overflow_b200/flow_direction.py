@@ -96,28 +96,26 @@ def flow_direction_for_raster(dem: np.ndarray, nodata_value: float, out: np.ndar
     return out
 
 
-def flow_direction(input_path, output_path, chunk_size=4000, streamed=None):
+def flow_direction(input_path, output_path, chunk_size=4000):
     """Generate a flow-direction GeoTIFF from a DEM file (reference flow_direction.py:99-124).
 
     Band 1 of `input_path` is read; the output is a 1-band Byte GeoTIFF with the same
     projection / geotransform and nodata 9.  `chunk_size` keeps its meaning as the I/O
     granularity; the result does not depend on it.  Float32 DEMs go through the band pipeline of
     streaming.py (file reads, PCIe copies, the stencil and file writes overlapped, rows streamed in bands of
-    chunk_size rows); `streamed=False` -- and every other band type -- takes the reference's own chunk loop,
-    one synchronous library call per chunk.
+    chunk_size rows); every other band type, which needs the generic stencil, and an empty raster take the
+    reference's own chunk loop, one synchronous library call per chunk.
     """
     from .util import raster as _raster
 
     src = _raster.open_raster(input_path)
     band = src.GetRasterBand(1)
     nodata_value = band.GetNoDataValue()
-    if streamed is None:
-        streamed = _raster.gdal_data_type_to_numpy_data_type(band.DataType) == np.float32 and band.XSize * band.YSize > 0
-    if streamed:
-        from .streaming import flow_direction_streamed
+    if _raster.gdal_data_type_to_numpy_data_type(band.DataType) == np.float32 and band.XSize * band.YSize > 0:
+        from .streaming import stream_routing
 
         src = band = None
-        flow_direction_streamed(input_path, output_path, band_rows=chunk_size)
+        stream_routing(input_path, output_path, None, band_rows=chunk_size)
         return
     dst = _raster.create_raster(
         output_path, src.RasterXSize, src.RasterYSize, "Byte",

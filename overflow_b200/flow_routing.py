@@ -57,7 +57,7 @@ def flow_routing_for_raster(dem: np.ndarray, nodata_value: float, out_fdr: np.nd
     return (out_fdr, out_fac, perim) if with_links else (out_fdr, out_fac)
 
 
-def flow_routing(input_path, flow_direction_path, flow_accumulation_path, chunk_size=2000, streamed=None):
+def flow_routing(input_path, flow_direction_path, flow_accumulation_path, chunk_size=2000):
     """DEM file -> flow-direction GeoTIFF and flow-accumulation GeoTIFF in one pass over the device.
 
     File-level counterpart of `flow_routing_for_raster`, in the pattern of the reference's
@@ -65,7 +65,8 @@ def flow_routing(input_path, flow_direction_path, flow_accumulation_path, chunk_
     Int64 raster (nodata FLOW_ACCUMULATION_NODATA) out, same projection / geotransform.  The outputs equal
     what `flow_direction()` followed by `flow_accumulation()` write; `chunk_size` is the I/O granularity: Float32
     DEMs move through the band pipeline of streaming.py in bands of chunk_size rows (reads, copies, kernels and
-    writes overlapped); `streamed=False` and other band types read the whole raster first.
+    writes overlapped); other band types, whose generic stencil the pipeline lacks, and empty rasters are read
+    whole first.
     """
     from .constants import FLOW_ACCUMULATION_NODATA, FLOW_DIRECTION_NODATA
     from .util import raster as _raster
@@ -74,13 +75,11 @@ def flow_routing(input_path, flow_direction_path, flow_accumulation_path, chunk_
     band = src.GetRasterBand(1)
     nodata_value = band.GetNoDataValue()
     assert nodata_value is not None, "the DEM band needs a nodata value (util/raster.py:59 in the reference)"
-    if streamed is None:
-        streamed = _raster.gdal_data_type_to_numpy_data_type(band.DataType) == np.float32 and band.XSize * band.YSize > 0
-    if streamed:
-        from .streaming import flow_routing_streamed
+    if _raster.gdal_data_type_to_numpy_data_type(band.DataType) == np.float32 and band.XSize * band.YSize > 0:
+        from .streaming import stream_routing
 
         src = band = None
-        return flow_routing_streamed(input_path, flow_direction_path, flow_accumulation_path, band_rows=chunk_size)
+        return stream_routing(input_path, flow_direction_path, flow_accumulation_path, band_rows=chunk_size)
     dem = _raster.read_band(band, chunk_size)
     fdr, fac = flow_routing_for_raster(dem, nodata_value)
     for path, name, nodata, arr in ((flow_direction_path, "Byte", FLOW_DIRECTION_NODATA, fdr),
