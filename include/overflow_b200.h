@@ -32,6 +32,8 @@
  *     buffers it owns and copies results back; OFL_MEM_DEVICE: pointers are CUDA device pointers)
  *   - `stream` is a cudaStream_t (NULL = the legacy default stream); device-pointer calls are
  *     asynchronous on it unless stated, host-pointer calls return after the results are in host memory
+ *   - a host-pointer call returns only after every copy it started has finished, whether it succeeds or
+ *     fails: on return the library no longer reads or writes the caller's host buffers
  *   - every function returns OFL_OK (0) or a negative ofl_status; ofl_last_error() gives the message
  *     for the calling thread
  *   - there is no CPU fallback: without a usable CUDA device every compute entry point fails

@@ -111,17 +111,21 @@ int pipe_events(int n) {
   return OFL_OK;
 }
 
-// Enqueues the whole banded pipeline; returns at the first error (the caller drains the streams).
-int direction_from_host_enqueue(const float* dem, int64_t in_rows, int64_t rows, int64_t cols, int64_t ld_dem,
-                                double nodata, int y_off, float* d_dem, int64_t ldd, uint8_t* d_fdr, int64_t ldo,
-                                uint8_t* fdr_host, int64_t ld_fdr, cudaStream_t st) {
+// dem: host, in_rows x cols.  d_dem / d_fdr: device staging (pitches ldd / ldo).  fdr_host may be null.
+// Output row y reads input rows y + y_off - 1 .. y + y_off + 1.  Enqueues the whole banded pipeline and returns
+// at the first error; finish_call drains the streams.
+int direction_from_host(const float* dem, int64_t in_rows, int64_t rows, int64_t cols, int64_t ld_dem, double nodata,
+                        int y_off, float* d_dem, int64_t ldd, uint8_t* d_fdr, int64_t ldo, uint8_t* fdr_host,
+                        int64_t ld_fdr, cudaStream_t st) {
+  int rc = pipe_streams();
+  if (rc != OFL_OK) return rc;
   int64_t band_bytes = PIPE_BAND_BYTES;
   if (const char* e = getenv("OFL_PIPE_BAND_BYTES")) band_bytes = atoll(e) > 0 ? atoll(e) : band_bytes;  // tests: many small bands
   int64_t band = band_bytes / (cols * (int64_t)sizeof(float));
   band = band < 64 ? 64 : band / 64 * 64;
   if ((in_rows + band - 1) / band > PIPE_MAX_BANDS) band = ((in_rows + PIPE_MAX_BANDS - 1) / PIPE_MAX_BANDS + 63) / 64 * 64;
   const int n_in = (int)((in_rows + band - 1) / band), n_out = (int)((rows + band - 1) / band);
-  int rc = pipe_events(n_in + n_out);
+  rc = pipe_events(n_in + n_out);
   if (rc != OFL_OK) return rc;
   cudaEvent_t* ev_up = g_pipe.pool;
   cudaEvent_t* ev_dir = g_pipe.pool + n_in;
@@ -150,22 +154,81 @@ int direction_from_host_enqueue(const float* dem, int64_t in_rows, int64_t rows,
   return OFL_OK;
 }
 
-// dem: host, in_rows x cols.  d_dem / d_fdr: device staging (pitches ldd / ldo).  fdr_host may be null.
-// Output row y reads input rows y + y_off - 1 .. y + y_off + 1.  With sync_downloads, or after any error, every
-// stream is idle on return: the caller's host buffers are never left in flight.
-int direction_from_host(const float* dem, int64_t in_rows, int64_t rows, int64_t cols, int64_t ld_dem, double nodata,
-                        int y_off, float* d_dem, int64_t ldd, uint8_t* d_fdr, int64_t ldo, uint8_t* fdr_host,
-                        int64_t ld_fdr, cudaStream_t st, bool sync_downloads) {
-  int rc = pipe_streams();
-  if (rc != OFL_OK) return rc;
-  rc = direction_from_host_enqueue(dem, in_rows, rows, cols, ld_dem, nodata, y_off, d_dem, ldd, d_fdr, ldo, fdr_host,
-                                   ld_fdr, st);
-  if (rc != OFL_OK || sync_downloads) {
-    cudaStreamSynchronize(g_pipe.h2d);
-    cudaStreamSynchronize(st);
-    cudaStreamSynchronize(g_pipe.d2h);
+// ---------------------------------------------------------------- staging of host-memory calls
+// Every entry point runs one body against device pointers.  Under OFL_MEM_DEVICE those are the caller's; under
+// OFL_MEM_HOST stage_in gives argument i scratch slot SCRATCH_STAGE0 + i and uploads it, and finish_call downloads
+// the results and returns only once nothing the call started is still copying, whether it succeeded or not.
+// Calls list their rasters widest element first, then their vectors, so that different calls share slots of
+// like size.
+enum { COPY_NONE = 0, COPY_IN = 1, COPY_OUT = 2 };
+
+struct CallArg {                      // one raster or vector (one row) argument of a call
+  const void* caller;                 // the caller's buffer; a host argument may be null (staging only)
+  int64_t rows, row_bytes, pitch;     // its layout in bytes
+  int copy;                           // what a host call moves between `caller` and its slot (COPY_*)
+  int64_t align;                      // a slot row is row_bytes rounded up to this; 1: packed rows, copied in one piece
+  void* dev;                          // set by stage_in: what the body reads and writes
+  int64_t dev_pitch;
+  template <class T> T* d() const { return static_cast<T*>(dev); }
+  int64_t ld(int64_t elem_bytes) const { return dev_pitch / elem_bytes; }
+};
+
+// A pitched raster goes as a 2-D copy even when its rows happen to be contiguous: on a B200 (1000 W), one
+// cudaMemcpyAsync of the 34 GB counts of a 65536^2 raster took ~2 ms longer than the 2-D copy.
+cudaError_t copy_rows(bool packed, void* dst, int64_t dpitch, const void* src, int64_t spitch, int64_t width,
+                      int64_t rows, cudaMemcpyKind kind, cudaStream_t st) {
+  if (packed) return cudaMemcpyAsync(dst, src, (size_t)(width * rows), kind, st);
+  return cudaMemcpy2DAsync(dst, dpitch, src, spitch, width, rows, kind, st);
+}
+
+template <int N>
+int stage_in(CallArg (&a)[N], int mem_kind, cudaStream_t st) {
+  static_assert(N <= SCRATCH_STAGE_SLOTS, "more arguments than staging slots");
+  for (int i = 0; i < N; ++i) {
+    CallArg& x = a[i];
+    if (mem_kind == OFL_MEM_DEVICE) {
+      x.dev = const_cast<void*>(x.caller);
+      x.dev_pitch = x.pitch;
+      continue;
+    }
+    x.dev_pitch = round_up(x.row_bytes, x.align);
+    int rc = scratch_get(SCRATCH_STAGE0 + i, (size_t)(x.rows * x.dev_pitch), &x.dev);
+    if (rc != OFL_OK) return rc;
+    if ((x.copy & COPY_IN) && x.caller && x.rows * x.row_bytes > 0)
+      OFL_CUDA(copy_rows(x.align == 1, x.dev, x.dev_pitch, x.caller, x.pitch, x.row_bytes, x.rows,
+                         cudaMemcpyHostToDevice, st));
   }
+  return OFL_OK;
+}
+
+// Host calls: after a successful body, download every COPY_OUT argument; then, in every case, wait for `st` and
+// the band pipeline.  Returns rc, or the first copy error if rc was OFL_OK.  Device calls: returns rc.
+template <int N>
+int finish_call(int rc, const CallArg (&a)[N], int mem_kind, cudaStream_t st) {
+  if (mem_kind == OFL_MEM_DEVICE) return rc;
+  cudaError_t e = cudaSuccess;
+  for (int i = 0; i < N && rc == OFL_OK && e == cudaSuccess; ++i) {
+    const CallArg& x = a[i];
+    if ((x.copy & COPY_OUT) && x.caller && x.rows * x.row_bytes > 0)
+      e = copy_rows(x.align == 1, const_cast<void*>(x.caller), x.pitch, x.dev, x.dev_pitch, x.row_bytes, x.rows,
+                    cudaMemcpyDeviceToHost, st);
+  }
+  cudaStream_t streams[3] = {st, g_pipe.h2d, g_pipe.d2h};  // the pipeline's exist once a call has used it
+  for (int i = 0; i < (g_pipe.h2d ? 3 : 1); ++i) {
+    const cudaError_t s = cudaStreamSynchronize(streams[i]);
+    if (e == cudaSuccess) e = s;
+  }
+  if (rc == OFL_OK && e != cudaSuccess) rc = cuda_fail(e, "host staging copy", __FILE__, __LINE__);
   return rc;
+}
+
+// Reads a device counter back; returns once it is in *out.
+int read_counter(int64_t* out, const void* d_cnt, cudaStream_t st) {
+  unsigned long long h = 0;
+  OFL_CUDA(cudaMemcpyAsync(&h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
+  OFL_CUDA(cudaStreamSynchronize(st));
+  *out = (int64_t)h;
+  return OFL_OK;
 }
 }  // namespace
 
@@ -196,36 +259,18 @@ int ofl_flow_direction_f32(const float* dem, int64_t rows, int64_t cols, int64_t
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int y_off = (mode == OFL_DIR_MODE_STRIP) ? 1 : 0;
   const int64_t in_rows = rows + 2 * y_off;
-
-  if (mem_kind == OFL_MEM_DEVICE) {
-    rc = launch_direction(dem, in_rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, y_off, st);
-    if (rc != OFL_OK) return rc;
-    if (mode == OFL_DIR_MODE_TILE) return launch_fill_border(fdr, rows, cols, ld_fdr, OFL_DIR_NODATA, st);
-    return OFL_OK;
-  }
-
-  // host rasters: pitched device staging, one H2D, kernel, one D2H
-  const int64_t ldd = round_up(cols, 4), ldo = round_up(cols, 16);
-  void *d_dem = nullptr, *d_fdr = nullptr;
-  rc = scratch_get(SCRATCH_DEM, (size_t)in_rows * ldd * sizeof(float), &d_dem);
-  if (rc != OFL_OK) return rc;
-  rc = scratch_get(SCRATCH_FDR, (size_t)rows * ldo, &d_fdr);
-  if (rc != OFL_OK) return rc;
-  if (mode != OFL_DIR_MODE_TILE)  // the ring fill of TILE mode follows the kernel: tiles take the plain path below
-    return direction_from_host(dem, in_rows, rows, cols, ld_dem, nodata, y_off, static_cast<float*>(d_dem), ldd,
-                               static_cast<uint8_t*>(d_fdr), ldo, fdr, ld_fdr, st, true);
-  OFL_CUDA(cudaMemcpy2DAsync(d_dem, ldd * sizeof(float), dem, ld_dem * sizeof(float), cols * sizeof(float), in_rows,
-                             cudaMemcpyHostToDevice, st));
-  rc = launch_direction(static_cast<const float*>(d_dem), in_rows, cols, ldd, nodata, static_cast<uint8_t*>(d_fdr),
-                        rows, ldo, y_off, st);
-  if (rc != OFL_OK) return rc;
-  if (mode == OFL_DIR_MODE_TILE) {
-    rc = launch_fill_border(static_cast<uint8_t*>(d_fdr), rows, cols, ldo, OFL_DIR_NODATA, st);
-    if (rc != OFL_OK) return rc;
-  }
-  OFL_CUDA(cudaMemcpy2DAsync(fdr, ld_fdr, d_fdr, ldo, cols, rows, cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  const bool tile = mode == OFL_DIR_MODE_TILE;
+  // host: the DEM goes up in bands; the codes come back band by band, or in TILE mode in one copy after the ring fill
+  CallArg a[] = {{dem, in_rows, cols * 4, ld_dem * 4, COPY_NONE, 16},
+                 {fdr, rows, cols, ld_fdr, tile ? COPY_OUT : COPY_NONE, 16}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = mem_kind == OFL_MEM_HOST
+             ? direction_from_host(dem, in_rows, rows, cols, ld_dem, nodata, y_off, a[0].d<float>(), a[0].ld(4),
+                                   a[1].d<uint8_t>(), a[1].ld(1), tile ? nullptr : fdr, ld_fdr, st)
+             : launch_direction(dem, in_rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, y_off, st);
+  if (rc == OFL_OK && tile) rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_flow_direction_x64(const void* dem, int elem_kind, int64_t rows, int64_t cols, int64_t ld_dem, double nodata,
@@ -244,32 +289,14 @@ int ofl_flow_direction_x64(const void* dem, int elem_kind, int64_t rows, int64_t
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int y_off = (mode == OFL_DIR_MODE_STRIP) ? 1 : 0;
   const int64_t in_rows = rows + 2 * y_off;
-  const void* d_in = dem;
-  uint8_t* d_out = fdr;
-  int64_t ldd = ld_dem, ldo = ld_fdr;
-  if (mem_kind == OFL_MEM_HOST) {
-    void *b0 = nullptr, *b1 = nullptr;
-    ldd = cols;
-    ldo = round_up(cols, 16);
-    rc = scratch_get(SCRATCH_DEM, (size_t)in_rows * ldd * 8, &b0);
-    if (rc != OFL_OK) return rc;
-    rc = scratch_get(SCRATCH_FDR, (size_t)rows * ldo, &b1);
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaMemcpy2DAsync(b0, ldd * 8, dem, ld_dem * 8, cols * 8, in_rows, cudaMemcpyHostToDevice, st));
-    d_in = b0;
-    d_out = static_cast<uint8_t*>(b1);
-  }
-  rc = launch_direction_generic(d_in, elem_kind, in_rows, cols, ldd, nodata, d_out, rows, ldo, y_off, st);
-  if (rc != OFL_OK) return rc;
-  if (mode == OFL_DIR_MODE_TILE) {
-    rc = launch_fill_border(d_out, rows, cols, ldo, OFL_DIR_NODATA, st);
-    if (rc != OFL_OK) return rc;
-  }
-  if (mem_kind == OFL_MEM_HOST) {
-    OFL_CUDA(cudaMemcpy2DAsync(fdr, ld_fdr, d_out, ldo, cols, rows, cudaMemcpyDeviceToHost, st));
-    OFL_CUDA(cudaStreamSynchronize(st));
-  }
-  return OFL_OK;
+  CallArg a[] = {{dem, in_rows, cols * 8, ld_dem * 8, COPY_IN, 8}, {fdr, rows, cols, ld_fdr, COPY_OUT, 16}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_direction_generic(a[0].dev, elem_kind, in_rows, cols, a[0].ld(8), nodata, a[1].d<uint8_t>(), rows,
+                                  a[1].ld(1), y_off, st);
+  if (rc == OFL_OK && mode == OFL_DIR_MODE_TILE)
+    rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_fill_border_u8(uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int value, void* stream) {
@@ -297,38 +324,17 @@ static int accumulation_entry(const uint8_t* fdr, int64_t rows, int64_t cols, in
     if (rc != OFL_OK) return rc;
     workspace_bytes = need;
   }
-  if (mem_kind == OFL_MEM_DEVICE)
-    return launch_accumulation(fdr, rows, cols, ld_fdr, reinterpret_cast<long long*>(fac), ld_fac,
-                               reinterpret_cast<long long*>(perim_links), workspace, workspace_bytes, st, false, false,
-                               reinterpret_cast<const long long*>(perim_inflow));
-
-  const int64_t ldi = round_up(cols, 16), ldo = round_up(cols, 2);
-  void *d_fdr = nullptr, *d_fac = nullptr, *d_links = nullptr;
-  rc = scratch_get(SCRATCH_FDR, (size_t)rows * ldi, &d_fdr);
-  if (rc != OFL_OK) return rc;
-  rc = scratch_get(SCRATCH_FAC, (size_t)rows * ldo * sizeof(int64_t), &d_fac);
-  if (rc != OFL_OK) return rc;
   const int64_t n_perim = perimeter_count(rows, cols);
-  if (perim_links || perim_inflow) {  // links [n][2], then the inflow [n]
-    rc = scratch_get(SCRATCH_LINKS, (size_t)n_perim * 3 * sizeof(int64_t), &d_links);
-    if (rc != OFL_OK) return rc;
-  }
-  long long* d_inflow = nullptr;
-  if (perim_inflow) {
-    d_inflow = static_cast<long long*>(d_links) + 2 * n_perim;
-    OFL_CUDA(cudaMemcpyAsync(d_inflow, perim_inflow, (size_t)n_perim * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-  }
-  OFL_CUDA(cudaMemcpy2DAsync(d_fdr, ldi, fdr, ld_fdr, cols, rows, cudaMemcpyHostToDevice, st));
-  rc = launch_accumulation(static_cast<const uint8_t*>(d_fdr), rows, cols, ldi, static_cast<long long*>(d_fac), ldo,
-                           perim_links ? static_cast<long long*>(d_links) : nullptr, workspace, workspace_bytes, st, false,
-                           false, d_inflow);
-  if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpy2DAsync(fac, ld_fac * sizeof(int64_t), d_fac, ldo * sizeof(int64_t), cols * sizeof(int64_t), rows,
-                             cudaMemcpyDeviceToHost, st));
-  if (perim_links)
-    OFL_CUDA(cudaMemcpyAsync(perim_links, d_links, (size_t)n_perim * 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_OUT, 16},
+                 {fdr, rows, cols, ld_fdr, COPY_IN, 16},
+                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1},
+                 {perim_inflow, 1, n_perim * 8, n_perim * 8, COPY_IN, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_accumulation(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<long long>(), a[0].ld(8),
+                             perim_links ? a[2].d<long long>() : nullptr, workspace, workspace_bytes, st, false, false,
+                             perim_inflow ? a[3].d<const long long>() : nullptr);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_flow_accumulation_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int64_t* fac,
@@ -376,35 +382,20 @@ int ofl_flow_routing_f32(const float* dem, int64_t rows, int64_t cols, int64_t l
     return launch_accumulation(fdr, rows, cols, ld_fdr, reinterpret_cast<long long*>(fac), ld_fac,
                                reinterpret_cast<long long*>(perim_links), work, need, st, true, true);
   }
-  const int64_t ldd = round_up(cols, 4), ldi = round_up(cols, 16), ldo = round_up(cols, 2);
-  void *d_dem = nullptr, *d_fdr = nullptr, *d_fac = nullptr, *d_links = nullptr;
-  rc = scratch_get(SCRATCH_DEM, (size_t)rows * ldd * sizeof(float), &d_dem);
-  if (rc != OFL_OK) return rc;
-  rc = scratch_get(SCRATCH_FDR, (size_t)rows * ldi, &d_fdr);
-  if (rc != OFL_OK) return rc;
-  rc = scratch_get(SCRATCH_FAC, (size_t)rows * ldo * sizeof(int64_t), &d_fac);
-  if (rc != OFL_OK) return rc;
+  // the DEM goes up and the codes come back in bands, overlapping; the counts follow the accumulation
   const int64_t n_perim = perimeter_count(rows, cols);
-  if (perim_links) {
-    rc = scratch_get(SCRATCH_LINKS, (size_t)n_perim * 2 * sizeof(int64_t), &d_links);
-    if (rc != OFL_OK) return rc;
-  }
-  // codes stream back to the host while later bands are still uploading; the counts follow the accumulation
-  rc = direction_from_host(dem, rows, rows, cols, ld_dem, nodata, 0, static_cast<float*>(d_dem), ldd,
-                           static_cast<uint8_t*>(d_fdr), ldi, fdr, ld_fdr, st, false);
-  if (rc != OFL_OK) return rc;
-  rc = launch_accumulation(static_cast<const uint8_t*>(d_fdr), rows, cols, ldi, static_cast<long long*>(d_fac), ldo,
-                           static_cast<long long*>(d_links), work, need, st, false, true);
-  if (rc == OFL_OK) {
-    cudaError_t e = cudaMemcpy2DAsync(fac, ld_fac * sizeof(int64_t), d_fac, ldo * sizeof(int64_t), cols * sizeof(int64_t),
-                                      rows, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess && perim_links)
-      e = cudaMemcpyAsync(perim_links, d_links, (size_t)n_perim * 2 * sizeof(int64_t), cudaMemcpyDeviceToHost, st);
-    if (e != cudaSuccess) rc = cuda_fail(e, "cudaMemcpyAsync(fac)", __FILE__, __LINE__);
-  }
-  cudaStreamSynchronize(st);
-  cudaStreamSynchronize(g_pipe.d2h);
-  return rc;
+  CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_OUT, 16},
+                 {dem, rows, cols * 4, ld_dem * 4, COPY_NONE, 16},
+                 {fdr, rows, cols, ld_fdr, COPY_NONE, 16},
+                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = direction_from_host(dem, rows, rows, cols, ld_dem, nodata, 0, a[1].d<float>(), a[1].ld(4), a[2].d<uint8_t>(),
+                             a[2].ld(1), fdr, ld_fdr, st);
+  if (rc == OFL_OK)
+    rc = launch_accumulation(a[2].d<const uint8_t>(), rows, cols, a[2].ld(1), a[0].d<long long>(), a[0].ld(8),
+                             perim_links ? a[3].d<long long>() : nullptr, work, need, st, false, true);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_check_accumulation_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* fac,
@@ -420,30 +411,13 @@ int ofl_check_accumulation_u8(const uint8_t* fdr, int64_t rows, int64_t cols, in
   void* d_cnt = nullptr;
   rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
   if (rc != OFL_OK) return rc;
-  const uint8_t* dfdr = fdr;
-  const long long* dfac = reinterpret_cast<const long long*>(fac);
-  int64_t ldi = ld_fdr, ldo = ld_fac;
-  if (mem_kind == OFL_MEM_HOST) {
-    void *b0 = nullptr, *b1 = nullptr;
-    ldi = round_up(cols, 16);
-    ldo = cols;
-    rc = scratch_get(SCRATCH_FDR, (size_t)rows * ldi, &b0);
-    if (rc != OFL_OK) return rc;
-    rc = scratch_get(SCRATCH_FAC, (size_t)rows * ldo * sizeof(int64_t), &b1);
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaMemcpy2DAsync(b0, ldi, fdr, ld_fdr, cols, rows, cudaMemcpyHostToDevice, st));
-    OFL_CUDA(cudaMemcpy2DAsync(b1, ldo * sizeof(int64_t), fac, ld_fac * sizeof(int64_t), cols * sizeof(int64_t), rows,
-                               cudaMemcpyHostToDevice, st));
-    dfdr = static_cast<const uint8_t*>(b0);
-    dfac = static_cast<const long long*>(b1);
-  }
-  rc = launch_check(dfdr, rows, cols, ldi, dfac, ldo, static_cast<unsigned long long*>(d_cnt), st);
-  if (rc != OFL_OK) return rc;
-  unsigned long long h = 0;
-  OFL_CUDA(cudaMemcpyAsync(&h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  *n_bad = (int64_t)h;
-  return OFL_OK;
+  CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_IN, 8}, {fdr, rows, cols, ld_fdr, COPY_IN, 16}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_check(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<const long long>(), a[0].ld(8),
+                      static_cast<unsigned long long*>(d_cnt), st);
+  if (rc == OFL_OK) rc = read_counter(n_bad, d_cnt, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_strip_check_accumulation_u8(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr,
@@ -463,11 +437,7 @@ int ofl_strip_check_accumulation_u8(const uint8_t* fdr_halo, int64_t rows, int64
                     static_cast<unsigned long long*>(d_cnt), st, 1, reinterpret_cast<const long long*>(fac_above),
                     reinterpret_cast<const long long*>(fac_below));
   if (rc != OFL_OK) return rc;
-  unsigned long long h = 0;
-  OFL_CUDA(cudaMemcpyAsync(&h, d_cnt, sizeof(h), cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  *n_bad = (int64_t)h;
-  return OFL_OK;
+  return read_counter(n_bad, d_cnt, st);
 }
 
 // ---------------------------------------------------------------- flat resolution (csrc/flats.cu)
@@ -482,8 +452,7 @@ size_t ofl_flats_workspace_bytes(int64_t rows, int64_t cols) {
   OFL_REQUIRE(__VA_ARGS__, OFL_ERR_INVALID, "null raster pointer");                                                    \
   int rc = ensure_init();                                                                                              \
   if (rc != OFL_OK) return rc;                                                                                         \
-  cudaStream_t st = static_cast<cudaStream_t>(stream);                                                                 \
-  const size_t n = (size_t)rows * (size_t)cols
+  cudaStream_t st = static_cast<cudaStream_t>(stream)
 
 int ofl_flat_edges_f32(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, uint8_t* edges, int64_t* n_low,
                        int64_t* n_high, int mem_kind, void* stream) {
@@ -493,58 +462,37 @@ int ofl_flat_edges_f32(const float* dem, const uint8_t* fdr, int64_t rows, int64
   void* d_cnt = nullptr;
   rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
   if (rc != OFL_OK) return rc;
-  if (mem_kind == OFL_MEM_DEVICE)
-    return launch_flat_edges(dem, fdr, rows, cols, edges, n_low, n_high, static_cast<unsigned*>(d_cnt), st);
-  void *d_dem = nullptr, *d_fdr = nullptr, *d_edges = nullptr;
-  if ((rc = scratch_get(SCRATCH_DEM, n * sizeof(float), &d_dem)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FDR, n, &d_fdr)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_LINKS, n, &d_edges)) != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(d_dem, dem, n * sizeof(float), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_fdr, fdr, n, cudaMemcpyHostToDevice, st));
-  rc = launch_flat_edges(static_cast<float*>(d_dem), static_cast<uint8_t*>(d_fdr), rows, cols,
-                         static_cast<uint8_t*>(d_edges), n_low, n_high, static_cast<unsigned*>(d_cnt), st);
-  if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(edges, d_edges, n, cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{dem, rows, cols * 4, cols * 4, COPY_IN, 1},
+                 {fdr, rows, cols, cols, COPY_IN, 1},
+                 {edges, rows, cols, cols, COPY_OUT, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_flat_edges(a[0].d<const float>(), a[1].d<const uint8_t>(), rows, cols, a[2].d<uint8_t>(), n_low,
+                           n_high, static_cast<unsigned*>(d_cnt), st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
-// resolve (+ optionally rewrite the codes): shared by ofl_resolve_flats_f32 and ofl_fix_flats_f32
-static int flats_run(const float* dem, const uint8_t* fdr_in, uint8_t* fdr_out, int64_t rows, int64_t cols,
-                     int32_t* flat_mask, int32_t* labels, int64_t* info, void* workspace, size_t workspace_bytes,
-                     int mem_kind, cudaStream_t st) {
-  const size_t n = (size_t)rows * (size_t)cols;
+// resolve (+ with `fix`, rewrite the codes in place): shared by ofl_resolve_flats_f32 and ofl_fix_flats_f32
+static int flats_run(const float* dem, const uint8_t* fdr, bool fix, int64_t rows, int64_t cols, int32_t* flat_mask,
+                     int32_t* labels, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
+                     cudaStream_t st) {
+  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || (flat_mask && labels), OFL_ERR_INVALID,
+              "device callers provide flat_mask and labels");
   int rc;
   if (!workspace) {
     workspace_bytes = flats_workspace_bytes(rows, cols);
     if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
   }
-  if (mem_kind == OFL_MEM_DEVICE) {
-    OFL_REQUIRE(flat_mask && labels, OFL_ERR_INVALID, "device callers provide flat_mask and labels");
-    rc = launch_resolve_flats(dem, fdr_in, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, st);
-    if (rc == OFL_OK && fdr_out) rc = launch_masked_flow_dirs(flat_mask, labels, fdr_out, rows, cols, st);
-    return rc;
-  }
-  void *d_dem = nullptr, *d_fdr = nullptr, *d_out = nullptr;
-  if ((rc = scratch_get(SCRATCH_DEM, n * sizeof(float), &d_dem)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FDR, n, &d_fdr)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FAC, 2 * n * sizeof(int32_t), &d_out)) != OFL_OK) return rc;
-  int32_t* d_mask = static_cast<int32_t*>(d_out);
-  int32_t* d_labels = d_mask + n;
-  OFL_CUDA(cudaMemcpyAsync(d_dem, dem, n * sizeof(float), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_fdr, fdr_in, n, cudaMemcpyHostToDevice, st));
-  rc = launch_resolve_flats(static_cast<float*>(d_dem), static_cast<uint8_t*>(d_fdr), rows, cols, d_mask, d_labels, info,
-                            workspace, workspace_bytes, st);
-  if (rc != OFL_OK) return rc;
-  if (fdr_out) {
-    rc = launch_masked_flow_dirs(d_mask, d_labels, static_cast<uint8_t*>(d_fdr), rows, cols, st);
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaMemcpyAsync(fdr_out, d_fdr, n, cudaMemcpyDeviceToHost, st));
-  }
-  if (flat_mask) OFL_CUDA(cudaMemcpyAsync(flat_mask, d_mask, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  if (labels) OFL_CUDA(cudaMemcpyAsync(labels, d_labels, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{dem, rows, cols * 4, cols * 4, COPY_IN, 1},
+                 {flat_mask, rows, cols * 4, cols * 4, COPY_OUT, 1},
+                 {labels, rows, cols * 4, cols * 4, COPY_OUT, 1},
+                 {fdr, rows, cols, cols, fix ? COPY_IN | COPY_OUT : COPY_IN, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_resolve_flats(a[0].d<const float>(), a[3].d<const uint8_t>(), rows, cols, a[1].d<int>(), a[2].d<int>(),
+                              info, workspace, workspace_bytes, st);
+  if (rc == OFL_OK && fix) rc = launch_masked_flow_dirs(a[1].d<int>(), a[2].d<int>(), a[3].d<uint8_t>(), rows, cols, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_resolve_flats_f32(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, int32_t* flat_mask,
@@ -552,70 +500,48 @@ int ofl_resolve_flats_f32(const float* dem, const uint8_t* fdr, int64_t rows, in
                           void* stream) {
   if (info) for (int k = 0; k < 5; ++k) info[k] = 0;
   OFL_FLATS_COMMON(dem && fdr && flat_mask && labels);
-  (void)n;
-  return flats_run(dem, fdr, nullptr, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
+  return flats_run(dem, fdr, false, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
 }
 
 int ofl_fix_flats_f32(const float* dem, uint8_t* fdr, int64_t rows, int64_t cols, int32_t* flat_mask, int32_t* labels,
                       int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind, void* stream) {
   if (info) for (int k = 0; k < 5; ++k) info[k] = 0;
   OFL_FLATS_COMMON(dem && fdr);
-  (void)n;
-  return flats_run(dem, fdr, fdr, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
+  return flats_run(dem, fdr, true, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
 }
 
 int ofl_d8_masked_flow_dirs_i32(const int32_t* flat_mask, const int32_t* labels, uint8_t* fdr, int64_t rows, int64_t cols,
                                 int mem_kind, void* stream) {
   OFL_FLATS_COMMON(flat_mask && labels && fdr);
-  if (mem_kind == OFL_MEM_DEVICE) return launch_masked_flow_dirs(flat_mask, labels, fdr, rows, cols, st);
-  void *d_fdr = nullptr, *d_in = nullptr;
-  if ((rc = scratch_get(SCRATCH_FDR, n, &d_fdr)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FAC, 2 * n * sizeof(int32_t), &d_in)) != OFL_OK) return rc;
-  int32_t* d_mask = static_cast<int32_t*>(d_in);
-  int32_t* d_labels = d_mask + n;
-  OFL_CUDA(cudaMemcpyAsync(d_mask, flat_mask, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_labels, labels, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_fdr, fdr, n, cudaMemcpyHostToDevice, st));
-  rc = launch_masked_flow_dirs(d_mask, d_labels, static_cast<uint8_t*>(d_fdr), rows, cols, st);
-  if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(fdr, d_fdr, n, cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{flat_mask, rows, cols * 4, cols * 4, COPY_IN, 1},
+                 {labels, rows, cols * 4, cols * 4, COPY_IN, 1},
+                 {fdr, rows, cols, cols, COPY_IN | COPY_OUT, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK) rc = launch_masked_flow_dirs(a[0].d<const int>(), a[1].d<const int>(), a[2].d<uint8_t>(), rows, cols, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_flat_gradient_i32(const int32_t* labels, const uint8_t* fdr, int64_t rows, int64_t cols, const int32_t* seeds,
                           int64_t n_seeds, int towards, int32_t* flat_mask, int32_t* flat_height, int64_t n_heights,
                           void* workspace, size_t workspace_bytes, int mem_kind, void* stream) {
   OFL_FLATS_COMMON(labels && fdr && flat_mask && (seeds || n_seeds == 0) && (flat_height || n_heights == 0));
-  OFL_REQUIRE(n_seeds >= 0 && n_heights >= 0 && (size_t)n_seeds <= n && (size_t)n_heights <= n, OFL_ERR_INVALID,
+  const int64_t n = rows * cols;
+  OFL_REQUIRE(n_seeds >= 0 && n_heights >= 0 && n_seeds <= n && n_heights <= n, OFL_ERR_INVALID,
               "seed / flat_height count out of range");
   if (!workspace) {
     workspace_bytes = flats_workspace_bytes(rows, cols);
     if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
   }
-  if (mem_kind == OFL_MEM_DEVICE)
-    return launch_flat_gradient(labels, fdr, rows, cols, seeds, n_seeds, towards, flat_mask, flat_height, n_heights,
-                                workspace, workspace_bytes, st);
-  void *d_fdr = nullptr, *d_io = nullptr, *d_small = nullptr;
-  if ((rc = scratch_get(SCRATCH_FDR, n, &d_fdr)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FAC, 2 * n * sizeof(int32_t), &d_io)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_LINKS, (size_t)(n_seeds + n_heights + 2) * sizeof(int32_t), &d_small)) != OFL_OK) return rc;
-  int32_t* d_mask = static_cast<int32_t*>(d_io);
-  int32_t* d_labels = d_mask + n;
-  int32_t* d_seeds = static_cast<int32_t*>(d_small);
-  int32_t* d_fh = d_seeds + n_seeds;
-  OFL_CUDA(cudaMemcpyAsync(d_mask, flat_mask, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_labels, labels, n * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  OFL_CUDA(cudaMemcpyAsync(d_fdr, fdr, n, cudaMemcpyHostToDevice, st));
-  if (n_seeds) OFL_CUDA(cudaMemcpyAsync(d_seeds, seeds, (size_t)n_seeds * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  if (n_heights) OFL_CUDA(cudaMemcpyAsync(d_fh, flat_height, (size_t)n_heights * sizeof(int32_t), cudaMemcpyHostToDevice, st));
-  rc = launch_flat_gradient(d_labels, static_cast<uint8_t*>(d_fdr), rows, cols, d_seeds, n_seeds, towards, d_mask, d_fh,
-                            n_heights, workspace, workspace_bytes, st);
-  if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(flat_mask, d_mask, n * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  if (n_heights) OFL_CUDA(cudaMemcpyAsync(flat_height, d_fh, (size_t)n_heights * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{labels, rows, cols * 4, cols * 4, COPY_IN, 1},
+                 {flat_mask, rows, cols * 4, cols * 4, COPY_IN | COPY_OUT, 1},
+                 {fdr, rows, cols, cols, COPY_IN, 1},
+                 {seeds, 1, n_seeds * 4, n_seeds * 4, COPY_IN, 1},
+                 {flat_height, 1, n_heights * 4, n_heights * 4, COPY_IN | COPY_OUT, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_flat_gradient(a[0].d<const int>(), a[2].d<const uint8_t>(), rows, cols, a[3].d<const int>(), n_seeds,
+                              towards, a[1].d<int>(), a[4].d<int>(), n_heights, workspace, workspace_bytes, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 // ---------------------------------------------------------------- single-cell pit breaching (csrc/pits.cu)
@@ -633,21 +559,13 @@ int ofl_breach_single_cell_pits_f32(float* chunk, int64_t rows, int64_t cols, in
     workspace_bytes = pits_workspace_bytes(rows, cols);
     if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
   }
-  if (mem_kind == OFL_MEM_DEVICE)
-    return launch_breach_pits(chunk, rows, cols, ld_chunk, nodata, unsolved, info, workspace, workspace_bytes, st);
-  void *d_chunk = nullptr, *d_uns = nullptr;
-  if ((rc = scratch_get(SCRATCH_DEM, n * sizeof(float), &d_chunk)) != OFL_OK) return rc;
-  if ((rc = scratch_get(SCRATCH_FDR, n, &d_uns)) != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpy2DAsync(d_chunk, cols * sizeof(float), chunk, ld_chunk * sizeof(float), cols * sizeof(float), rows,
-                             cudaMemcpyHostToDevice, st));
-  rc = launch_breach_pits(static_cast<float*>(d_chunk), rows, cols, cols, nodata, static_cast<int8_t*>(d_uns), info,
-                          workspace, workspace_bytes, st);
-  if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpy2DAsync(chunk, ld_chunk * sizeof(float), d_chunk, cols * sizeof(float), cols * sizeof(float), rows,
-                             cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaMemcpyAsync(unsolved, d_uns, n, cudaMemcpyDeviceToHost, st));
-  OFL_CUDA(cudaStreamSynchronize(st));
-  return OFL_OK;
+  CallArg a[] = {{chunk, rows, cols * 4, ld_chunk * 4, COPY_IN | COPY_OUT, 4},
+                 {unsolved, rows, cols, cols, COPY_OUT, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_breach_pits(a[0].d<float>(), rows, cols, a[0].ld(4), nodata, a[1].d<int8_t>(), info, workspace,
+                            workspace_bytes, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 size_t ofl_strip_workspace_bytes(int64_t rows, int64_t cols) { return strip_workspace_bytes(rows, cols); }

@@ -58,8 +58,10 @@ int device_generation();
 // ofl_shutdown): destroy what was created there.
 void register_device_cleanup(void (*fn)());
 
-// Library-owned device scratch, grown on demand and kept until ofl_shutdown (slot-indexed).
-enum ScratchSlot { SCRATCH_DEM = 0, SCRATCH_FDR, SCRATCH_FAC, SCRATCH_WORK, SCRATCH_LINKS, SCRATCH_MISC, SCRATCH_DIRCTR, SCRATCH_SLOTS };
+// Library-owned device scratch, grown on demand and kept until ofl_shutdown (slot-indexed).  A host-memory call
+// stages its argument i in slot SCRATCH_STAGE0 + i (api.cu).
+constexpr int SCRATCH_STAGE_SLOTS = 5;
+enum ScratchSlot { SCRATCH_STAGE0 = 0, SCRATCH_WORK = SCRATCH_STAGE0 + SCRATCH_STAGE_SLOTS, SCRATCH_MISC, SCRATCH_DIRCTR, SCRATCH_SLOTS };
 int scratch_get(int slot, size_t bytes, void** out);
 // Pinned host scratch (slot-indexed) for small read-backs.
 int pinned_get(size_t bytes, void** out);

@@ -16,6 +16,7 @@ import numpy as np
 
 from . import _native
 from .constants import FLOW_DIRECTION_UNDEFINED
+from .flow_accumulation import as_codes
 
 _MAX_CELLS = 2**32
 
@@ -33,19 +34,11 @@ def _dem_f32(dem) -> np.ndarray:
     return np.ascontiguousarray(dem)
 
 
-def _codes(fdr, like=None) -> np.ndarray:
-    fdr = np.asarray(fdr)
-    if fdr.ndim != 2:
-        raise ValueError("flow direction raster must be a 2-D array")
-    if like is not None and fdr.shape != like.shape:
+def _codes(fdr, like) -> np.ndarray:
+    fdr = as_codes(fdr)
+    if fdr.shape != like.shape:
         raise ValueError(f"shape mismatch: {fdr.shape} vs {like.shape}")
-    if fdr.dtype != np.uint8:
-        if not np.issubdtype(fdr.dtype, np.integer):
-            raise TypeError(f"flow direction codes must be integers, got {fdr.dtype}")
-        if fdr.size and (fdr.min() < 0 or fdr.max() > 255):
-            raise ValueError("flow direction codes must be in 0..255")
-        fdr = fdr.astype(np.uint8)
-    return np.ascontiguousarray(fdr)
+    return fdr
 
 
 def _i32(a, what, like) -> np.ndarray:

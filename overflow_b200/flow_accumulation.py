@@ -68,13 +68,15 @@ def follow_path(flow_direction, row, col, links):
     raise ValueError("flow direction raster contains a cycle")
 
 
-def _as_codes(flow_direction: np.ndarray) -> np.ndarray:
+def as_codes(flow_direction) -> np.ndarray:
+    """A flow-direction raster as the C-contiguous uint8 codes the library takes.  Any integer dtype is accepted;
+    a code outside 0..255 raises ValueError instead of wrapping."""
     fdr = np.asarray(flow_direction)
     if fdr.ndim != 2:
-        raise ValueError("flow_direction must be a 2-D array")
+        raise ValueError("flow direction raster must be a 2-D array")
     if fdr.dtype != np.uint8:
         if not np.issubdtype(fdr.dtype, np.integer):
-            raise TypeError(f"flow_direction must hold integer codes, got {fdr.dtype}")
+            raise TypeError(f"flow direction codes must be integers, got {fdr.dtype}")
         if fdr.size and (fdr.min() < 0 or fdr.max() > 255):
             raise ValueError("flow direction codes must be in 0..255")
         fdr = fdr.astype(np.uint8)
@@ -88,7 +90,7 @@ def flow_accumulation_for_raster(flow_direction: np.ndarray, with_links: bool = 
     NODATA cells hold -9998 exactly as the reference leaves them.  `out` may be a preallocated
     C-contiguous int64 array (e.g. pinned memory) of the raster's shape.
     """
-    fdr = _as_codes(flow_direction)
+    fdr = as_codes(flow_direction)
     rows, cols = fdr.shape
     if out is None:
         fac = np.empty((rows, cols), dtype=np.int64)
@@ -116,7 +118,7 @@ def single_tile_flow_accumulation(flow_direction: np.ndarray):
     are FLOW_EXTERNAL / FLOW_TERMINATES / the (row, col) of the exit cell; interior entries,
     uninitialised in the reference, are zero.
     """
-    fdr = _as_codes(flow_direction)
+    fdr = as_codes(flow_direction)
     fac, perim = flow_accumulation_for_raster(fdr, with_links=True)
     links = np.zeros(fdr.shape + (2,), dtype=np.int64)
     if len(perim):
@@ -129,7 +131,7 @@ def check_flow_accumulation(flow_direction: np.ndarray, flow_accumulation_raster
     """Cells violating fac = 1 + sum(upstream fac) (data) or fac = -9998 (nodata); 0 proves exactness."""
     import ctypes
 
-    fdr = _as_codes(flow_direction)
+    fdr = as_codes(flow_direction)
     fac = np.ascontiguousarray(flow_accumulation_raster, dtype=np.int64)
     rows, cols = fdr.shape
     n_bad = ctypes.c_int64(0)

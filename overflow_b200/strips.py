@@ -26,6 +26,7 @@ import numpy as np
 import torch
 
 from . import _native
+from .flow_accumulation import as_codes
 
 TILE = 64  # strips must start on multiples of the accumulation tile side
 
@@ -419,7 +420,7 @@ def flow_accumulation_out_of_core(read_rows, write_rows, rows, cols, strip_rows,
         """Codes of strip s plus one halo row above and below (raster edges: the halo row is never looked at)."""
         r0, r1 = bounds[s]
         lo, hi = max(0, r0 - 1), min(rows, r1 + 1)
-        block = np.ascontiguousarray(read_rows(lo, hi), dtype=np.uint8)
+        block = as_codes(read_rows(lo, hi))
         if block.shape != (hi - lo, cols):
             raise ValueError(f"read_rows({lo}, {hi}) returned shape {block.shape}, expected {(hi - lo, cols)}")
         view = fdr_halo[: r1 - r0 + 2]

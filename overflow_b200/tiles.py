@@ -22,6 +22,7 @@ import numpy as np
 
 from . import _native
 from .constants import FLOW_DIRECTION_NODATA
+from .flow_accumulation import as_codes
 
 _DY = np.array([0, -1, -1, -1, 0, 1, 1, 1], dtype=np.int64)  # E, NE, N, NW, W, SW, S, SE (constants.py:29-40)
 _DX = np.array([1, 1, 0, -1, -1, -1, 0, 1], dtype=np.int64)
@@ -167,7 +168,7 @@ def flow_accumulation_tiled(read_window, write_window, rows, cols, tile_rows, ti
 
     def load(t):
         r0, r1, c0, c1 = tiles[t]
-        block = np.ascontiguousarray(read_window(r0, r1, c0, c1), dtype=np.uint8)
+        block = as_codes(read_window(r0, r1, c0, c1))
         if block.shape != (r1 - r0, c1 - c0):
             raise ValueError(f"read_window{(r0, r1, c0, c1)} returned shape {block.shape}")
         return block

@@ -141,6 +141,14 @@ def test_out_of_core_matches_whole_raster(name, dem, strip_rows):
     assert np.array_equal(got, want_fac)
 
 
+def test_out_of_core_refuses_a_code_outside_0_255():
+    fdr = np.full((130, 20), 8, dtype=np.int64)
+    fdr[100, 7] = 265  # would wrap to 9 (NODATA) as uint8
+    with pytest.raises(ValueError, match="0..255"):
+        strips.flow_accumulation_out_of_core(lambda r0, r1: fdr[r0:r1], lambda r0, fac: None, 130, 20, 64,
+                                             engine=NumpyStripEngine())
+
+
 def test_out_of_core_file_driver(tmp_path):
     from overflow_b200.util.raster import create_raster, open_raster
 

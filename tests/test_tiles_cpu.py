@@ -92,6 +92,14 @@ def test_cycle_across_tiles_is_reported():
     assert ei.value.status == _native.OFL_ERR_CYCLE
 
 
+def test_code_outside_0_255_is_refused():
+    fdr = np.full((4, 8), 8, dtype=np.int64)
+    fdr[2, 5] = 265  # would wrap to 9 (NODATA) as uint8
+    with pytest.raises(ValueError, match="0..255"):
+        tiles.flow_accumulation_tiled(lambda r0, r1, c0, c1: fdr[r0:r1, c0:c1], lambda *a: None, 4, 8, 4, 4,
+                                      engine=OracleTileEngine())
+
+
 def test_tiled_file_driver(tmp_path):
     from overflow_b200.util.raster import create_raster, open_raster
 
