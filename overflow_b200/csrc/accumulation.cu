@@ -15,7 +15,7 @@
 //           warp-ballot compacted frontier queues), follow the perimeter cells that can receive
 //           inflow from outside the tile to where their path leaves it (Alg. 2), and emit the
 //           reduced graph: the successor perimeter cell in the next tile, the locally accumulated
-//           counts that cross the tile edge, and -- on whole-raster calls -- the solve's initial state.
+//           counts that cross the tile edge, and the solve's initial state.
 //   solve   (pj_solve_kernel)        the reduced graph is a forest over ~2% of the cells;
 //           subtree sums over it by pointer doubling: O(log depth) rounds of
 //           "add my sum to my 2^j-th ancestor, then jump", integer atomics, exact; all rounds in one
@@ -33,6 +33,7 @@
 // out-of-bounds NEIGHBOR_OFFSETS read); NODATA cells end at -9998 (:119-121,129-137).
 #include <atomic>
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -107,8 +108,10 @@ struct AccParams {
   int vec_store;  // fac rows are 16-byte aligned: the final pass may use 16-byte stores
   int* wide_list;  // [0]: number of tiles the 32-bit final pass left to the 64-bit variant, [1..]: their ids
   int force_wide;  // test hook: send every tile with an inflow through the 64-bit variant
-  // whole-raster calls: pass A publishes its slots straight into the solve's initial state (pointer
-  // buffers, cleared delta entries, per-segment active lists) instead of `succ` + a separate init kernel
+  // pass A publishes its slots straight into the solve's initial state (pointer buffers, cleared delta entries,
+  // per-segment active lists); keep_succ: it also writes `succ`, from which a strip solves its forest a second time.
+  // The host always sets fuse_init.  Removing it (and publish_slot's early return) changes the parameter block of
+  // every kernel that takes AccParams, so that is left to the next measured change to pass A.
   int fuse_init, keep_succ;
   int trusted_codes;  // the codes come straight from direction_kernel (0..9 only): pass A skips its sanitising sweep
   int32_t *ptr_a, *ptr_b, *list0;
@@ -1211,30 +1214,100 @@ static PjSeg pj_segments(int64_t n) {
   return g;
 }
 
-// Subtree sums over the forest `succ` (succ[u] = parent node or -1): on return (stream order) S[u] holds
-// the sum of the initial S over u's subtree and both pointer buffers hold ~root(u) for every node.  succ is
-// preserved.  lists: 2 * (blocks * seg) int32; counts: [0, PJ_MAX_BLOCKS) the per-segment active counts when
-// pass A published the initial state (with_init = false), then the kernel's barrier words; d0/d1 need no
-// initialisation.  Does not synchronise: *leftover is set when the forest did not converge (a cycle).
-static int pj_solve(const int32_t* succ, int32_t* ptr_a, int32_t* ptr_b, int32_t* lists, int* counts, int* leftover,
-                    unsigned long long* S, unsigned long long* d0, unsigned long long* d1, int64_t n, cudaStream_t st,
-                    bool with_init = true, const int* run_flag = nullptr) {
+// Words of a perimeter graph's flag block, cleared with its sums.  The tile flag (pass A saw a cycle, or a window its
+// queue cannot address) and the solve flag (a solve did not converge: a cycle) are the errors a call reports; they are
+// read as one pair.  The seed-route word is not an error: it says which route a strip's inflow from other strips
+// takes (strip_accum_final).
+enum GraphFlag { FLAG_TILE = 0, FLAG_SOLVE = 1, FLAG_SEED_ROUTE = 8, GRAPH_FLAG_WORDS = 16 };
+static_assert(FLAG_SOLVE == FLAG_TILE + 1, "the two error flags are copied as one pair");
+
+constexpr int PJ_SYNC_WORDS = PJ_MAX_ROUNDS + 4;  // the solve's grid barrier and nodes left after each round
+
+// A whole raster's graph, a row strip's (it solves the same forest a second time, into S2), or the strips' boundary
+// graph (no tiles: no pass A, and the solve builds its own initial state).
+enum class GraphKind { RASTER, STRIP, BOUNDARY };
+
+// The workspace of one perimeter graph with n nodes.
+struct Graph {
+  GraphKind kind;
+  int64_t n;
+  int32_t *succ, *ptr_a, *ptr_b;
+  int32_t* lists;                        // 2 ping-pong lists of blocks * seg >= n entries
+  unsigned long long *S, *S2, *d0, *d1;  // S2 is S except on a strip
+  uint16_t* link;
+  int* counts;     // [2 * PJ_MAX_BLOCKS]: the per-segment active nodes pass A publishes for round 0
+  unsigned* sync;  // [PJ_SYNC_WORDS], zeroed by each solve
+  int* flags;      // [GRAPH_FLAG_WORDS], see GraphFlag
+  uint16_t* L;     // tile-local counts of pass A (empty on the boundary graph)
+  int* wide;       // tiles the final pass leaves to its 64-bit variant (empty on the boundary graph)
+  size_t bytes;    // size of the workspace
+};
+
+// Cuts the graph's buffers out of the workspace at `base`, each 256-byte aligned.  With a null base only `bytes` is
+// meaningful.
+static Graph carve_graph(void* base, int64_t n, GraphKind kind) {
+  Graph g;
+  g.kind = kind;
+  g.n = n;
+  size_t o = 0;
+  auto take = [&](auto& ptr, size_t bytes) {
+    ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(reinterpret_cast<uintptr_t>(base) + o);
+    o = align_up(o + bytes, 256);
+  };
+  const size_t nodes = (size_t)n;
+  const bool tiled = kind != GraphKind::BOUNDARY;
+  take(g.succ, nodes * 4);
+  take(g.ptr_a, nodes * 4);
+  take(g.ptr_b, nodes * 4);
+  take(g.lists, (nodes + 64 * (size_t)PJ_MAX_BLOCKS) * 8);
+  take(g.S, nodes * 8);
+  g.S2 = g.S;
+  if (kind == GraphKind::STRIP) take(g.S2, nodes * 8);
+  take(g.d0, nodes * 8);
+  take(g.d1, nodes * 8);
+  take(g.link, nodes * 2);
+  take(g.counts, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int));
+  take(g.sync, PJ_SYNC_WORDS * sizeof(unsigned));
+  take(g.flags, GRAPH_FLAG_WORDS * sizeof(int));
+  take(g.L, tiled ? nodes / SLOTS * AT * AT * sizeof(uint16_t) : 0);
+  take(g.wide, tiled ? (nodes / SLOTS + 1) * sizeof(int) : 0);
+  g.bytes = o;
+  return g;
+}
+
+// Zero what a call that starts on the graph accumulates into: the sums S and S2 (together before d0; the solve clears
+// what it uses of the delta buffers itself), the flag words and, where pass A publishes the solve's initial state, the
+// per-segment counts it adds to.
+static int clear_graph(const Graph& g, cudaStream_t st) {
+  OFL_CUDA(cudaMemsetAsync(g.S, 0, reinterpret_cast<uint8_t*>(g.d0) - reinterpret_cast<uint8_t*>(g.S), st));
+  OFL_CUDA(cudaMemsetAsync(g.flags, 0, GRAPH_FLAG_WORDS * sizeof(int), st));
+  if (g.kind != GraphKind::BOUNDARY) OFL_CUDA(cudaMemsetAsync(g.counts, 0, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int), st));
+  return OFL_OK;
+}
+
+// Subtree sums over the graph's forest: on return (stream order) S[u] (S is the graph's S or S2) holds the sum of the
+// initial S over u's subtree and both pointer buffers hold ~root(u) for every node.  with_init: the solve starts from
+// `succ`, which it preserves; otherwise from the state pass A published.  run_flag (nullable): a device word; the
+// solve is skipped when it is 0.  Does not synchronise: the solve flag is set when the forest did not converge (a
+// cycle).
+static int pj_solve(const Graph& graph, unsigned long long* S, cudaStream_t st, bool with_init,
+                    const int* run_flag = nullptr) {
   PjArgs a;
   a.run_flag = run_flag;
-  a.succ = succ;
-  a.ptr_a = ptr_a;
-  a.ptr_b = ptr_b;
-  a.lists = lists;
-  a.counts0 = counts;
+  a.succ = graph.succ;
+  a.ptr_a = graph.ptr_a;
+  a.ptr_b = graph.ptr_b;
+  a.lists = graph.lists;
+  a.counts0 = graph.counts;
   a.S = S;
-  a.d0 = d0;
-  a.d1 = d1;
-  a.sync = reinterpret_cast<unsigned*>(counts + 2 * PJ_MAX_BLOCKS);
-  a.leftover = leftover;
-  a.g = pj_segments(n);
+  a.d0 = graph.d0;
+  a.d1 = graph.d1;
+  a.sync = graph.sync;
+  a.leftover = graph.flags + FLAG_SOLVE;
+  a.g = pj_segments(graph.n);
   a.with_init = with_init ? 1 : 0;
-  a.max_rounds = pj_rounds_for(n);
-  OFL_CUDA(cudaMemsetAsync(a.sync, 0, (size_t)(PJ_MAX_ROUNDS + 4) * sizeof(unsigned), st));
+  a.max_rounds = pj_rounds_for(graph.n);
+  OFL_CUDA(cudaMemsetAsync(a.sync, 0, PJ_SYNC_WORDS * sizeof(unsigned), st));
   void* args[] = {&a};
   OFL_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(pj_solve_kernel), dim3((unsigned)a.g.blocks), dim3(256),
                                        args, 0, st));
@@ -1242,48 +1315,15 @@ static int pj_solve(const int32_t* succ, int32_t* ptr_a, int32_t* ptr_b, int32_t
   return OFL_OK;
 }
 
-// One synchronisation at the end of a call: err[0] = cycle seen by a tile kernel, err[1] = a solve did
-// not converge.
-static int check_flags(const int* err_flags, cudaStream_t st) {
-  int h[2] = {0, 0};
-  OFL_CUDA(cudaMemcpyAsync(h, err_flags, sizeof(h), cudaMemcpyDeviceToHost, st));
+// One synchronisation at the end of a call.
+static int check_flags(const Graph& g, cudaStream_t st) {
+  int h[2] = {0, 0};  // tile flag, solve flag
+  OFL_CUDA(cudaMemcpyAsync(h, g.flags + FLAG_TILE, sizeof(h), cudaMemcpyDeviceToHost, st));
   OFL_CUDA(cudaStreamSynchronize(st));
   OFL_REQUIRE(h[0] != 3, OFL_ERR_INVALID, "shared-memory window above 64 KB: the tile kernel's 16-bit queue does not apply");
   OFL_REQUIRE(h[0] == 0, OFL_ERR_CYCLE, "flow-direction raster contains a cycle (tile flag %d)", h[0]);
   OFL_REQUIRE(h[1] == 0, OFL_ERR_CYCLE, "flow-direction raster contains a cycle (perimeter graph)");
   return OFL_OK;
-}
-
-// Workspace of one perimeter graph with n nodes.  `keep_succ`: strips solve the same forest twice.
-struct GraphLayout {
-  int64_t n;
-  size_t off_succ, off_pa, off_pb, off_lists, off_S, off_S2, off_d0, off_d1, off_link, off_counts, off_err, off_L, off_wide, total;
-};
-
-static GraphLayout graph_layout(int64_t n, bool strip, bool with_tiles = true) {
-  GraphLayout L;
-  L.n = n;
-  size_t o = 0;
-  auto take = [&](size_t bytes) {
-    const size_t at = o;
-    o = align_up(o + bytes, 256);
-    return at;
-  };
-  L.off_succ = take((size_t)n * 4);
-  L.off_pa = take((size_t)n * 4);
-  L.off_pb = take((size_t)n * 4);
-  L.off_lists = take(((size_t)n + 64 * (size_t)PJ_MAX_BLOCKS) * 8);  // 2 ping-pong lists of blocks*seg >= n entries
-  L.off_S = take((size_t)n * 8);
-  L.off_S2 = strip ? take((size_t)n * 8) : L.off_S;
-  L.off_d0 = take((size_t)n * 8);
-  L.off_d1 = take((size_t)n * 8);
-  L.off_link = take((size_t)n * 2);
-  L.off_counts = take(((size_t)2 * PJ_MAX_BLOCKS + PJ_MAX_ROUNDS + 4) * sizeof(int));
-  L.off_err = take(64);
-  L.off_L = with_tiles ? take((size_t)(n / SLOTS) * AT * AT * sizeof(uint16_t)) : o;
-  L.off_wide = with_tiles ? take((size_t)(n / SLOTS + 1) * sizeof(int)) : o;
-  L.total = o;
-  return L;
 }
 
 static inline int64_t node_count(int64_t rows, int64_t cols) {
@@ -1292,32 +1332,20 @@ static inline int64_t node_count(int64_t rows, int64_t cols) {
 
 size_t accumulation_workspace_bytes(int64_t rows, int64_t cols) {
   if (rows <= 0 || cols <= 0) return 256;
-  return graph_layout(node_count(rows, cols), false).total;
+  return carve_graph(nullptr, node_count(rows, cols), GraphKind::RASTER).bytes;
 }
 
 size_t strip_workspace_bytes(int64_t rows, int64_t cols) {
   if (rows <= 0 || cols <= 0) return 256;
-  return graph_layout(node_count(rows, cols), true).total;
-}
-
-// Zero the sums [from_off, off_d0) of the workspace (the solve clears what it uses of the delta buffers
-// itself) and the error flags.
-static int ws_begin(uint8_t* ws, const GraphLayout& L, size_t from_off, cudaStream_t st) {
-  OFL_CUDA(cudaMemsetAsync(ws + from_off, 0, L.off_d0 - from_off, st));
-  OFL_CUDA(cudaMemsetAsync(ws + L.off_err, 0, 64, st));
-  return OFL_OK;
+  return carve_graph(nullptr, node_count(rows, cols), GraphKind::STRIP).bytes;
 }
 
 // Everything one raster (or strip) needs to launch its kernels.
 struct AccCtx {
   AccParams p;
-  CUtensorMap tm;        // codes + halo box for pass A
-  GraphLayout L;
-  uint8_t* ws;
+  CUtensorMap tm;  // codes + halo box for pass A
+  Graph graph;
   int64_t ntiles;
-  int32_t *pa, *pb, *lists;
-  unsigned long long *S2, *d0, *d1;
-  int* counts;
 };
 
 static int acc_setup(AccCtx& C, const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int y_off, int has_above,
@@ -1328,59 +1356,49 @@ static int acc_setup(AccCtx& C, const uint8_t* fdr, int64_t rows, int64_t cols, 
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(fac) & 7) == 0 && ld_fac >= cols, OFL_ERR_ALIGNMENT, "fac must be 8-byte aligned");
   const int64_t n = node_count(rows, cols);
   OFL_REQUIRE(n < (1ll << 31), OFL_ERR_INVALID, "raster too large for 32-bit perimeter node ids");
-  C.L = graph_layout(n, strip);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= C.L.total, OFL_ERR_WORKSPACE,
-              "accumulation workspace too small: need %zu bytes, have %zu", C.L.total, workspace_bytes);
-  C.ws = static_cast<uint8_t*>(workspace);
+  C.graph = carve_graph(workspace, n, strip ? GraphKind::STRIP : GraphKind::RASTER);
+  const Graph& g = C.graph;
+  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE,
+              "accumulation workspace too small: need %zu bytes, have %zu", g.bytes, workspace_bytes);
   AccParams& p = C.p;
   p.rows = (int)rows;
   p.cols = (int)cols;
   p.nty = (int)((rows + AT - 1) / AT);
   p.ntx = (int)((cols + AT - 1) / AT);
-  p.succ = reinterpret_cast<int32_t*>(C.ws + C.L.off_succ);
-  p.link = reinterpret_cast<uint16_t*>(C.ws + C.L.off_link);
-  p.S = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_S);
+  p.succ = g.succ;
+  p.link = g.link;
+  p.S = g.S;
   p.fac = fac;
   p.ld_fac = ld_fac;
-  p.err = reinterpret_cast<int*>(C.ws + C.L.off_err);
-  p.L = reinterpret_cast<uint16_t*>(C.ws + C.L.off_L);
-  p.wide_list = reinterpret_cast<int*>(C.ws + C.L.off_wide);
+  p.err = g.flags + FLAG_TILE;
+  p.L = g.L;
+  p.wide_list = g.wide;
   p.force_wide = getenv("OFL_FORCE_WIDE_FINAL") ? 1 : 0;
   p.trusted_codes = 0;
-  {
-    const PjSeg g = pj_segments(n);
-    p.fuse_init = getenv("OFL_NO_FUSED_INIT") ? 0 : 1;
-    p.keep_succ = (strip || !p.fuse_init) ? 1 : 0;
-    p.ptr_a = reinterpret_cast<int32_t*>(C.ws + C.L.off_pa);
-    p.ptr_b = reinterpret_cast<int32_t*>(C.ws + C.L.off_pb);
-    p.list0 = reinterpret_cast<int32_t*>(C.ws + C.L.off_lists);
-    p.d0 = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_d0);
-    p.d1 = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_d1);
-    p.counts0 = reinterpret_cast<int*>(C.ws + C.L.off_counts);
-    p.tiles_per_seg = (int)(g.seg / SLOTS);
-    p.seg = g.seg;
-  }
+  p.fuse_init = 1;
+  p.keep_succ = strip ? 1 : 0;
+  p.ptr_a = g.ptr_a;
+  p.ptr_b = g.ptr_b;
+  p.list0 = g.lists;
+  p.d0 = g.d0;
+  p.d1 = g.d1;
+  p.counts0 = g.counts;
+  const PjSeg seg = pj_segments(n);
+  p.tiles_per_seg = (int)(seg.seg / SLOTS);
+  p.seg = seg.seg;
   p.y_off = y_off;
   p.strip_above = has_above ? 1 : 0;
   p.strip_below = has_below ? 1 : 0;
   p.tile_base = 0;
   p.vec_store = ((reinterpret_cast<uintptr_t>(fac) & 15) == 0 && (ld_fac % 2) == 0) ? 1 : 0;
-  C.pa = reinterpret_cast<int32_t*>(C.ws + C.L.off_pa);
-  C.pb = reinterpret_cast<int32_t*>(C.ws + C.L.off_pb);
-  C.lists = reinterpret_cast<int32_t*>(C.ws + C.L.off_lists);
-  C.S2 = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_S2);
-  C.d0 = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_d0);
-  C.d1 = reinterpret_cast<unsigned long long*>(C.ws + C.L.off_d1);
-  C.counts = reinterpret_cast<int*>(C.ws + C.L.off_counts);
   C.ntiles = (int64_t)p.nty * p.ntx;
   int rc = make_tensor_map_2d(&C.tm, fdr, 1, (uint64_t)cols, (uint64_t)(rows + 2 * y_off), (uint64_t)ld_fdr, ACS_W, ACS_H);
   if (rc != OFL_OK) return rc;
   return ensure_tile_attrs();
 }
 
-
 // Final pass over `grid` tiles starting at p.tile_base: the 32-bit kernel, then the 64-bit one on whatever it listed.
-static int launch_final(const AccCtx& C, const AccParams& p, unsigned grid, cudaStream_t st) {
+static int launch_final(const AccParams& p, unsigned grid, cudaStream_t st) {
   OFL_CUDA(cudaMemsetAsync(p.wide_list, 0, sizeof(int), st));
   acc_final_kernel<<<grid, ACC_THREADS, FinalSmem::BYTES_FAST, st>>>(p);
   OFL_CHECK_LAUNCH();
@@ -1390,21 +1408,35 @@ static int launch_final(const AccCtx& C, const AccParams& p, unsigned grid, cuda
   return OFL_OK;
 }
 
-// The part of a whole-raster accumulation that does not depend on the codes: clearing the sums, the error
-// flags and round 0's counters.  A caller that produces the codes on the same device (ofl_flow_routing_f32)
-// runs it on a second stream next to the direction kernel and passes prepared = true below.
+// The phases the whole-raster and strip calls share, each timed as one phase.
+static int pass_a(const AccCtx& C, cudaStream_t st) {
+  {
+    PhaseScope ps(PHASE_ACC_TILE_A, st);
+    acc_tile_kernel<<<(unsigned)C.ntiles, ACC_THREADS, TileSmem::BYTES, st>>>(C.tm, C.p);
+  }
+  OFL_CHECK_LAUNCH();
+  return OFL_OK;
+}
+
+static int solve_published(const AccCtx& C, cudaStream_t st) {  // from the initial state pass A published
+  PhaseScope ps(PHASE_ACC_SOLVE, st);
+  return pj_solve(C.graph, C.graph.S, st, false);
+}
+
+static int final_pass(const AccCtx& C, cudaStream_t st) {  // over every tile
+  PhaseScope ps(PHASE_ACC_TILE_B, st);
+  return launch_final(C.p, (unsigned)C.ntiles, st);
+}
+
+// The part of a whole-raster accumulation that does not depend on the codes: clear_graph.  A caller that produces the
+// codes on the same device (ofl_flow_routing_f32) runs it on a second stream next to the direction kernel and passes
+// prepared = true below.
 int accumulation_prepare(int64_t rows, int64_t cols, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   if (rows <= 0 || cols <= 0) return OFL_OK;
-  const int64_t n = node_count(rows, cols);
-  const GraphLayout L = graph_layout(n, false);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= L.total, OFL_ERR_WORKSPACE,
-              "accumulation workspace too small: need %zu bytes, have %zu", L.total, workspace_bytes);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  int rc = ws_begin(ws, L, L.off_S, st);  // S
-  if (rc != OFL_OK) return rc;
-  // round 0's active / retired counts: pass A adds to the first, nothing retires before round 0
-  OFL_CUDA(cudaMemsetAsync(ws + L.off_counts, 0, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int), st));
-  return OFL_OK;
+  const Graph g = carve_graph(workspace, node_count(rows, cols), GraphKind::RASTER);
+  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE,
+              "accumulation workspace too small: need %zu bytes, have %zu", g.bytes, workspace_bytes);
+  return clear_graph(g, st);
 }
 
 int launch_accumulation(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, long long* fac,
@@ -1415,40 +1447,29 @@ int launch_accumulation(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t 
   int rc = acc_setup(C, fdr, rows, cols, ld_fdr, 0, 0, 0, fac, ld_fac, workspace, workspace_bytes, false);
   if (rc != OFL_OK) return rc;
   C.p.trusted_codes = trusted_codes ? 1 : 0;
-  const GraphLayout& L = C.L;
   if (!prepared) {
-    rc = accumulation_prepare(rows, cols, workspace, workspace_bytes, st);
+    rc = clear_graph(C.graph, st);
     if (rc != OFL_OK) return rc;
   }
-  {
-    PhaseScope ps(PHASE_ACC_TILE_A, st);
-    acc_tile_kernel<<<(unsigned)C.ntiles, ACC_THREADS, TileSmem::BYTES, st>>>(C.tm, C.p);
-  }
-  OFL_CHECK_LAUNCH();
+  rc = pass_a(C, st);
+  if (rc != OFL_OK) return rc;
+  const int64_t n_perim = perimeter_count(rows, cols);
   if (perim_inflow_dev) {
-    const int64_t n = perimeter_count(rows, cols);
-    perim_seed_kernel<<<grid_for(n, 16), 256, 0, st>>>(perim_inflow_dev, C.p, C.p.S, n);
+    perim_seed_kernel<<<grid_for(n_perim, 16), 256, 0, st>>>(perim_inflow_dev, C.p, C.p.S, n_perim);
     OFL_CHECK_LAUNCH();
   }
-  {
-    PhaseScope ps(PHASE_ACC_SOLVE, st);
-    rc = pj_solve(C.p.succ, C.pa, C.pb, C.lists, C.counts, C.p.err + 1, C.p.S, C.d0, C.d1, L.n, st, !C.p.fuse_init);
-  }
+  rc = solve_published(C, st);
   if (rc != OFL_OK) return rc;
-  {
-    PhaseScope ps(PHASE_ACC_TILE_B, st);
-    rc = launch_final(C, C.p, (unsigned)C.ntiles, st);
-  }
+  rc = final_pass(C, st);
   if (rc != OFL_OK) return rc;
   if (perim_links_dev) {
-    const int64_t n = perimeter_count(rows, cols);
     {
       PhaseScope ps(PHASE_ACC_LINKS, st);
-      links_kernel<<<grid_for(n, 16), 256, 0, st>>>(fdr, ld_fdr, C.pa, C.p.link, C.p, perim_links_dev, n);
+      links_kernel<<<grid_for(n_perim, 16), 256, 0, st>>>(fdr, ld_fdr, C.p.ptr_a, C.p.link, C.p, perim_links_dev, n_perim);
     }
     OFL_CHECK_LAUNCH();
   }
-  return check_flags(C.p.err, st);
+  return check_flags(C.graph, st);
 }
 
 // ================================================================ row strips (multi-GPU)
@@ -1632,39 +1653,31 @@ int strip_accum_local(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64
   AccCtx C;
   int rc = strip_setup(C, fdr_halo, rows, cols, ld_fdr, has_above, has_below, fac, ld_fac, workspace, workspace_bytes);
   if (rc != OFL_OK) return rc;
-  const GraphLayout& L = C.L;
-  rc = ws_begin(C.ws, L, L.off_S, st);  // S, S2
+  rc = clear_graph(C.graph, st);
   if (rc != OFL_OK) return rc;
-  if (C.p.fuse_init) OFL_CUDA(cudaMemsetAsync(C.counts, 0, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int), st));
-  {
-    PhaseScope ps(PHASE_ACC_TILE_A, st);
-    acc_tile_kernel<<<(unsigned)C.ntiles, ACC_THREADS, TileSmem::BYTES, st>>>(C.tm, C.p);
-  }
-  OFL_CHECK_LAUNCH();
-  {
-    PhaseScope ps(PHASE_ACC_SOLVE, st);
-    rc = pj_solve(C.p.succ, C.pa, C.pb, C.lists, C.counts, C.p.err + 1, C.p.S, C.d0, C.d1, L.n, st, !C.p.fuse_init);
-  }
+  rc = pass_a(C, st);
+  if (rc != OFL_OK) return rc;
+  rc = solve_published(C, st);
   if (rc != OFL_OK) return rc;
   // strip-local counts of the first and last tile row (their cells include both boundary rows)
   {
     PhaseScope ps(PHASE_STRIP_EDGE, st);
     AccParams pb = C.p;
-    rc = launch_final(C, pb, (unsigned)pb.ntx, st);
+    rc = launch_final(pb, (unsigned)pb.ntx, st);
     if (rc == OFL_OK && pb.nty > 1) {
       pb.tile_base = (pb.nty - 1) * pb.ntx;
-      rc = launch_final(C, pb, (unsigned)pb.ntx, st);
+      rc = launch_final(pb, (unsigned)pb.ntx, st);
     }
   }
   if (rc != OFL_OK) return rc;
-  strip_boundary_extract_kernel<<<grid_for(2 * cols, 8), 256, 0, st>>>(fdr_halo, ld_fdr, fac, ld_fac, C.pa, C.p.link, C.p,
+  strip_boundary_extract_kernel<<<grid_for(2 * cols, 8), 256, 0, st>>>(fdr_halo, ld_fdr, fac, ld_fac, C.p.ptr_a, C.p.link, C.p,
                                                                        static_cast<uint8_t*>(record));
   OFL_CHECK_LAUNCH();
   return OFL_OK;
 }
 
 size_t strip_boundary_workspace_bytes(int n_strips, int64_t cols) {
-  return graph_layout((int64_t)n_strips * 2 * cols, false, false).total;
+  return carve_graph(nullptr, (int64_t)n_strips * 2 * cols, GraphKind::BOUNDARY).bytes;
 }
 
 int strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, long long* J_all, void* workspace,
@@ -1672,31 +1685,22 @@ int strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, lo
   OFL_REQUIRE(n_strips >= 1 && cols >= 1, OFL_ERR_INVALID, "bad boundary graph size");
   const int64_t n = (int64_t)n_strips * 2 * cols;
   OFL_REQUIRE(n < (1ll << 31), OFL_ERR_INVALID, "boundary graph too large");
-  const GraphLayout L = graph_layout(n, false, false);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= L.total, OFL_ERR_WORKSPACE, "boundary workspace too small");
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
-  int32_t* succ = reinterpret_cast<int32_t*>(ws + L.off_succ);
-  unsigned long long* S = reinterpret_cast<unsigned long long*>(ws + L.off_S);
-  int* counts = reinterpret_cast<int*>(ws + L.off_counts);
-  int* err = reinterpret_cast<int*>(ws + L.off_err);
-  OFL_CUDA(cudaMemsetAsync(ws + L.off_S, 0, L.off_d0 - L.off_S, st));
-  OFL_CUDA(cudaMemsetAsync(err, 0, 64, st));
+  const Graph g = carve_graph(workspace, n, GraphKind::BOUNDARY);
+  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE, "boundary workspace too small");
+  int rc = clear_graph(g, st);
+  if (rc != OFL_OK) return rc;
   RecView rec;
   rec.base = static_cast<const uint8_t*>(records_all);
   rec.stride = (int64_t)strip_record_bytes(cols);
   rec.cols = cols;
-  strip_graph_build_kernel<<<grid_for(n, 8), 256, 0, st>>>(rec, n_strips, succ, S);
+  strip_graph_build_kernel<<<grid_for(n, 8), 256, 0, st>>>(rec, n_strips, g.succ, g.S);
   OFL_CHECK_LAUNCH();
-  int rc;
   {
     PhaseScope ps(PHASE_ACC_SOLVE, st);
-    rc = pj_solve(succ, reinterpret_cast<int32_t*>(ws + L.off_pa), reinterpret_cast<int32_t*>(ws + L.off_pb),
-                  reinterpret_cast<int32_t*>(ws + L.off_lists), counts, err + 1, S,
-                  reinterpret_cast<unsigned long long*>(ws + L.off_d0), reinterpret_cast<unsigned long long*>(ws + L.off_d1), n,
-                  st);
+    rc = pj_solve(g, g.S, st, true);
   }
   if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(J_all, S, (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
+  OFL_CUDA(cudaMemcpyAsync(J_all, g.S, (size_t)n * 8, cudaMemcpyDeviceToDevice, st));
   return OFL_OK;
 }
 
@@ -1707,14 +1711,12 @@ int strip_collect_flags(const void* strip_workspace, int64_t rows, int64_t cols,
                         int n_strips, int32_t* flags_dev, cudaStream_t st) {
   OFL_CUDA(cudaMemsetAsync(flags_dev, 0, 4 * sizeof(int32_t), st));
   if (strip_workspace) {
-    const GraphLayout L = graph_layout(node_count(rows, cols), true);
-    OFL_CUDA(cudaMemcpyAsync(flags_dev, static_cast<const uint8_t*>(strip_workspace) + L.off_err, 2 * sizeof(int32_t),
-                             cudaMemcpyDeviceToDevice, st));
+    const Graph g = carve_graph(const_cast<void*>(strip_workspace), node_count(rows, cols), GraphKind::STRIP);
+    OFL_CUDA(cudaMemcpyAsync(flags_dev, g.flags + FLAG_TILE, 2 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
   }
   if (boundary_workspace) {
-    const GraphLayout L = graph_layout((int64_t)n_strips * 2 * cols, false, false);
-    OFL_CUDA(cudaMemcpyAsync(flags_dev + 2, static_cast<const uint8_t*>(boundary_workspace) + L.off_err,
-                             2 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
+    const Graph g = carve_graph(const_cast<void*>(boundary_workspace), (int64_t)n_strips * 2 * cols, GraphKind::BOUNDARY);
+    OFL_CUDA(cudaMemcpyAsync(flags_dev + 2, g.flags + FLAG_TILE, 2 * sizeof(int32_t), cudaMemcpyDeviceToDevice, st));
   }
   return OFL_OK;
 }
@@ -1725,33 +1727,29 @@ int strip_accum_final(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64
   AccCtx C;
   int rc = strip_setup(C, fdr_halo, rows, cols, ld_fdr, has_above, has_below, fac, ld_fac, workspace, workspace_bytes);
   if (rc != OFL_OK) return rc;
-  const GraphLayout& L = C.L;
+  const Graph& g = C.graph;
   // inflow from other strips: walked down the forest from its entry cells when every such path is short, else
   // (device flag) subtree sums of the seeds over the whole forest -- see strip_seed_chase_kernel
-  int* too_long = C.p.err + 8;  // not an error flag: the route the seeds take
+  int* too_long = g.flags + FLAG_SEED_ROUTE;
   const bool force_general = getenv("OFL_SEED_GENERAL") != nullptr;  // test hook: always the general route
   OFL_CUDA(cudaMemsetAsync(too_long, force_general ? 1 : 0, sizeof(int), st));
   {
     PhaseScope ps(PHASE_ACC_SOLVE, st);
     const int gs = grid_for(2 * cols, 8);
-    strip_seed_chase_kernel<true><<<gs, 256, 0, st>>>(J_mine, C.p, C.p.succ, C.p.S, too_long);
+    strip_seed_chase_kernel<true><<<gs, 256, 0, st>>>(J_mine, C.p, g.succ, g.S, too_long);
     OFL_CHECK_LAUNCH();
-    strip_seed_chase_kernel<false><<<gs, 256, 0, st>>>(J_mine, C.p, C.p.succ, C.p.S, too_long);
+    strip_seed_chase_kernel<false><<<gs, 256, 0, st>>>(J_mine, C.p, g.succ, g.S, too_long);
     OFL_CHECK_LAUNCH();
-    strip_seed_kernel_if<<<grid_for(L.n, 8), 256, 0, st>>>(J_mine, C.p, C.S2, L.n, too_long);
+    strip_seed_kernel_if<<<grid_for(g.n, 8), 256, 0, st>>>(J_mine, C.p, g.S2, g.n, too_long);
     OFL_CHECK_LAUNCH();
-    strip_seed_set_kernel_if<<<gs, 256, 0, st>>>(J_mine, C.p, C.S2, too_long);
+    strip_seed_set_kernel_if<<<gs, 256, 0, st>>>(J_mine, C.p, g.S2, too_long);
     OFL_CHECK_LAUNCH();
-    rc = pj_solve(C.p.succ, C.pa, C.pb, C.lists, C.counts, C.p.err + 1, C.S2, C.d0, C.d1, L.n, st, true, too_long);
+    rc = pj_solve(g, g.S2, st, true, too_long);
     if (rc != OFL_OK) return rc;
-    pj_add_kernel_if<<<grid_for(L.n, 8), 256, 0, st>>>(C.p.S, C.S2, L.n, too_long);  // S += S2
+    pj_add_kernel_if<<<grid_for(g.n, 8), 256, 0, st>>>(g.S, g.S2, g.n, too_long);  // S += S2
     OFL_CHECK_LAUNCH();
   }
-  {
-    PhaseScope ps(PHASE_ACC_TILE_B, st);
-    rc = launch_final(C, C.p, (unsigned)C.ntiles, st);
-  }
-  return rc;
+  return final_pass(C, st);
 }
 
 int launch_check(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* fac, int64_t ld_fac,
@@ -1759,11 +1757,8 @@ int launch_check(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr,
                  const long long* fac_below) {
   OFL_CUDA(cudaMemsetAsync(n_bad_dev, 0, sizeof(unsigned long long), st));
   if (rows <= 0 || cols <= 0) return OFL_OK;
-  const int64_t n = rows * cols;
-  const int64_t want = (n + 255) / 256;
-  const int blocks = (int)(want < (int64_t)sm_count() * 16 ? want : (int64_t)sm_count() * 16);
-  check_kernel<<<blocks, 256, 0, st>>>(fdr, ld_fdr, fac, ld_fac, (int)rows, (int)cols, y_off, fac_above, fac_below,
-                                       n_bad_dev);
+  check_kernel<<<grid_for(rows * cols, 16), 256, 0, st>>>(fdr, ld_fdr, fac, ld_fac, (int)rows, (int)cols, y_off, fac_above,
+                                                          fac_below, n_bad_dev);
   OFL_CHECK_LAUNCH();
   return OFL_OK;
 }
