@@ -24,6 +24,9 @@
  *   ofl_d8_masked_flow_dirs_i32   src/overflow/fix_flats.py:291-339  d8_masked_flow_dirs
  *   ofl_fix_flats_f32             resolve_flats followed by d8_masked_flow_dirs, codes rewritten in place
  *   ofl_breach_single_cell_pits_f32  src/overflow/breach_single_cell_pits.py:9-63  breach_single_cell_pits_in_chunk
+ *   ofl_label_basins_u8           no reference counterpart: drainage basins -- the outlet (or pour point) each cell's
+ *                                 D8 path reaches, over the accumulation's edge rule
+ *   ofl_check_basins_u8           no reference counterpart: exactness check of a basin labelling
  *   ofl_synth_dem_f32             no reference counterpart: seeded synthetic DEM for benchmarks
  *
  * Conventions
@@ -112,8 +115,9 @@ void ofl_launch_count_reset(void);
  *   3 accumulation tile pass B   4 perimeter links   5 strip mode: pass B on the strip's first/last tile row
  *   6 flat resolution: the edge / masked-direction stencils   7 flat labelling (edges, components, label order)
  *   8 the two gradient sweeps of flat resolution   9 single-cell pit breaching
+ *   10 basins tile pass (with the pour-point scatter)   11 basins perimeter-node solve   12 basins final pass
  */
-#define OFL_PHASE_COUNT 10
+#define OFL_PHASE_COUNT 13
 void ofl_phase_timing_enable(int on);
 int ofl_phase_timing_read(double* ms, int64_t* counts, int n, int reset);
 
@@ -289,6 +293,35 @@ size_t ofl_pits_workspace_bytes(int64_t rows, int64_t cols);
 int ofl_breach_single_cell_pits_f32(float* chunk, int64_t rows, int64_t cols, int64_t ld_chunk, double nodata,
                                     int8_t* unsolved, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
                                     void* stream);
+
+/*
+ * Drainage basins.  Edge rule of the accumulation: cell c drains into d iff code(c) is 0..7, d lies inside the
+ * raster and code(d) != 9.  A data cell that drains nowhere is an OUTLET (code 8, codes >= 10, a step off the
+ * raster or into NODATA); outlet (r, c) has the label r * cols + c + 1.
+ *   fdr          uint8 codes, rows x cols, leading dimension ld_fdr
+ *   pour_points  nullable; n_pour row-major cell indices r * cols + c.  With pour points, a pour point is a root
+ *                (its outgoing edge is cut) and labels its cells p + 1, where p is the first pour point on the
+ *                cell's path (the cell itself included); a cell whose path meets none gets 0.  A pour point on a
+ *                NODATA cell has no effect; duplicates are allowed; an index outside [0, rows * cols) is
+ *                OFL_ERR_INVALID.
+ *   labels       int64 out, rows x cols, leading dimension ld_labels: the label of the outlet (or pour point) the
+ *                cell's path ends at; NODATA cells get OFL_BASIN_NODATA
+ *   workspace    device scratch of at least ofl_basins_workspace_bytes, which includes the pour-point mask
+ *                (NULL: library-owned, cached)
+ * Alignment contracts as for ofl_flow_accumulation_u8: fdr like its fdr, labels like its fac.  A cyclic raster
+ * is OFL_ERR_CYCLE.  Synchronous with respect to the host (the cycle and pour-point checks read device flags).
+ * ofl_check_basins_u8 counts the cells that break the rule: a NODATA cell has label 0, a cell that drains into a
+ * cell and is not a pour point has that cell's label, a root has its own index + 1 (0 for a natural outlet when
+ * pour points are given).  On an acyclic raster zero violations prove the labels exact.  Synchronises the stream.
+ */
+#define OFL_BASIN_NODATA 0
+size_t ofl_basins_workspace_bytes(int64_t rows, int64_t cols);
+int ofl_label_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
+                        int64_t n_pour, int64_t* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes,
+                        int mem_kind, void* stream);
+int ofl_check_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
+                        int64_t n_pour, const int64_t* labels, int64_t ld_labels, int64_t* n_bad, int mem_kind,
+                        void* stream);
 
 /*
  * Seeded synthetic DEM written straight into device memory (benchmarks / large parity runs).

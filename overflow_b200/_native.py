@@ -19,7 +19,9 @@ OFL_ELEM_F64 = 0
 OFL_ELEM_I64 = 1
 OFL_ELEM_U64 = 2
 
+OFL_ERR_INVALID = -1
 OFL_ERR_CYCLE = -5
+OFL_ERR_WORKSPACE = -6
 
 
 class OverflowB200Error(RuntimeError):
@@ -68,6 +70,9 @@ SIGNATURES = {
     "ofl_fix_flats_f32": (_int, [_vp, _vp, _i64, _i64, _vp, _vp, ctypes.POINTER(_i64), _vp, _sz, _int, _vp]),
     "ofl_pits_workspace_bytes": (_sz, [_i64, _i64]),
     "ofl_breach_single_cell_pits_f32": (_int, [_vp, _i64, _i64, _i64, _f64, _vp, ctypes.POINTER(_i64), _vp, _sz, _int, _vp]),
+    "ofl_basins_workspace_bytes": (_sz, [_i64, _i64]),
+    "ofl_label_basins_u8": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _i64, _vp, _sz, _int, _vp]),
+    "ofl_check_basins_u8": (_int, [_vp, _i64, _i64, _i64, _vp, _i64, _vp, _i64, ctypes.POINTER(_i64), _int, _vp]),
     "ofl_synth_dem_f32": (_int, [_vp, _i64, _i64, _i64, _i64, _i64, ctypes.c_uint64, _int, ctypes.c_float, _int,
                                  ctypes.c_float, _vp]),
 }
@@ -119,7 +124,8 @@ def launch_count_reset():
     lib().ofl_launch_count_reset()
 
 
-PHASES = ("direction", "acc_tile_a", "acc_solve", "acc_tile_b", "acc_links", "strip_edge", "flats_stencils", "flats_label", "flats_sweeps", "breach_pits")
+PHASES = ("direction", "acc_tile_a", "acc_solve", "acc_tile_b", "acc_links", "strip_edge", "flats_stencils", "flats_label", "flats_sweeps", "breach_pits",
+          "basins_tile", "basins_solve", "basins_final")
 
 
 def phase_timing_enable(on=True):

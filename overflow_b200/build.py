@@ -15,7 +15,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(HERE), "include")
 LIB = os.path.join(HERE, "liboverflow_b200.so")
-SOURCES = ["runtime.cu", "direction.cu", "direction_generic.cu", "accumulation.cu", "flats.cu", "pits.cu", "synth.cu", "api.cu"]
+SOURCES = ["runtime.cu", "direction.cu", "direction_generic.cu", "accumulation.cu", "flats.cu", "pits.cu", "synth.cu", "basins.cu", "api.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-lineinfo", "-std=c++17",

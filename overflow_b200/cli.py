@@ -1,11 +1,13 @@
 """Command line interface -- mirror of the reference's src/overflow_cli.py for the D8 path.
 
 `flow-direction` keeps the reference's options, messages and exit codes (overflow_cli.py:54-84);
-`breach-single-cell-pits` likewise (overflow_cli.py:18-51); `flow-accumulation` and `flow-routing` (both steps, one
-pass over the device) are added with the same conventions (the reference snapshot has no such commands).
+`breach-single-cell-pits` likewise (overflow_cli.py:18-51); `flow-accumulation`, `flow-routing` (both steps, one
+pass over the device) and `basins` (drainage basins or watersheds of a flow-direction raster) are added with the same
+conventions (the reference snapshot has no such commands).
 """
 import click
 
+from .basins import basins, read_pour_points
 from .breach_single_cell_pits import breach_single_cell_pits
 from .constants import DEFAULT_CHUNK_SIZE
 from .flow_accumulation import flow_accumulation
@@ -76,6 +78,21 @@ def flow_routing_cli(input_file: str, flow_direction_file: str, flow_accumulatio
         flow_routing(input_file, flow_direction_file, flow_accumulation_file, chunk_size)
     except Exception as exc:
         print(f"flow_routing failed with the following exception: {str(exc)}")
+        raise click.Abort()
+
+
+@main.command(name="basins")
+@click.option("--input_file", help="path to the flow direction raster")
+@click.option("--output_file", help="path to the output file")
+@click.option("--chunk_size", help="chunk size", default=DEFAULT_CHUNK_SIZE)
+@click.option("--pour_points", default=None, help="text file with one row,col pour point per line: label watersheds "
+              "of these points instead of the basins of every outlet")
+def basins_cli(input_file: str, output_file: str, chunk_size: int, pour_points: str = None):
+    """Label every cell of a D8 flow direction raster with the outlet (or pour point) it drains to."""
+    try:
+        basins(input_file, output_file, chunk_size, read_pour_points(pour_points) if pour_points else None)
+    except Exception as exc:
+        print(f"basins failed with the following exception: {str(exc)}")
         raise click.Abort()
 
 

@@ -54,6 +54,11 @@ int launch_masked_flow_dirs(const int* flat_mask, const int* labels, uint8_t* fd
 size_t pits_workspace_bytes(int64_t rows, int64_t cols);
 int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, double nodata, int8_t* unsolved,
                        int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st);
+size_t basins_workspace_bytes(int64_t rows, int64_t cols);
+int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
+                  long long* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes, cudaStream_t st);
+int check_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
+                 const long long* labels, int64_t ld_labels, int64_t* n_bad, cudaStream_t st);
 int launch_synth(float* dem, int64_t rows, int64_t cols, int64_t ld, int64_t row0, int64_t total_rows, uint64_t seed,
                  int kind, float relief, int holes_permille, float nodata, cudaStream_t st);
 }  // namespace ofl
@@ -614,6 +619,58 @@ int ofl_strip_accum_final(const uint8_t* fdr_halo, int64_t rows, int64_t cols, i
   return strip_accum_final(fdr_halo, rows, cols, ld_fdr, has_above, has_below, reinterpret_cast<const long long*>(J_mine),
                            workspace, workspace_bytes, reinterpret_cast<long long*>(fac), ld_fac,
                            static_cast<cudaStream_t>(stream));
+}
+
+// ---------------------------------------------------------------- drainage basins (csrc/basins.cu)
+size_t ofl_basins_workspace_bytes(int64_t rows, int64_t cols) { return basins_workspace_bytes(rows, cols); }
+
+int ofl_label_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
+                        int64_t n_pour, int64_t* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes,
+                        int mem_kind, void* stream) {
+  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_pour >= 0, OFL_ERR_INVALID, "negative raster size or pour-point count");
+  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
+  if (rows == 0 || cols == 0) return OFL_OK;
+  OFL_REQUIRE(fdr != nullptr && labels != nullptr, OFL_ERR_INVALID, "null raster pointer");
+  OFL_REQUIRE(pour_points != nullptr || n_pour == 0, OFL_ERR_INVALID, "null pour-point list");
+  OFL_REQUIRE(ld_fdr >= cols && ld_labels >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
+  int rc = ensure_init();
+  if (rc != OFL_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (workspace == nullptr) {
+    workspace_bytes = basins_workspace_bytes(rows, cols);
+    if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
+  }
+  CallArg a[] = {{labels, rows, cols * 8, ld_labels * 8, COPY_OUT, 16},
+                 {fdr, rows, cols, ld_fdr, COPY_IN, 16},
+                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = launch_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(), n_pour,
+                       a[0].d<long long>(), a[0].ld(8), workspace, workspace_bytes, st);
+  return finish_call(rc, a, mem_kind, st);
+}
+
+int ofl_check_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
+                        int64_t n_pour, const int64_t* labels, int64_t ld_labels, int64_t* n_bad, int mem_kind,
+                        void* stream) {
+  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_pour >= 0 && n_bad != nullptr, OFL_ERR_INVALID, "bad argument");
+  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
+  *n_bad = 0;
+  if (rows == 0 || cols == 0) return OFL_OK;
+  OFL_REQUIRE(fdr != nullptr && labels != nullptr, OFL_ERR_INVALID, "null raster pointer");
+  OFL_REQUIRE(pour_points != nullptr || n_pour == 0, OFL_ERR_INVALID, "null pour-point list");
+  OFL_REQUIRE(ld_fdr >= cols && ld_labels >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
+  int rc = ensure_init();
+  if (rc != OFL_OK) return rc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  CallArg a[] = {{labels, rows, cols * 8, ld_labels * 8, COPY_IN, 8},
+                 {fdr, rows, cols, ld_fdr, COPY_IN, 16},
+                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1}};
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK)
+    rc = check_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(), n_pour,
+                      a[0].d<const long long>(), a[0].ld(8), n_bad, st);
+  return finish_call(rc, a, mem_kind, st);
 }
 
 int ofl_synth_dem_f32(float* dem, int64_t rows, int64_t cols, int64_t ld_dem, int64_t row0, int64_t total_rows,

@@ -40,7 +40,7 @@ bool debug_sync();  // OFL_DEBUG_SYNC=1: synchronise after every launch so fault
 // ---------------------------------------------------------------- per-phase CUDA-event timing
 // When enabled (ofl_phase_timing_enable), every phase is bracketed by cudaEventRecord on the
 // launching stream; ofl_phase_timing_read drains the pairs into per-phase sums.
-enum Phase { PHASE_DIRECTION = 0, PHASE_ACC_TILE_A, PHASE_ACC_SOLVE, PHASE_ACC_TILE_B, PHASE_ACC_LINKS, PHASE_STRIP_EDGE, PHASE_FLATS, PHASE_FLATS_LABEL, PHASE_FLATS_SWEEP, PHASE_PITS, PHASE_COUNT };
+enum Phase { PHASE_DIRECTION = 0, PHASE_ACC_TILE_A, PHASE_ACC_SOLVE, PHASE_ACC_TILE_B, PHASE_ACC_LINKS, PHASE_STRIP_EDGE, PHASE_FLATS, PHASE_FLATS_LABEL, PHASE_FLATS_SWEEP, PHASE_PITS, PHASE_BASINS_TILE, PHASE_BASINS_SOLVE, PHASE_BASINS_FINAL, PHASE_COUNT };
 struct PhaseScope {
   int phase;
   cudaStream_t st;

@@ -200,6 +200,81 @@ def check_accumulation(fdr: torch.Tensor, fac: torch.Tensor) -> int:
     return int(n_bad.value)
 
 
+def basins_workspace(rows, cols, device="cuda") -> torch.Tensor:
+    n = int(_native.lib().ofl_basins_workspace_bytes(rows, cols))
+    return torch.empty((n,), dtype=torch.uint8, device=device)
+
+
+def _pour_indices(pour_points, fdr):
+    """Row-major int64 cell indices on fdr's device of an (k, 2) array or tensor of (row, col); None when there are
+    no pour points.  A point outside the raster raises ValueError (for a tensor this reads one flag back)."""
+    if pour_points is None:
+        return None
+    rows, cols = fdr.shape
+    if isinstance(pour_points, torch.Tensor):
+        pp = pour_points.reshape(0, 2) if pour_points.numel() == 0 else pour_points
+        if pp.dim() != 2 or pp.shape[1] != 2 or pp.dtype.is_floating_point or pp.dtype.is_complex or pp.dtype == torch.bool:
+            raise ValueError("pour points must be an integer (k, 2) tensor of (row, col)")
+        pp = pp.to(device=fdr.device, dtype=torch.int64)
+        if bool(((pp[:, 0] < 0) | (pp[:, 0] >= rows) | (pp[:, 1] < 0) | (pp[:, 1] >= cols)).any()):
+            raise ValueError(f"pour point outside the {rows} x {cols} raster")
+        idx = (pp[:, 0] * cols + pp[:, 1]).contiguous()
+    else:
+        from .basins import pour_point_indices
+
+        idx = torch.from_numpy(pour_point_indices(pour_points, (rows, cols))).to(fdr.device)
+    return idx if idx.numel() else None
+
+
+def label_basins(fdr: torch.Tensor, *, pour_points=None, out=None, workspace=None) -> torch.Tensor:
+    """int64 basin labels of a uint8 CUDA flow-direction raster (overflow_b200.basins has the rules): the label of
+    the outlet, or with pour points ((k, 2) of (row, col)) of the first pour point, that each cell's path reaches.
+    Synchronises the stream (the call reports cycles and pour points outside the raster)."""
+    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or fdr.stride(1) != 1:
+        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
+    _init_for(fdr)
+    rows, cols = fdr.shape
+    idx = _pour_indices(pour_points, fdr)
+    if rows and cols and (fdr.stride(0) % 16 or fdr.data_ptr() % 16):
+        fdr = _pitched(rows, cols, torch.uint8, fdr.device, 16).copy_(fdr)  # dense odd widths: re-pitch
+    if out is None:
+        out = torch.empty((rows, cols), dtype=torch.int64, device=fdr.device)
+    else:
+        _check_raster("out", out, torch.int64, (rows, cols), fdr)
+    need = int(_native.lib().ofl_basins_workspace_bytes(rows, cols))
+    if workspace is None:
+        workspace = basins_workspace(rows, cols, fdr.device)
+    else:
+        _check_workspace("workspace", workspace, need, fdr)
+    _native.check(
+        _native.lib().ofl_label_basins_u8(
+            fdr.data_ptr(), rows, cols, fdr.stride(0), idx.data_ptr() if idx is not None else None,
+            0 if idx is None else idx.numel(), out.data_ptr(), out.stride(0), workspace.data_ptr(), workspace.numel(),
+            _native.OFL_MEM_DEVICE, _stream(fdr),
+        )
+    )
+    return out
+
+
+def check_basins(fdr: torch.Tensor, labels: torch.Tensor, pour_points=None) -> int:
+    """Number of cells breaking the basin labelling rule (0 proves the labels exact on an acyclic raster)."""
+    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or (fdr.shape[1] > 1 and fdr.stride(1) != 1):
+        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
+    _init_for(fdr)
+    rows, cols = fdr.shape
+    _check_raster("labels", labels, torch.int64, (rows, cols), fdr)
+    idx = _pour_indices(pour_points, fdr)
+    n_bad = ctypes.c_int64(0)
+    _native.check(
+        _native.lib().ofl_check_basins_u8(
+            fdr.data_ptr(), rows, cols, fdr.stride(0), idx.data_ptr() if idx is not None else None,
+            0 if idx is None else idx.numel(), labels.data_ptr(), labels.stride(0), ctypes.byref(n_bad),
+            _native.OFL_MEM_DEVICE, _stream(fdr),
+        )
+    )
+    return int(n_bad.value)
+
+
 def flats_workspace(rows, cols, device="cuda") -> torch.Tensor:
     n = int(_native.lib().ofl_flats_workspace_bytes(rows, cols))
     return torch.empty((max(n, 256),), dtype=torch.uint8, device=device)
