@@ -33,20 +33,17 @@
 // out-of-bounds NEIGHBOR_OFFSETS read); NODATA cells end at -9998 (:119-121,129-137).
 #include <atomic>
 #include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
+#include "tile_geometry.cuh"
 
 namespace ofl {
 
-constexpr int AT = 64;                 // tile side (cells)
-constexpr int AT_SHIFT = 6;
 constexpr int ACS_W = 96;              // code tile pitch: columns x0-16 .. x0+79 (TMA box inner = 96 B, 16-B aligned start)
 constexpr int ACS_H = AT + 2;          // rows y0-1 .. y0+64
 constexpr int ACS_X0 = 16;
 constexpr int ACS_Y0 = 1;
 constexpr uint32_t ACS_BYTES = ACS_W * ACS_H;
-constexpr int SLOTS = 4 * AT;          // perimeter slots per tile (top, bottom, left, right)
 constexpr int ACC_THREADS = 256;
 constexpr uint8_t CODE_OUTSIDE = 15;   // positions outside the raster (halo or partial tile)
 constexpr uint8_t CODE_HALO_LIVE = 14; // halo cell that is a live (non-NODATA) cell of the next tile
@@ -57,39 +54,6 @@ constexpr uint16_t KIND_TERM = 0;        // path ends inside the raster (pit, or
 constexpr uint16_t KIND_TILE_EXIT = 1;   // path continues in the next tile (succ >= 0)
 constexpr uint16_t KIND_RASTER_EXIT = 2; // path leaves the raster at the link cell
 constexpr uint16_t KIND_STRIP_EXIT = 3;  // path continues in the neighbouring row strip (resolved by the strip exchange)
-
-__device__ __forceinline__ int dir_dy(int code) { return ((0xA901 >> (2 * code)) & 3) - 1; }  // dy+1 = 1,0,0,0,1,2,2,2
-__device__ __forceinline__ int dir_dx(int code) { return ((0x901A >> (2 * code)) & 3) - 1; }  // dx+1 = 2,2,1,0,0,0,1,2
-
-__device__ __forceinline__ int slot_of(int y, int x, int h, int w) {
-  if (y == 0) return x;
-  if (y == h - 1) return AT + x;
-  if (x == 0) return 2 * AT + y;
-  if (x == w - 1) return 3 * AT + y;
-  return -1;
-}
-
-__device__ __forceinline__ bool cell_of_slot(int s, int h, int w, int& y, int& x) {
-  const int side = s >> AT_SHIFT, k = s & (AT - 1);
-  if (side == 0) {
-    y = 0;
-    x = k;
-    return k < w;
-  }
-  if (side == 1) {
-    y = h - 1;
-    x = k;
-    return k < w && h > 1;
-  }
-  if (side == 2) {
-    y = k;
-    x = 0;
-    return k > 0 && k < h - 1;
-  }
-  y = k;
-  x = w - 1;
-  return k > 0 && k < h - 1 && w > 1;
-}
 
 struct AccParams {
   int rows, cols;  // raster size
@@ -144,12 +108,6 @@ __device__ __forceinline__ void publish_slot(const AccParams& p, int tile, bool 
     base = __shfl_sync(0xffffffffu, base, 0);
     if (active) p.list0[(size_t)sidx * p.seg + base + __popc(bal & lt_mask)] = (int32_t)u;
   }
-}
-
-__device__ __forceinline__ int node_of_cell(int gy, int gx, const AccParams& p) {
-  const int ty = gy >> AT_SHIFT, tx = gx >> AT_SHIFT;
-  const int h = min(AT, p.rows - (ty << AT_SHIFT)), w = min(AT, p.cols - (tx << AT_SHIFT));
-  return (ty * p.ntx + tx) * SLOTS + slot_of(gy & (AT - 1), gx & (AT - 1), h, w);
 }
 
 // ---------------------------------------------------------------- in-tile frontier propagation
@@ -328,9 +286,8 @@ __global__ void __launch_bounds__(ACC_THREADS, OFL_ACC_MIN_CTAS) acc_tile_kernel
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int tile = blockIdx.x + p.tile_base;
-  const int ty = tile / p.ntx, tx = tile - ty * p.ntx;
-  const int y0 = ty << AT_SHIFT, x0 = tx << AT_SHIFT;
-  const int h = min(AT, p.rows - y0), w = min(AT, p.cols - x0);
+  int y0, x0, h, w;
+  tile_rect(tile, p.ntx, p.rows, p.cols, y0, x0, h, w);
 
   if (sb + SM::BYTES > 0x10000u) {  // the frontier queue holds shared addresses as 16-bit values
     if (tid == 0) atomicExch(p.err, 3);
@@ -536,7 +493,7 @@ __global__ void __launch_bounds__(ACC_THREADS, OFL_ACC_MIN_CTAS) acc_tile_kernel
       const int jn = (int)(an - a_word) >> 2;
       const int ny = jn / WP - 1, nx = jn - (ny + 1) * WP - WX0;
       if (!((uint32_t)ny < (uint32_t)AT && (uint32_t)nx < (uint32_t)AT) && (wn & 3u) == KIND_TILE_EXIT)
-        own_target = node_of_cell(y0 + ny, x0 + nx, p);
+        own_target = node_of_cell(y0 + ny, x0 + nx, p.rows, p.cols, p.ntx);
     }
     const bool follow = live && (target || edge);
     const uint32_t bal = __ballot_sync(0xffffffffu, follow);
@@ -688,7 +645,7 @@ __global__ void __launch_bounds__(ACC_THREADS, OFL_ACC_MIN_CTAS) acc_tile_kernel
           kind = (ny < h && nx < w) ? KIND_TERM : KIND_RASTER_EXIT;
         } else {
           kind = wn & 3u;  // the halo word says how the path continues
-          if (kind == KIND_TILE_EXIT) succ = node_of_cell(y0 + ny, x0 + nx, p);
+          if (kind == KIND_TILE_EXIT) succ = node_of_cell(y0 + ny, x0 + nx, p.rows, p.cols, p.ntx);
         }
       }
       const int ls = slot_of(cy, cx, h, w);
@@ -756,9 +713,8 @@ __device__ __forceinline__ bool final_tile(const AccParams& p, int tile, uint32_
   using SM = FinalSmem;
   const uint32_t a_cs0 = sb + SM::CS, a_lo = sb + SM::LO, a_hi = sb + SM::HI;  // a_cs0: code of cell (0,0), pitch AT
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int ty = tile / p.ntx, tx = tile - ty * p.ntx;
-  const int y0 = ty << AT_SHIFT, x0 = tx << AT_SHIFT;
-  const int h = min(AT, p.rows - y0), w = min(AT, p.cols - x0);
+  int y0, x0, h, w;
+  tile_rect(tile, p.ntx, p.rows, p.cols, y0, x0, h, w);
 
   if (tid == 0) sts32(sb + SM::CNT, 0);
   // tile-local counts with the codes on top (pass A: 12 + 4 bits per cell) and this thread's perimeter inflow
@@ -1041,38 +997,46 @@ __global__ void __launch_bounds__(256, 8) pj_solve_kernel(const PjArgs a) {
 }
 
 // ---------------------------------------------------------------- links for the raster perimeter
-// perimeter_indices order (flow_accumulation.py:40-51): every row's left then right cell, then for
-// columns 1..C-2 the top then the bottom cell.
+// Cell (r, c) at position k of perimeter_indices order (flow_accumulation.py:40-51): every row's left then right
+// cell, then for columns 1..C-2 the top then the bottom cell.
+__device__ __forceinline__ void perimeter_cell(int64_t k, int rows, int cols, int& r, int& c) {
+  if (k < 2 * (int64_t)rows) {
+    r = (int)(k >> 1);
+    c = (k & 1) ? cols - 1 : 0;
+  } else {
+    const int64_t kk = k - 2 * (int64_t)rows;
+    c = 1 + (int)(kk >> 1);
+    r = (kk & 1) ? rows - 1 : 0;
+  }
+}
+
+// Raster cell (row, column) where the in-tile path of perimeter node `root` ends: the exit slot of its link `lk`.
+__device__ __forceinline__ int2 link_exit_cell(int root, uint16_t lk, const AccParams& p) {
+  int y0, x0, h, w, y, x;
+  tile_rect(root / SLOTS, p.ntx, p.rows, p.cols, y0, x0, h, w);
+  cell_of_slot(lk & 0xFF, h, w, y, x);
+  return make_int2(y0 + y, x0 + x);
+}
+
 __global__ void links_kernel(const uint8_t* __restrict__ fdr, int64_t ld_fdr, const int32_t* __restrict__ root_ptr,
                              const uint16_t* __restrict__ link, AccParams p, long long* __restrict__ out, int64_t n) {
   for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
     int r, c;
-    if (k < 2 * (int64_t)p.rows) {
-      r = (int)(k >> 1);
-      c = (k & 1) ? p.cols - 1 : 0;
-    } else {
-      const int64_t kk = k - 2 * (int64_t)p.rows;
-      c = 1 + (int)(kk >> 1);
-      r = (kk & 1) ? p.rows - 1 : 0;
-    }
+    perimeter_cell(k, p.rows, p.cols, r, c);
     long long lr, lc;
     const int code = fdr[(int64_t)r * ld_fdr + c];
     if (code >= 8) {
       // reference quirk: the out-of-bounds offset read sends codes 8/9 "outside" on the first step
       lr = lc = OFL_LINK_EXTERNAL;
     } else {
-      const int u = node_of_cell(r, c, p);
+      const int u = node_of_cell(r, c, p.rows, p.cols, p.ntx);
       const int32_t pr = root_ptr[u];
       const int root = pr < 0 ? ~pr : u;
       const uint16_t lk = link[root];
       const int kind = lk >> 8;
       if (kind == KIND_RASTER_EXIT) {
-        const int tile = root / SLOTS;
-        const int ty = tile / p.ntx, tx = tile - ty * p.ntx;
-        const int h = min(AT, p.rows - (ty << AT_SHIFT)), w = min(AT, p.cols - (tx << AT_SHIFT));
-        int y, x;
-        cell_of_slot(lk & 0xFF, h, w, y, x);
-        const int er = (ty << AT_SHIFT) + y, ec = (tx << AT_SHIFT) + x;
+        const int2 e = link_exit_cell(root, lk, p);
+        const int er = e.x, ec = e.y;
         if (er == r && ec == c) {
           lr = lc = OFL_LINK_EXTERNAL;
         } else {
@@ -1099,15 +1063,8 @@ __global__ void perim_seed_kernel(const long long* __restrict__ inflow, AccParam
     const long long v = inflow[k];
     if (v == 0) continue;
     int r, c;
-    if (k < 2 * (int64_t)p.rows) {
-      r = (int)(k >> 1);
-      c = (k & 1) ? p.cols - 1 : 0;
-    } else {
-      const int64_t kk = k - 2 * (int64_t)p.rows;
-      c = 1 + (int)(kk >> 1);
-      r = (kk & 1) ? p.rows - 1 : 0;
-    }
-    atomicAdd(&S[node_of_cell(r, c, p)], (unsigned long long)v);
+    perimeter_cell(k, p.rows, p.cols, r, c);
+    atomicAdd(&S[node_of_cell(r, c, p.rows, p.cols, p.ntx)], (unsigned long long)v);
   }
 }
 
@@ -1151,8 +1108,6 @@ __global__ void check_kernel(const uint8_t* __restrict__ fdr, int64_t ld_fdr, co
 }
 
 // ---------------------------------------------------------------- host orchestration (device pointers)
-static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
-
 int64_t perimeter_count(int64_t rows, int64_t cols) {
   if (rows <= 0 || cols <= 0) return 0;
   const int64_t inner = cols - 2 > 0 ? cols - 2 : 0;
@@ -1174,38 +1129,20 @@ static int ensure_tile_attrs() {
   return OFL_OK;
 }
 
-static inline int grid_for(int64_t n, int per_sm) {
-  const int64_t want = (n + 255) / 256;
-  const int64_t cap = (int64_t)sm_count() * per_sm;
-  return (int)(want < cap ? (want > 0 ? want : 1) : cap);
-}
-
 static int pj_rounds_for(int64_t n) {
   int r = 2;
   while ((1ll << (r - 1)) < n && r < PJ_MAX_ROUNDS) ++r;
   return r + 1;  // one more round copies the last retirees' roots into both pointer buffers
 }
 
-// CTAs of pj_solve_kernel that are resident at once on the current device (the kernel is launched
-// cooperatively with one CTA per segment).
-static int pj_max_blocks() {
-  static std::atomic<int> gen{-1}, cached{0};
-  if (gen.load() != device_generation() || cached.load() == 0) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pj_solve_kernel, 256, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-    if (per_sm > 8) per_sm = 8;
-    cached.store(per_sm * sm_count());
-    gen.store(device_generation());
-  }
-  return cached.load();
-}
 constexpr int PJ_MAX_BLOCKS = 8 * 256;  // counts0 holds this many segments (8 CTAs on each of up to 256 SMs)
 
 static PjSeg pj_segments(int64_t n) {
   PjSeg g;
   g.n = n;
   int64_t blocks = (n + 2047) / 2048;  // at least 2048 nodes per segment
-  int64_t cap = pj_max_blocks();
+  // the solve is launched cooperatively with one CTA per segment: every segment's CTA must be resident
+  int64_t cap = resident_ctas(reinterpret_cast<const void*>(pj_solve_kernel), 256, 8);
   if (cap > PJ_MAX_BLOCKS) cap = PJ_MAX_BLOCKS;
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
@@ -1249,29 +1186,25 @@ static Graph carve_graph(void* base, int64_t n, GraphKind kind) {
   Graph g;
   g.kind = kind;
   g.n = n;
-  size_t o = 0;
-  auto take = [&](auto& ptr, size_t bytes) {
-    ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(reinterpret_cast<uintptr_t>(base) + o);
-    o = align_up(o + bytes, 256);
-  };
+  Carver w(base);
   const size_t nodes = (size_t)n;
   const bool tiled = kind != GraphKind::BOUNDARY;
-  take(g.succ, nodes * 4);
-  take(g.ptr_a, nodes * 4);
-  take(g.ptr_b, nodes * 4);
-  take(g.lists, (nodes + 64 * (size_t)PJ_MAX_BLOCKS) * 8);
-  take(g.S, nodes * 8);
+  w.take(g.succ, nodes * 4);
+  w.take(g.ptr_a, nodes * 4);
+  w.take(g.ptr_b, nodes * 4);
+  w.take(g.lists, (nodes + 64 * (size_t)PJ_MAX_BLOCKS) * 8);
+  w.take(g.S, nodes * 8);
   g.S2 = g.S;
-  if (kind == GraphKind::STRIP) take(g.S2, nodes * 8);
-  take(g.d0, nodes * 8);
-  take(g.d1, nodes * 8);
-  take(g.link, nodes * 2);
-  take(g.counts, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int));
-  take(g.sync, PJ_SYNC_WORDS * sizeof(unsigned));
-  take(g.flags, GRAPH_FLAG_WORDS * sizeof(int));
-  take(g.L, tiled ? nodes / SLOTS * AT * AT * sizeof(uint16_t) : 0);
-  take(g.wide, tiled ? (nodes / SLOTS + 1) * sizeof(int) : 0);
-  g.bytes = o;
+  if (kind == GraphKind::STRIP) w.take(g.S2, nodes * 8);
+  w.take(g.d0, nodes * 8);
+  w.take(g.d1, nodes * 8);
+  w.take(g.link, nodes * 2);
+  w.take(g.counts, 2 * (size_t)PJ_MAX_BLOCKS * sizeof(int));
+  w.take(g.sync, PJ_SYNC_WORDS * sizeof(unsigned));
+  w.take(g.flags, GRAPH_FLAG_WORDS * sizeof(int));
+  w.take(g.L, tiled ? nodes / SLOTS * AT * AT * sizeof(uint16_t) : 0);
+  w.take(g.wide, tiled ? (nodes / SLOTS + 1) * sizeof(int) : 0);
+  g.bytes = w.bytes;
   return g;
 }
 
@@ -1327,7 +1260,7 @@ static int check_flags(const Graph& g, cudaStream_t st) {
 }
 
 static inline int64_t node_count(int64_t rows, int64_t cols) {
-  return ((rows + AT - 1) / AT) * ((cols + AT - 1) / AT) * SLOTS;
+  return tiles_along(rows) * tiles_along(cols) * SLOTS;
 }
 
 size_t accumulation_workspace_bytes(int64_t rows, int64_t cols) {
@@ -1363,8 +1296,8 @@ static int acc_setup(AccCtx& C, const uint8_t* fdr, int64_t rows, int64_t cols, 
   AccParams& p = C.p;
   p.rows = (int)rows;
   p.cols = (int)cols;
-  p.nty = (int)((rows + AT - 1) / AT);
-  p.ntx = (int)((cols + AT - 1) / AT);
+  p.nty = (int)tiles_along(rows);
+  p.ntx = (int)tiles_along(cols);
   p.succ = g.succ;
   p.link = g.link;
   p.S = g.S;
@@ -1519,17 +1452,13 @@ __global__ void strip_boundary_extract_kernel(const uint8_t* __restrict__ fdr, i
     floc[k] = fac[(int64_t)r * ld_fac + c];
     int32_t sl = -1;
     if (code < 8) {
-      const int u = node_of_cell(r, c, p);
+      const int u = node_of_cell(r, c, p.rows, p.cols, p.ntx);
       const int32_t pr = root_ptr[u];
       const int root = pr < 0 ? ~pr : u;
       const uint16_t lk = link[root];
       if ((lk >> 8) == KIND_STRIP_EXIT) {
-        const int tile = root / SLOTS;
-        const int ty = tile / p.ntx, tx = tile - ty * p.ntx;
-        const int h = min(AT, p.rows - (ty << AT_SHIFT)), w = min(AT, p.cols - (tx << AT_SHIFT));
-        int y, x;
-        cell_of_slot(lk & 0xFF, h, w, y, x);
-        const int er = (ty << AT_SHIFT) + y, ec = (tx << AT_SHIFT) + x;
+        const int2 e = link_exit_cell(root, lk, p);
+        const int er = e.x, ec = e.y;
         sl = ((er == 0 ? 0 : 1) << 30) | ec;
       }
     }
@@ -1594,7 +1523,7 @@ __global__ void strip_seed_chase_kernel(const long long* __restrict__ J, AccPara
     const long long j = J[k];
     if (j == 0) continue;
     const int t = (int)(k / p.cols), c = (int)(k - (int64_t)t * p.cols);
-    int u = node_of_cell(t ? p.rows - 1 : 0, c, p);
+    int u = node_of_cell(t ? p.rows - 1 : 0, c, p.rows, p.cols, p.ntx);
     if (DRY) {
       int steps = 0;
       while ((u = succ[u]) >= 0)
@@ -1625,7 +1554,7 @@ __global__ void strip_seed_set_kernel_if(const long long* __restrict__ J, AccPar
   for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) {
     const int t = (int)(k / p.cols), c = (int)(k - (int64_t)t * p.cols);
     const long long j = J[k];
-    if (j != 0) S2[node_of_cell(t ? p.rows - 1 : 0, c, p)] = (unsigned long long)j;
+    if (j != 0) S2[node_of_cell(t ? p.rows - 1 : 0, c, p.rows, p.cols, p.ntx)] = (unsigned long long)j;
   }
 }
 

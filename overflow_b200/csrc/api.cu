@@ -65,8 +65,6 @@ int launch_synth(float* dem, int64_t rows, int64_t cols, int64_t ld, int64_t row
 
 using namespace ofl;
 
-static inline int64_t round_up(int64_t v, int64_t a) { return (v + a - 1) / a * a; }
-
 // ---------------------------------------------------------------- host rasters: banded pipeline
 // A host DEM goes to the device in row bands on its own stream; the stencil of band b runs as soon as
 // the first row of band b+1 has arrived, and its codes return to the host on a third stream, so the
@@ -196,7 +194,7 @@ int stage_in(CallArg (&a)[N], int mem_kind, cudaStream_t st) {
       x.dev_pitch = x.pitch;
       continue;
     }
-    x.dev_pitch = round_up(x.row_bytes, x.align);
+    x.dev_pitch = align_up(x.row_bytes, x.align);
     int rc = scratch_get(SCRATCH_STAGE0 + i, (size_t)(x.rows * x.dev_pitch), &x.dev);
     if (rc != OFL_OK) return rc;
     if ((x.copy & COPY_IN) && x.caller && x.rows * x.row_bytes > 0)

@@ -22,22 +22,18 @@
 // HBM traffic per cell: tile pass 1 B codes + 2 B terminals, final pass 2 B terminals + 8 B labels, the solve
 // ~0.5 B; against 9 B/cell compulsory (codes in, labels out).
 #include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
+#include "tile_geometry.cuh"
 
 namespace ofl {
 namespace {
 
-constexpr int BT = 64;  // tile side (cells)
-constexpr int BT_SHIFT = 6;
-constexpr int BT_CELLS = BT * BT;
-constexpr int B_SLOTS = 4 * BT;   // perimeter nodes per tile (top, bottom, left, right), as in the accumulation
 constexpr int B_THREADS = 256;
-constexpr int B_PER_THREAD = BT_CELLS / B_THREADS;  // 16 cells: rows (tid >> 6) + 4k, column tid & 63
-constexpr int CS_W = BT + 4;                        // code tile pitch: columns -1 .. 64 at 1 .. 66
-constexpr int CS_H = BT + 2;                        // rows -1 .. 64
-constexpr int TILE_ROUNDS = 13;                     // ceil(log2 4096) + 1
+constexpr int B_PER_THREAD = AT * AT / B_THREADS;   // 16 cells: rows (tid >> 6) + 4k, column tid & 63
+constexpr int CS_W = AT + 4;                        // code tile pitch: columns -1 .. 64 at 1 .. 66
+constexpr int CS_H = AT + 2;                        // rows -1 .. 64
+constexpr int TILE_ROUNDS = 2 * AT_SHIFT + 1;       // ceil(log2(AT * AT)) + 1
 constexpr uint16_t P_TERM = 0x8000;                 // pointer flag: the cell pointed at is a terminal
 constexpr uint16_t T_ZERO = 0xFFFF;                 // stored terminal: the cell's label is 0
 constexpr unsigned long long R_RESOLVED = 1ull << 63;  // node record: the low bits are the final label
@@ -52,40 +48,10 @@ constexpr uint8_t K_EXIT = 3;   // the cell's step leaves the tile into a data c
 enum { BF_TILE = 0, BF_POUR = 1, BF_WORDS = 4 };
 constexpr int MAX_ROUNDS = 40;
 
-__device__ __forceinline__ int b_dy(int code) { return ((0xA901 >> (2 * code)) & 3) - 1; }  // dy+1 = 1,0,0,0,1,2,2,2
-__device__ __forceinline__ int b_dx(int code) { return ((0x901A >> (2 * code)) & 3) - 1; }  // dx+1 = 2,2,1,0,0,0,1,2
-
-// Perimeter slot of tile cell (y, x) in an h x w tile, -1 inside (accumulation.cu slot_of).
-__device__ __forceinline__ int b_slot(int y, int x, int h, int w) {
-  if (y == 0) return x;
-  if (y == h - 1) return BT + x;
-  if (x == 0) return 2 * BT + y;
-  if (x == w - 1) return 3 * BT + y;
-  return -1;
-}
-
-// Tile cell of slot s; false when the slot names no cell of an h x w tile (accumulation.cu cell_of_slot).
-__device__ __forceinline__ bool b_cell_of_slot(int s, int h, int w, int& y, int& x) {
-  const int side = s >> BT_SHIFT, k = s & (BT - 1);
-  if (side == 0) {
-    y = 0;
-    x = k;
-    return k < w;
-  }
-  if (side == 1) {
-    y = h - 1;
-    x = k;
-    return k < w && h > 1;
-  }
-  if (side == 2) {
-    y = k;
-    x = 0;
-    return k > 0 && k < h - 1;
-  }
-  y = k;
-  x = w - 1;
-  return k > 0 && k < h - 1 && w > 1;
-}
+static_assert(B_PER_THREAD * B_THREADS == AT * AT, "the threads of a CTA cover its tile");
+static_assert(B_PER_THREAD == 16, "the tile pass loads one 16-byte piece of codes per thread");
+static_assert(B_THREADS == SLOTS, "one thread per perimeter slot writes and reads the node records");
+static_assert(AT * AT <= 0x8000, "an in-tile pointer holds a cell in 15 bits, P_TERM in bit 15");
 
 struct BasinParams {
   const uint8_t* fdr;
@@ -94,29 +60,23 @@ struct BasinParams {
   int64_t ld_labels;
   int rows, cols;
   int ntx, nty;
-  unsigned long long* rec;  // [ntiles * B_SLOTS] perimeter node records
+  unsigned long long* rec;  // [ntiles * SLOTS] perimeter node records
   uint16_t* term;           // [ntiles][64 * 64] in-tile terminal of each cell (T_ZERO: label 0)
   const uint32_t* pour;     // pour-point bit per cell (raster order), null without pour points
   int* flags;               // [BF_WORDS]
   int vec_store;            // labels rows are 16-byte aligned: the final pass stores two labels at once
 };
 
-__device__ __forceinline__ int64_t node_of(int gy, int gx, const BasinParams& p) {
-  const int ty = gy >> BT_SHIFT, tx = gx >> BT_SHIFT;
-  const int h = min(BT, p.rows - (ty << BT_SHIFT)), w = min(BT, p.cols - (tx << BT_SHIFT));
-  return ((int64_t)ty * p.ntx + tx) * B_SLOTS + b_slot(gy & (BT - 1), gx & (BT - 1), h, w);
-}
-
 __device__ __forceinline__ bool pour_bit(const uint32_t* pour, int64_t i) { return (pour[i >> 5] >> (i & 31)) & 1u; }
 
 __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParams p) {
   __shared__ __align__(16) uint8_t codes[CS_H * CS_W];  // cell (y, x) at (y + 1) * CS_W + x + 1; 9 outside the raster
-  __shared__ uint16_t ptr[BT_CELLS];
-  __shared__ uint8_t kind[BT_CELLS];
+  __shared__ uint16_t ptr[AT * AT];
+  __shared__ uint8_t kind[AT * AT];
   const int tid = threadIdx.x;
   const int tile = blockIdx.x;
-  const int ty0 = (tile / p.ntx) << BT_SHIFT, tx0 = (tile % p.ntx) << BT_SHIFT;
-  const int h = min(BT, p.rows - ty0), w = min(BT, p.cols - tx0);
+  int ty0, tx0, h, w;
+  tile_rect(tile, p.ntx, p.rows, p.cols, ty0, tx0, h, w);
 
   // codes: the 64 x 64 body in 16-byte pieces (a piece never runs past the row pitch: ld_fdr % 16 == 0), the ring
   // byte by byte
@@ -129,10 +89,10 @@ __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParam
 #pragma unroll
     for (int i = 0; i < 16; ++i) codes[(y + 1) * CS_W + x + 1 + i] = (x + i < w) ? b[i] : (uint8_t)OFL_DIR_NODATA;
   }
-  for (int i = tid; i < 4 * (BT + 2); i += B_THREADS) {
-    const int side = i / (BT + 2), k = i % (BT + 2) - 1;  // k = -1 .. 64
-    const int y = side == 0 ? -1 : side == 1 ? BT : k, x = side < 2 ? k : (side == 2 ? -1 : BT);
-    if (side >= 2 && (k < 0 || k >= BT)) continue;  // the corners come with the top and bottom rows
+  for (int i = tid; i < 4 * (AT + 2); i += B_THREADS) {
+    const int side = i / (AT + 2), k = i % (AT + 2) - 1;  // k = -1 .. 64
+    const int y = side == 0 ? -1 : side == 1 ? AT : k, x = side < 2 ? k : (side == 2 ? -1 : AT);
+    if (side >= 2 && (k < 0 || k >= AT)) continue;  // the corners come with the top and bottom rows
     const int gy = ty0 + y, gx = tx0 + x;
     const bool in = gy >= 0 && gy < p.rows && gx >= 0 && gx < p.cols;
     codes[(y + 1) * CS_W + x + 1] = in ? p.fdr[(int64_t)gy * p.ld_fdr + gx] : (uint8_t)OFL_DIR_NODATA;
@@ -143,7 +103,7 @@ __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParam
   uint16_t nxt[B_PER_THREAD];
 #pragma unroll
   for (int k = 0; k < B_PER_THREAD; ++k) {
-    const int c = tid + k * B_THREADS, y = c >> BT_SHIFT, x = c & (BT - 1);
+    const int c = tid + k * B_THREADS, y = c >> AT_SHIFT, x = c & (AT - 1);
     const int code = codes[(y + 1) * CS_W + x + 1];
     uint8_t kd;
     nxt[k] = (uint16_t)c;
@@ -154,14 +114,14 @@ __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParam
     } else if (code > 7) {
       kd = p.pour ? K_ZERO : K_ROOT;
     } else {
-      const int ny = y + b_dy(code), nx = x + b_dx(code);
+      const int ny = y + dir_dy(code), nx = x + dir_dx(code);
       if (codes[(ny + 1) * CS_W + nx + 1] == OFL_DIR_NODATA) {  // NODATA or outside the raster
         kd = p.pour ? K_ZERO : K_ROOT;
-      } else if (ny < 0 || ny >= BT || nx < 0 || nx >= BT) {
+      } else if (ny < 0 || ny >= AT || nx < 0 || nx >= AT) {
         kd = K_EXIT;
       } else {
         kd = K_PATH;
-        nxt[k] = (uint16_t)((ny << BT_SHIFT) | nx);
+        nxt[k] = (uint16_t)((ny << AT_SHIFT) | nx);
       }
     }
     kind[c] = kd;
@@ -200,10 +160,10 @@ __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParam
   }
 
   // terminals of the cells
-  uint16_t* term = p.term + (size_t)tile * BT_CELLS;
+  uint16_t* term = p.term + (size_t)tile * (AT * AT);
 #pragma unroll
   for (int k = 0; k < B_PER_THREAD; ++k) {
-    const int t = nxt[k] & (BT_CELLS - 1);
+    const int t = nxt[k] & (AT * AT - 1);
     term[tid + k * B_THREADS] = kind[t] == K_ZERO ? T_ZERO : (uint16_t)t;
   }
 
@@ -212,18 +172,18 @@ __global__ void __launch_bounds__(B_THREADS) basins_tile_kernel(const BasinParam
     const int s = tid;
     int y, x;
     unsigned long long r = R_RESOLVED;
-    if (b_cell_of_slot(s, h, w, y, x)) {
-      const int t = ptr[(y << BT_SHIFT) | x] & (BT_CELLS - 1);
-      const int tyy = t >> BT_SHIFT, txx = t & (BT - 1);
+    if (cell_of_slot(s, h, w, y, x)) {
+      const int t = ptr[(y << AT_SHIFT) | x] & (AT * AT - 1);
+      const int tyy = t >> AT_SHIFT, txx = t & (AT - 1);
       const uint8_t kd = kind[t];
       if (kd == K_ROOT) {
         r = R_RESOLVED | (unsigned long long)((int64_t)(ty0 + tyy) * p.cols + tx0 + txx + 1);
       } else if (kd == K_EXIT) {
         const int code = codes[(tyy + 1) * CS_W + txx + 1];
-        r = (unsigned long long)node_of(ty0 + tyy + b_dy(code), tx0 + txx + b_dx(code), p);
+        r = (unsigned long long)node_of_cell(ty0 + tyy + dir_dy(code), tx0 + txx + dir_dx(code), p.rows, p.cols, p.ntx);
       }
     }
-    p.rec[(size_t)tile * B_SLOTS + s] = r;
+    p.rec[(size_t)tile * SLOTS + s] = r;
   }
 }
 
@@ -274,18 +234,18 @@ __global__ void __launch_bounds__(256) basins_solve_kernel(unsigned long long* _
 }
 
 __global__ void __launch_bounds__(B_THREADS) basins_final_kernel(const BasinParams p) {
-  __shared__ long long srec[B_SLOTS];
+  __shared__ long long srec[SLOTS];
   const int tid = threadIdx.x;
   const int tile = blockIdx.x;
-  const int ty0 = (tile / p.ntx) << BT_SHIFT, tx0 = (tile % p.ntx) << BT_SHIFT;
-  const int h = min(BT, p.rows - ty0), w = min(BT, p.cols - tx0);
-  srec[tid] = (long long)(__ldcg(&p.rec[(size_t)tile * B_SLOTS + tid]) & ~R_RESOLVED);
+  int ty0, tx0, h, w;
+  tile_rect(tile, p.ntx, p.rows, p.cols, ty0, tx0, h, w);
+  srec[tid] = (long long)(__ldcg(&p.rec[(size_t)tile * SLOTS + tid]) & ~R_RESOLVED);
   __syncthreads();
-  const uint32_t* term = reinterpret_cast<const uint32_t*>(p.term + (size_t)tile * BT_CELLS);
+  const uint32_t* term = reinterpret_cast<const uint32_t*>(p.term + (size_t)tile * (AT * AT));
 #pragma unroll 4
-  for (int k = 0; k < BT_CELLS / 2 / B_THREADS; ++k) {
+  for (int k = 0; k < AT * AT / 2 / B_THREADS; ++k) {
     const int pair = tid + k * B_THREADS;
-    const int y = pair >> (BT_SHIFT - 1), x = (pair & (BT / 2 - 1)) * 2;
+    const int y = pair >> (AT_SHIFT - 1), x = (pair & (AT / 2 - 1)) * 2;
     if (y >= h || x >= w) continue;
     const uint32_t tt = __ldcs(&term[pair]);
     long long lab[2];
@@ -295,8 +255,8 @@ __global__ void __launch_bounds__(B_THREADS) basins_final_kernel(const BasinPara
       if (t == T_ZERO) {
         lab[j] = 0;
       } else {
-        const int yy = (int)(t >> BT_SHIFT), xx = (int)(t & (BT - 1));
-        const int s = b_slot(yy, xx, h, w);
+        const int yy = (int)(t >> AT_SHIFT), xx = (int)(t & (AT - 1));
+        const int s = slot_of(yy, xx, h, w);
         lab[j] = s >= 0 ? srec[s] : (long long)(ty0 + yy) * p.cols + tx0 + xx + 1;
       }
     }
@@ -330,8 +290,8 @@ __global__ void basins_check_kernel(const uint8_t* __restrict__ fdr, int64_t ld_
       bool has_succ = false;
       int nr = 0, nc = 0;
       if (code <= 7) {
-        nr = r + b_dy(code);
-        nc = c + b_dx(code);
+        nr = r + dir_dy(code);
+        nc = c + dir_dx(code);
         has_succ = nr >= 0 && nr < rows && nc >= 0 && nc < cols && fdr[(int64_t)nr * ld_fdr + nc] != OFL_DIR_NODATA;
       }
       if (has_succ && !is_pour) {
@@ -347,8 +307,6 @@ __global__ void basins_check_kernel(const uint8_t* __restrict__ fdr, int64_t ld_
 }
 
 // ---------------------------------------------------------------- host orchestration (device pointers)
-inline size_t b_align(size_t v) { return (v + 255) / 256 * 256; }
-
 struct BasinLayout {
   unsigned long long* rec;
   uint16_t* term;
@@ -361,29 +319,18 @@ struct BasinLayout {
 
 BasinLayout carve(void* base, int64_t rows, int64_t cols) {
   BasinLayout L;
-  const size_t ntiles = (size_t)((rows + BT - 1) / BT) * (size_t)((cols + BT - 1) / BT);
-  const size_t nodes = ntiles * B_SLOTS;
-  size_t o = 0;
-  auto take = [&](auto*& ptr, size_t bytes) {
-    ptr = reinterpret_cast<std::remove_reference_t<decltype(ptr)>>(reinterpret_cast<uintptr_t>(base) + o);
-    o = b_align(o + bytes);
-  };
-  take(L.rec, nodes * 8);
-  take(L.term, ntiles * BT_CELLS * 2);
-  take(L.list_a, nodes * 4);
-  take(L.list_b, nodes * 4);
-  L.counts = reinterpret_cast<int*>(reinterpret_cast<uintptr_t>(base) + o);
+  const size_t ntiles = (size_t)tiles_along(rows) * (size_t)tiles_along(cols);
+  const size_t nodes = ntiles * SLOTS;
+  Carver w(base);
+  w.take(L.rec, nodes * 8);
+  w.take(L.term, ntiles * (AT * AT) * 2);
+  w.take(L.list_a, nodes * 4);
+  w.take(L.list_b, nodes * 4);
+  w.take(L.counts, (MAX_ROUNDS + BF_WORDS) * sizeof(int));
   L.flags = L.counts + MAX_ROUNDS;
-  o = b_align(o + (MAX_ROUNDS + BF_WORDS) * sizeof(int));
-  take(L.pour, ((size_t)rows * (size_t)cols + 31) / 32 * 4);
-  L.bytes = o;
+  w.take(L.pour, ((size_t)rows * (size_t)cols + 31) / 32 * 4);
+  L.bytes = w.bytes;
   return L;
-}
-
-int grid_cap(int64_t n, int per_sm) {
-  const int64_t want = (n + 255) / 256;
-  const int64_t cap = (int64_t)sm_count() * per_sm;
-  return (int)(want < cap ? (want > 0 ? want : 1) : cap);
 }
 
 // ceil(log2 nodes) + 2 rounds: a longer chain of perimeter nodes than there are nodes is a cycle
@@ -396,7 +343,7 @@ int solve_rounds(int64_t nodes) {
 // Clear the pour mask and scatter the pour points into it (n_pour > 0).
 int scatter_pour(const long long* pour, int64_t n_pour, int64_t n_cells, uint32_t* mask, int* flags, cudaStream_t st) {
   OFL_CUDA(cudaMemsetAsync(mask, 0, (size_t)(n_cells + 31) / 32 * 4, st));
-  basins_pour_kernel<<<grid_cap(n_pour, 4), 256, 0, st>>>(pour, n_pour, n_cells, mask, flags);
+  basins_pour_kernel<<<grid_for(n_pour, 4), 256, 0, st>>>(pour, n_pour, n_cells, mask, flags);
   OFL_CHECK_LAUNCH();
   return OFL_OK;
 }
@@ -416,8 +363,8 @@ int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr
               "fdr must be 16-byte aligned with ld_fdr %% 16 == 0 (ld_fdr=%lld)", (long long)ld_fdr);
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(labels) & 7) == 0 && ld_labels >= cols, OFL_ERR_ALIGNMENT,
               "labels must be 8-byte aligned");
-  const int ntx = (int)((cols + BT - 1) / BT), nty = (int)((rows + BT - 1) / BT);
-  const int64_t ntiles = (int64_t)ntx * nty, nodes = ntiles * B_SLOTS;
+  const int ntx = (int)tiles_along(cols), nty = (int)tiles_along(rows);
+  const int64_t ntiles = (int64_t)ntx * nty, nodes = ntiles * SLOTS;
   OFL_REQUIRE(nodes < (1ll << 31), OFL_ERR_INVALID, "raster too large for 32-bit perimeter node ids");
   const BasinLayout L = carve(workspace, rows, cols);
   OFL_REQUIRE(workspace != nullptr && workspace_bytes >= L.bytes, OFL_ERR_WORKSPACE,
@@ -449,7 +396,7 @@ int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr
   }
   {
     PhaseScope ps(PHASE_BASINS_SOLVE, st);
-    const int grid = grid_cap(nodes, 8);
+    const int grid = grid_for(nodes, 8);
     for (int r = 0; r < rounds; ++r) {
       int32_t* lists[2] = {L.list_a, L.list_b};
       basins_solve_kernel<<<grid, 256, 0, st>>>(L.rec, nodes, r ? lists[(r - 1) & 1] : nullptr,
@@ -489,7 +436,7 @@ int check_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr,
     if (rc == OFL_OK) rc = scatter_pour(pour, n_pour, rows * cols, mask, flags, st);
     if (rc != OFL_OK) return rc;
   }
-  basins_check_kernel<<<grid_cap(rows * cols, 16), 256, 0, st>>>(fdr, ld_fdr, labels, ld_labels, (int)rows, (int)cols,
+  basins_check_kernel<<<grid_for(rows * cols, 16), 256, 0, st>>>(fdr, ld_fdr, labels, ld_labels, (int)rows, (int)cols,
                                                                   mask, d_bad);
   OFL_CHECK_LAUNCH();
   struct {

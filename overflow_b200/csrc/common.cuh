@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_runtime.h>
+#include <limits.h>
 #include <stdint.h>
 #include <stdio.h>
 
@@ -66,13 +67,44 @@ int scratch_get(int slot, size_t bytes, void** out);
 // Pinned host scratch (slot-indexed) for small read-backs.
 int pinned_get(size_t bytes, void** out);
 
+// ---------------------------------------------------------------- launch sizes and workspace layout (host)
+inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+
+// Grid of a grid-stride kernel with 256 threads per CTA over n items: a CTA per 256 items, at most per_sm CTAs per SM.
+inline int grid_for(int64_t n, int per_sm) {
+  const int64_t want = (n + 255) / 256;
+  const int64_t cap = (int64_t)sm_count() * per_sm;
+  return (int)(want < cap ? (want > 0 ? want : 1) : cap);
+}
+
+// CTAs of a cooperatively launched kernel (`threads` per CTA, no dynamic shared memory) that are resident at once on
+// the current device, at most max_per_sm on each SM.  Cached per kernel and device_generation().
+int resident_ctas(const void* kernel, int threads, int max_per_sm = INT_MAX);
+
+// Cuts a workspace at `base` into buffers, in the order they are taken, each 256-byte aligned.  With a null base only
+// `bytes`, the size of the workspace, is meaningful.
+struct Carver {
+  uintptr_t base;
+  size_t bytes = 0;
+  explicit Carver(void* base_) : base(reinterpret_cast<uintptr_t>(base_)) {}
+  template <class T>
+  void take(T*& ptr, size_t n_bytes) {
+    ptr = reinterpret_cast<T*>(base + bytes);
+    bytes = align_up(bytes + n_bytes, 256);
+  }
+};
+
 // ---------------------------------------------------------------- TMA tensor maps (host)
 // 2-D row-major tensor, element size `esz`, `cols` x `rows`, row pitch in bytes, box_w x box_h tile.
 int make_tensor_map_2d(CUtensorMap* tm, const void* base, int esz, uint64_t cols, uint64_t rows,
                        uint64_t pitch_bytes, uint32_t box_w, uint32_t box_h, int l2_promotion_bytes = 128);
 
-// ---------------------------------------------------------------- device-side PTX wrappers
+// ---------------------------------------------------------------- device-side helpers and PTX wrappers
 #ifdef __CUDACC__
+// Step of D8 code 0..7 (E, NE, N, NW, W, SW, S, SE).
+__device__ __forceinline__ int dir_dy(int code) { return ((0xA901 >> (2 * code)) & 3) - 1; }  // dy+1 = 1,0,0,0,1,2,2,2
+__device__ __forceinline__ int dir_dx(int code) { return ((0x901A >> (2 * code)) & 3) - 1; }  // dx+1 = 2,2,1,0,0,0,1,2
+
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }

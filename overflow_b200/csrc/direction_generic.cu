@@ -75,7 +75,7 @@ __global__ void direction_generic_kernel(const GenParams p) {
       bool any_pos = false;
 #pragma unroll
       for (int k = 0; k < 8; ++k) {
-        const int dy = ((0xA901 >> (2 * k)) & 3) - 1, dx = ((0x901A >> (2 * k)) & 3) - 1;
+        const int dy = dir_dy(k), dx = dir_dx(k);
         const T v = at(iy + dy, x + dx);
         double s;
         if (ElemOf<KIND>::widen(v) == p.nodata)

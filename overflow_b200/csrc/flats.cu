@@ -23,7 +23,6 @@
 #include <stdio.h>
 #include <stdlib.h>
 
-#include <atomic>
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -1149,46 +1148,32 @@ struct FlatsWork {
   uint8_t* edges;
   unsigned* cnt;
   int* tiles;   // three tile lists and the tile stamps of the sweeps
+  size_t bytes;  // size of the workspace
 };
-
-size_t flats_align(size_t v) { return (v + 255) / 256 * 256; }
 
 int64_t sweep_tiles(int64_t rows, int64_t cols) { return ((rows + FT - 1) / FT) * ((cols + FT - 1) / FT); }
 
-size_t flats_bytes(int64_t rows, int64_t cols) {
-  const int64_t n = rows * cols;
-  return 4 * flats_align((size_t)n * sizeof(int)) + flats_align((size_t)n) + flats_align(CNT_SLOTS * sizeof(unsigned)) +
-         flats_align((size_t)sweep_tiles(rows, cols) * 5 * sizeof(int));
+// Cuts the workspace at `base` into its buffers; with a null base only `bytes` is meaningful.
+FlatsWork flats_layout(void* base, int64_t rows, int64_t cols) {
+  const size_t n = (size_t)(rows * cols);
+  FlatsWork w;
+  Carver c(base);
+  c.take(w.parent, n * sizeof(int));
+  c.take(w.q0, n * sizeof(int));
+  c.take(w.q1, n * sizeof(int));
+  c.take(w.open, n * sizeof(int));
+  c.take(w.edges, n);
+  c.take(w.cnt, CNT_SLOTS * sizeof(unsigned));
+  c.take(w.tiles, (size_t)sweep_tiles(rows, cols) * 5 * sizeof(int));
+  w.bytes = c.bytes;
+  return w;
 }
 
 int carve(void* workspace, size_t workspace_bytes, int64_t rows, int64_t cols, FlatsWork* w) {
-  const int64_t n = rows * cols;
-  const size_t a = flats_align((size_t)n * sizeof(int)), e = flats_align((size_t)n), c = flats_align(CNT_SLOTS * sizeof(unsigned));
-  OFL_REQUIRE(workspace_bytes >= flats_bytes(rows, cols), OFL_ERR_WORKSPACE, "flats workspace too small: %zu < %zu",
-              workspace_bytes, flats_bytes(rows, cols));
-  char* p = static_cast<char*>(workspace);
-  w->parent = reinterpret_cast<unsigned*>(p);
-  w->q0 = reinterpret_cast<int*>(p + a);
-  w->q1 = reinterpret_cast<unsigned*>(p + 2 * a);
-  w->open = reinterpret_cast<unsigned*>(p + 3 * a);
-  w->edges = reinterpret_cast<uint8_t*>(p + 4 * a);
-  w->cnt = reinterpret_cast<unsigned*>(p + 4 * a + e);
-  w->tiles = reinterpret_cast<int*>(p + 4 * a + e + c);
+  *w = flats_layout(workspace, rows, cols);
+  OFL_REQUIRE(workspace_bytes >= w->bytes, OFL_ERR_WORKSPACE, "flats workspace too small: %zu < %zu", workspace_bytes,
+              w->bytes);
   return OFL_OK;
-}
-
-// CTAs of the persistent sweep kernel: as many as are resident at once (the grid barrier needs them all)
-int sweep_blocks() {
-  static std::atomic<int> gen{-1};
-  static std::atomic<int> blocks{0};
-  if (gen.load() != device_generation()) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, flat_tile_sweep_kernel, FS_THREADS, 0) != cudaSuccess || per_sm < 1)
-      per_sm = 1;
-    blocks.store(per_sm * sm_count());
-    gen.store(device_generation());
-  }
-  return blocks.load();
 }
 
 // One sweep from the seed list in w.q1 (count in cnt[CNT_SEEDS]): levels by tile relaxation, then mask values.
@@ -1221,9 +1206,10 @@ int run_gradient(int rows, int cols, const int* labels, const uint8_t* fdr, int 
   flat_tile_seed_kernel<<<(unsigned)(sm_count() * 8), FL_THREADS, 0, st>>>(w.q1, flat_mask, a);
   OFL_CHECK_LAUNCH();
   {
+    // persistent: as many CTAs as are resident at once (the grid barrier needs them all)
+    const void* sweep = reinterpret_cast<const void*>(flat_tile_sweep_kernel);
     void* args[] = {&a};
-    OFL_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<const void*>(flat_tile_sweep_kernel), dim3((unsigned)sweep_blocks()),
-                                         dim3(FS_THREADS), args, 0, st));
+    OFL_CUDA(cudaLaunchCooperativeKernel(sweep, dim3((unsigned)resident_ctas(sweep, FS_THREADS)), dim3(FS_THREADS), args, 0, st));
   }
   if (n % 4 == 0 && (reinterpret_cast<uintptr_t>(flat_mask) & 15) == 0 && !getenv("OFL_FLATS_SCALAR"))
     flat_tile_assign4_kernel<<<blocks_for(n / 4, FL_THREADS), FL_THREADS, 0, st>>>(
@@ -1259,7 +1245,7 @@ int run_gradient(int rows, int cols, const int* labels, const uint8_t* fdr, int 
 
 }  // namespace
 
-size_t flats_workspace_bytes(int64_t rows, int64_t cols) { return flats_bytes(rows, cols); }
+size_t flats_workspace_bytes(int64_t rows, int64_t cols) { return flats_layout(nullptr, rows, cols).bytes; }
 
 static int check_shape(int64_t rows, int64_t cols) {
   OFL_REQUIRE(rows > 0 && cols > 0 && rows < (1ll << 31) && cols < (1ll << 31) && rows * cols <= (1ll << 32), OFL_ERR_INVALID,

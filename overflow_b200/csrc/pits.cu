@@ -283,13 +283,25 @@ __global__ void __launch_bounds__(PT) pits_rounds_kernel(const PitsArgs a) {
   if (tid == 0) a.cnt[PC_ROUNDS] = rounds;
 }
 
-inline size_t align256(size_t v) { return (v + 255) / 256 * 256; }
+// Cuts the workspace at `base` into a's pit lists, flags and counters and returns its size; with a null base only the
+// size is meaningful.
+size_t pits_layout(void* base, int64_t rows, int64_t cols, PitsArgs& a) {
+  const size_t n = (size_t)rows * (size_t)cols;
+  Carver c(base);
+  // pits are never adjacent, so there are at most n / 4 of them: two lists fit the n ints
+  c.take(a.list_a, n * sizeof(int));
+  a.list_b = a.list_a + (n + 1) / 2;
+  c.take(a.waiting, n);
+  c.take(a.ready, n);
+  c.take(a.cnt, PC_SLOTS * sizeof(unsigned));
+  return c.bytes;
+}
 
 }  // namespace
 
 size_t pits_workspace_bytes(int64_t rows, int64_t cols) {
-  const size_t n = (size_t)rows * (size_t)cols;
-  return align256(n * sizeof(int)) + 2 * align256(n) + align256(PC_SLOTS * sizeof(unsigned));
+  PitsArgs a;
+  return pits_layout(nullptr, rows, cols, a);
 }
 
 // chunk: device, rows x cols with leading dimension ld, breached in place.  unsolved: device int8, dense.
@@ -298,17 +310,18 @@ int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, dou
                        int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st) {
   OFL_REQUIRE(rows > 0 && cols > 0 && rows < (1ll << 31) && cols < (1ll << 31) && rows * cols <= (1ll << 32), OFL_ERR_INVALID,
               "pit breaching works on one chunk of at most 2^32 cells (got %lld x %lld)", (long long)rows, (long long)cols);
-  OFL_REQUIRE(workspace_bytes >= pits_workspace_bytes(rows, cols), OFL_ERR_WORKSPACE, "pits workspace too small");
+  PitsArgs a;
+  const size_t need = pits_layout(workspace, rows, cols, a);
+  OFL_REQUIRE(workspace_bytes >= need, OFL_ERR_WORKSPACE, "pits workspace too small");
+  a.chunk = chunk;
+  a.rows = (int)rows;
+  a.cols = (int)cols;
+  a.ld = ld;
+  a.nodata = nodata;
+  a.unsolved = unsolved;
   const size_t n = (size_t)rows * (size_t)cols;
-  char* p = static_cast<char*>(workspace);
-  // pits are never adjacent, so there are at most n / 4 of them: two lists fit the n ints
-  unsigned* list_a = reinterpret_cast<unsigned*>(p);
-  unsigned* list_b = list_a + (n + 1) / 2;
-  uint8_t* waiting = reinterpret_cast<uint8_t*>(p + align256(n * sizeof(int)));
-  uint8_t* ready = waiting + align256(n);
-  unsigned* cnt = reinterpret_cast<unsigned*>(ready + align256(n));
   PhaseScope ps(PHASE_PITS, st);
-  OFL_CUDA(cudaMemsetAsync(cnt, 0, PC_SLOTS * sizeof(unsigned), st));
+  OFL_CUDA(cudaMemsetAsync(a.cnt, 0, PC_SLOTS * sizeof(unsigned), st));
   const float nd_f = (float)nodata;
   const bool nd_exact = (double)nd_f == nodata;  // false for NaN and for values float32 cannot hold: nothing matches then
   const bool vec = cols % 4 == 0 && ld % 4 == 0 && (reinterpret_cast<uintptr_t>(chunk) & 15) == 0 &&
@@ -316,25 +329,15 @@ int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, dou
   if (vec) {
     const dim3 grid((unsigned)((cols / 4 + 31) / 32), (unsigned)((rows + PT / 32 - 1) / (PT / 32)));
     OFL_REQUIRE(grid.y <= 65535u, OFL_ERR_INVALID, "chunk has too many rows for one launch");
-    pits_detect4_kernel<<<grid, PT, 0, st>>>(chunk, (int)rows, (int)cols, ld, nd_f, nd_exact, unsolved, waiting, list_a, cnt);
+    pits_detect4_kernel<<<grid, PT, 0, st>>>(chunk, (int)rows, (int)cols, ld, nd_f, nd_exact, unsolved, a.waiting, a.list_a,
+                                             a.cnt);
   } else {
     const unsigned nb = (unsigned)((n + PT - 1) / PT);
-    pits_detect_kernel<<<nb, PT, 0, st>>>(chunk, (int)rows, (int)cols, ld, nd_f, nd_exact, unsolved, waiting, list_a, cnt);
+    pits_detect_kernel<<<nb, PT, 0, st>>>(chunk, (int)rows, (int)cols, ld, nd_f, nd_exact, unsolved, a.waiting, a.list_a,
+                                          a.cnt);
   }
   OFL_CHECK_LAUNCH();
   {
-    PitsArgs a;
-    a.list_a = list_a;
-    a.list_b = list_b;
-    a.waiting = waiting;
-    a.ready = ready;
-    a.chunk = chunk;
-    a.rows = (int)rows;
-    a.cols = (int)cols;
-    a.ld = ld;
-    a.nodata = nodata;
-    a.unsolved = unsolved;
-    a.cnt = cnt;
     // round 1 over the whole list (its length is only known on the device: the grid covers the worst case a
     // strided loop needs, one pit per thread and 16 turns)
     const unsigned g1 = (unsigned)(sm_count() * 8);
@@ -350,7 +353,7 @@ int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, dou
   unsigned* h = nullptr;
   int rc = pinned_get(64, reinterpret_cast<void**>(&h));
   if (rc != OFL_OK) return rc;
-  OFL_CUDA(cudaMemcpyAsync(h, cnt, 3 * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
+  OFL_CUDA(cudaMemcpyAsync(h, a.cnt, 3 * sizeof(unsigned), cudaMemcpyDeviceToHost, st));
   OFL_CUDA(cudaStreamSynchronize(st));
   if (info) {
     info[0] = h[PC_PITS];

@@ -201,6 +201,30 @@ int shutdown() {
 
 int sm_count() { return g_state.sms > 0 ? g_state.sms : 148; }
 
+int resident_ctas(const void* kernel, int threads, int max_per_sm) {
+  struct Entry {
+    const void* kernel;
+    int generation, ctas;
+  };
+  static std::mutex mu;
+  static std::vector<Entry> cache;
+  std::lock_guard<std::mutex> lk(mu);
+  Entry* e = nullptr;
+  for (Entry& c : cache)
+    if (c.kernel == kernel) e = &c;
+  if (!e) {
+    cache.push_back({kernel, -1, 0});
+    e = &cache.back();
+  }
+  if (e->generation != device_generation()) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
+    e->ctas = (per_sm < max_per_sm ? per_sm : max_per_sm) * sm_count();
+    e->generation = device_generation();
+  }
+  return e->ctas;
+}
+
 int scratch_get(int slot, size_t bytes, void** out) {
   std::lock_guard<std::mutex> lk(g_mu);
   if (bytes == 0) bytes = 256;
