@@ -39,6 +39,9 @@
  *     fails: on return the library no longer reads or writes the caller's host buffers
  *   - every function returns OFL_OK (0) or a negative ofl_status; ofl_last_error() gives the message
  *     for the calling thread
+ *   - argument errors (OFL_ERR_INVALID, and OFL_ERR_WORKSPACE for a caller workspace) are reported before the
+ *     call allocates, copies or launches anything; what depends on the data read is found only by running the
+ *     call: a cycle (OFL_ERR_CYCLE), a pour point outside the raster, more than 2^29 flats in one tile
  *   - there is no CPU fallback: without a usable CUDA device every compute entry point fails
  */
 #ifndef OVERFLOW_B200_H

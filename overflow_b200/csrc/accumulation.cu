@@ -1273,6 +1273,13 @@ size_t strip_workspace_bytes(int64_t rows, int64_t cols) {
   return carve_graph(nullptr, node_count(rows, cols), GraphKind::STRIP).bytes;
 }
 
+// The rasters one accumulation call takes: 30-bit sides (AccParams holds ints) and 32-bit perimeter node ids.
+int accumulation_shape(int64_t rows, int64_t cols) {
+  OFL_REQUIRE(rows >= 1 && cols >= 1 && rows < (1ll << 30) && cols < (1ll << 30), OFL_ERR_INVALID, "bad raster size");
+  OFL_REQUIRE(node_count(rows, cols) < (1ll << 31), OFL_ERR_INVALID, "raster too large for 32-bit perimeter node ids");
+  return OFL_OK;
+}
+
 // Everything one raster (or strip) needs to launch its kernels.
 struct AccCtx {
   AccParams p;
@@ -1282,17 +1289,13 @@ struct AccCtx {
 };
 
 static int acc_setup(AccCtx& C, const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int y_off, int has_above,
-                     int has_below, long long* fac, int64_t ld_fac, void* workspace, size_t workspace_bytes, bool strip) {
-  OFL_REQUIRE(rows >= 1 && cols >= 1 && rows < (1ll << 30) && cols < (1ll << 30), OFL_ERR_INVALID, "bad raster size");
+                     int has_below, long long* fac, int64_t ld_fac, void* workspace, bool strip) {
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(fdr) & 15) == 0 && (ld_fdr % 16) == 0 && ld_fdr >= cols, OFL_ERR_ALIGNMENT,
               "fdr must be 16-byte aligned with ld_fdr %% 16 == 0 (ld_fdr=%lld)", (long long)ld_fdr);
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(fac) & 7) == 0 && ld_fac >= cols, OFL_ERR_ALIGNMENT, "fac must be 8-byte aligned");
   const int64_t n = node_count(rows, cols);
-  OFL_REQUIRE(n < (1ll << 31), OFL_ERR_INVALID, "raster too large for 32-bit perimeter node ids");
   C.graph = carve_graph(workspace, n, strip ? GraphKind::STRIP : GraphKind::RASTER);
   const Graph& g = C.graph;
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE,
-              "accumulation workspace too small: need %zu bytes, have %zu", g.bytes, workspace_bytes);
   AccParams& p = C.p;
   p.rows = (int)rows;
   p.cols = (int)cols;
@@ -1364,20 +1367,17 @@ static int final_pass(const AccCtx& C, cudaStream_t st) {  // over every tile
 // The part of a whole-raster accumulation that does not depend on the codes: clear_graph.  A caller that produces the
 // codes on the same device (ofl_flow_routing_f32) runs it on a second stream next to the direction kernel and passes
 // prepared = true below.
-int accumulation_prepare(int64_t rows, int64_t cols, void* workspace, size_t workspace_bytes, cudaStream_t st) {
+int accumulation_prepare(int64_t rows, int64_t cols, void* workspace, cudaStream_t st) {
   if (rows <= 0 || cols <= 0) return OFL_OK;
-  const Graph g = carve_graph(workspace, node_count(rows, cols), GraphKind::RASTER);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE,
-              "accumulation workspace too small: need %zu bytes, have %zu", g.bytes, workspace_bytes);
-  return clear_graph(g, st);
+  return clear_graph(carve_graph(workspace, node_count(rows, cols), GraphKind::RASTER), st);
 }
 
 int launch_accumulation(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, long long* fac,
-                        int64_t ld_fac, long long* perim_links_dev, void* workspace, size_t workspace_bytes,
-                        cudaStream_t st, bool prepared, bool trusted_codes, const long long* perim_inflow_dev) {
+                        int64_t ld_fac, long long* perim_links_dev, void* workspace, cudaStream_t st, bool prepared,
+                        bool trusted_codes, const long long* perim_inflow_dev) {
   if (rows <= 0 || cols <= 0) return OFL_OK;
   AccCtx C;
-  int rc = acc_setup(C, fdr, rows, cols, ld_fdr, 0, 0, 0, fac, ld_fac, workspace, workspace_bytes, false);
+  int rc = acc_setup(C, fdr, rows, cols, ld_fdr, 0, 0, 0, fac, ld_fac, workspace, false);
   if (rc != OFL_OK) return rc;
   C.p.trusted_codes = trusted_codes ? 1 : 0;
   if (!prepared) {
@@ -1567,20 +1567,18 @@ __global__ void pj_add_kernel_if(unsigned long long* __restrict__ S, const unsig
   }
 }
 
-static int strip_setup(AccCtx& C, const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above,
-                       int has_below, long long* fac, int64_t ld_fac, void* workspace, size_t workspace_bytes) {
+int strip_shape(int64_t rows, int64_t cols, int has_below) {
   OFL_REQUIRE(rows >= 2, OFL_ERR_INVALID, "a strip needs at least 2 rows");
   OFL_REQUIRE(!has_below || rows % AT == 0, OFL_ERR_INVALID,
               "a strip with a strip below it must have a multiple of %d rows (got %lld)", AT, (long long)rows);
-  return acc_setup(C, fdr_halo, rows, cols, ld_fdr, 1, has_above, has_below, fac, ld_fac, workspace, workspace_bytes, true);
+  return accumulation_shape(rows, cols);
 }
 
 // The three strip calls below only enqueue work; strip_collect_flags hands out their error flags.
 int strip_accum_local(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above, int has_below,
-                      long long* fac, int64_t ld_fac, void* workspace, size_t workspace_bytes, void* record,
-                      cudaStream_t st) {
+                      long long* fac, int64_t ld_fac, void* workspace, void* record, cudaStream_t st) {
   AccCtx C;
-  int rc = strip_setup(C, fdr_halo, rows, cols, ld_fdr, has_above, has_below, fac, ld_fac, workspace, workspace_bytes);
+  int rc = acc_setup(C, fdr_halo, rows, cols, ld_fdr, 1, has_above, has_below, fac, ld_fac, workspace, true);
   if (rc != OFL_OK) return rc;
   rc = clear_graph(C.graph, st);
   if (rc != OFL_OK) return rc;
@@ -1605,17 +1603,20 @@ int strip_accum_local(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64
   return OFL_OK;
 }
 
-size_t strip_boundary_workspace_bytes(int n_strips, int64_t cols) {
+size_t strip_boundary_workspace_bytes(int64_t n_strips, int64_t cols) {
   return carve_graph(nullptr, (int64_t)n_strips * 2 * cols, GraphKind::BOUNDARY).bytes;
 }
 
-int strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, long long* J_all, void* workspace,
-                         size_t workspace_bytes, cudaStream_t st) {
+int boundary_shape(int64_t n_strips, int64_t cols) {
   OFL_REQUIRE(n_strips >= 1 && cols >= 1, OFL_ERR_INVALID, "bad boundary graph size");
+  OFL_REQUIRE(n_strips * 2 * cols < (1ll << 31), OFL_ERR_INVALID, "boundary graph too large");
+  return OFL_OK;
+}
+
+int strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, long long* J_all, void* workspace,
+                         cudaStream_t st) {
   const int64_t n = (int64_t)n_strips * 2 * cols;
-  OFL_REQUIRE(n < (1ll << 31), OFL_ERR_INVALID, "boundary graph too large");
   const Graph g = carve_graph(workspace, n, GraphKind::BOUNDARY);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= g.bytes, OFL_ERR_WORKSPACE, "boundary workspace too small");
   int rc = clear_graph(g, st);
   if (rc != OFL_OK) return rc;
   RecView rec;
@@ -1651,10 +1652,9 @@ int strip_collect_flags(const void* strip_workspace, int64_t rows, int64_t cols,
 }
 
 int strip_accum_final(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above, int has_below,
-                      const long long* J_mine, void* workspace, size_t workspace_bytes, long long* fac, int64_t ld_fac,
-                      cudaStream_t st) {
+                      const long long* J_mine, void* workspace, long long* fac, int64_t ld_fac, cudaStream_t st) {
   AccCtx C;
-  int rc = strip_setup(C, fdr_halo, rows, cols, ld_fdr, has_above, has_below, fac, ld_fac, workspace, workspace_bytes);
+  int rc = acc_setup(C, fdr_halo, rows, cols, ld_fdr, 1, has_above, has_below, fac, ld_fac, workspace, true);
   if (rc != OFL_OK) return rc;
   const Graph& g = C.graph;
   // inflow from other strips: walked down the forest from its entry cells when every such path is short, else

@@ -1,6 +1,7 @@
 // api.cu -- the extern "C" surface declared in include/overflow_b200.h.
 // Host-pointer calls stage through library-owned device buffers; device-pointer calls launch directly.
 #include <cstdlib>
+#include <initializer_list>
 
 #include "common.cuh"
 
@@ -14,6 +15,7 @@ void launch_count_reset();
 void phase_timing_enable(int on);
 int phase_timing_read(double* ms, int64_t* counts, int n, int reset);
 
+int direction_shape(int64_t in_rows, int64_t cols);
 int launch_direction(const float* dem, int64_t in_rows, int64_t cols, int64_t ld_dem, double nodata, uint8_t* fdr,
                      int64_t rows, int64_t ld_fdr, int y_off, cudaStream_t st);
 int launch_direction_generic(const void* dem, int kind, int64_t in_rows, int64_t cols, int64_t ld_dem, double nodata,
@@ -21,42 +23,46 @@ int launch_direction_generic(const void* dem, int kind, int64_t in_rows, int64_t
 int launch_fill_border(uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld, int value, cudaStream_t st);
 int64_t perimeter_count(int64_t rows, int64_t cols);
 size_t accumulation_workspace_bytes(int64_t rows, int64_t cols);
+int accumulation_shape(int64_t rows, int64_t cols);
 int launch_accumulation(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, long long* fac, int64_t ld_fac,
-                        long long* perim_links_dev, void* workspace, size_t workspace_bytes, cudaStream_t st,
-                        bool prepared = false, bool trusted_codes = false, const long long* perim_inflow_dev = nullptr);
-int accumulation_prepare(int64_t rows, int64_t cols, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                        long long* perim_links_dev, void* workspace, cudaStream_t st, bool prepared = false,
+                        bool trusted_codes = false, const long long* perim_inflow_dev = nullptr);
+int accumulation_prepare(int64_t rows, int64_t cols, void* workspace, cudaStream_t st);
 size_t strip_workspace_bytes(int64_t rows, int64_t cols);
-size_t strip_boundary_workspace_bytes(int n_strips, int64_t cols);
+size_t strip_boundary_workspace_bytes(int64_t n_strips, int64_t cols);
 size_t strip_record_bytes(int64_t cols);
+int strip_shape(int64_t rows, int64_t cols, int has_below);
 int strip_accum_local(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above, int has_below,
-                      long long* fac, int64_t ld_fac, void* workspace, size_t workspace_bytes, void* record,
-                      cudaStream_t st);
+                      long long* fac, int64_t ld_fac, void* workspace, void* record, cudaStream_t st);
+int boundary_shape(int64_t n_strips, int64_t cols);
 int strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, long long* J_all, void* workspace,
-                         size_t workspace_bytes, cudaStream_t st);
+                         cudaStream_t st);
 int strip_collect_flags(const void* strip_workspace, int64_t rows, int64_t cols, const void* boundary_workspace,
                         int n_strips, int32_t* flags_dev, cudaStream_t st);
 int strip_accum_final(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above, int has_below,
-                      const long long* J_mine, void* workspace, size_t workspace_bytes, long long* fac, int64_t ld_fac,
-                      cudaStream_t st);
+                      const long long* J_mine, void* workspace, long long* fac, int64_t ld_fac, cudaStream_t st);
 int launch_check(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* fac, int64_t ld_fac,
                  unsigned long long* n_bad_dev, cudaStream_t st, int y_off = 0, const long long* fac_above = nullptr,
                  const long long* fac_below = nullptr);
 size_t flats_workspace_bytes(int64_t rows, int64_t cols);
+int flats_shape(int64_t rows, int64_t cols);
 int launch_flat_edges(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, uint8_t* edges, int64_t* n_low,
                       int64_t* n_high, unsigned* cnt_dev, cudaStream_t st);
 int launch_resolve_flats(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, int* flat_mask, int* labels,
-                         int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                         int64_t* info, void* workspace, cudaStream_t st);
 int launch_flat_gradient(const int* labels, const uint8_t* fdr, int64_t rows, int64_t cols, const int* seeds,
                          int64_t n_seeds, int towards, int* flat_mask, int* flat_height, int64_t n_heights,
-                         void* workspace, size_t workspace_bytes, cudaStream_t st);
+                         void* workspace, cudaStream_t st);
 int launch_masked_flow_dirs(const int* flat_mask, const int* labels, uint8_t* fdr, int64_t rows, int64_t cols,
                             cudaStream_t st);
 size_t pits_workspace_bytes(int64_t rows, int64_t cols);
+int pits_shape(int64_t rows, int64_t cols);
 int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, double nodata, int8_t* unsolved,
-                       int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                       int64_t* info, void* workspace, cudaStream_t st);
 size_t basins_workspace_bytes(int64_t rows, int64_t cols);
+int basins_shape(int64_t rows, int64_t cols);
 int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
-                  long long* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes, cudaStream_t st);
+                  long long* labels, int64_t ld_labels, void* workspace, cudaStream_t st);
 int check_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
                  const long long* labels, int64_t ld_labels, int64_t* n_bad, cudaStream_t st);
 int launch_synth(float* dem, int64_t rows, int64_t cols, int64_t ld, int64_t row0, int64_t total_rows, uint64_t seed,
@@ -166,10 +172,11 @@ int direction_from_host(const float* dem, int64_t in_rows, int64_t rows, int64_t
 enum { COPY_NONE = 0, COPY_IN = 1, COPY_OUT = 2 };
 
 struct CallArg {                      // one raster or vector (one row) argument of a call
-  const void* caller;                 // the caller's buffer; a host argument may be null (staging only)
+  const void* caller;                 // the caller's buffer; a nullable host argument may be null (staging only)
   int64_t rows, row_bytes, pitch;     // its layout in bytes
   int copy;                           // what a host call moves between `caller` and its slot (COPY_*)
   int64_t align;                      // a slot row is row_bytes rounded up to this; 1: packed rows, copied in one piece
+  bool nullable;                      // the call accepts a null `caller`
   void* dev;                          // set by stage_in: what the body reads and writes
   int64_t dev_pitch;
   template <class T> T* d() const { return static_cast<T*>(dev); }
@@ -233,6 +240,67 @@ int read_counter(int64_t* out, const void* d_cnt, cudaStream_t st) {
   *out = (int64_t)h;
   return OFL_OK;
 }
+
+// ---------------------------------------------------------------- argument checks
+// Every compute entry point lists its CallArgs and runs through run_call; checks that need more than its raster's
+// shape (enums, counts, a strip's rows) come before it.  So an argument error is reported before the call touches
+// the device, and a host call is refused only before its first copy.  After that a call fails only on the data it
+// reads (a cycle, a pour point outside the raster, more than 2^29 flats in one tile) or on CUDA.
+struct Result {  // a scalar result in host memory: zeroed first, so that a refused call leaves zeros behind
+  int64_t* p;
+  int n;
+  bool nullable;
+};
+
+struct Workspace {  // a device workspace: the caller's, which must hold need(rows, cols) bytes, or else the library's
+  void** ptr;
+  size_t* bytes;
+  size_t (*need)(int64_t, int64_t);
+  const char* what;
+};
+
+inline int no_limit(int64_t, int64_t) { return OFL_OK; }
+constexpr int EMPTY_RASTER = 1;
+
+template <int N, class Limit>
+int check_call(const CallArg (&a)[N], int64_t rows, int64_t cols, int mem_kind, std::initializer_list<Result> results,
+               Limit shape_limit, const Workspace& w) {
+  for (const Result& r : results) {
+    OFL_REQUIRE(r.p || r.nullable, OFL_ERR_INVALID, "null result pointer");
+    for (int k = 0; r.p && k < r.n; ++k) r.p[k] = 0;
+  }
+  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");
+  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
+  if (rows == 0 || cols == 0) return EMPTY_RASTER;
+  for (const CallArg& x : a) {
+    OFL_REQUIRE(x.caller || x.nullable, OFL_ERR_INVALID, "null raster pointer");
+    OFL_REQUIRE(!x.caller || x.pitch >= x.row_bytes, OFL_ERR_INVALID, "leading dimension smaller than cols");
+  }
+  int rc = shape_limit(rows, cols);
+  if (rc != OFL_OK) return rc;
+  const size_t need = w.ptr ? w.need(rows, cols) : 0;
+  OFL_REQUIRE(!w.ptr || !*w.ptr || *w.bytes >= need, OFL_ERR_WORKSPACE, "%s workspace too small: need %zu bytes, have %zu",
+              w.what, need, w.ptr ? *w.bytes : 0);
+  rc = ensure_init();
+  if (rc != OFL_OK || !w.ptr || *w.ptr) return rc;
+  *w.bytes = need;
+  return scratch_get(SCRATCH_WORK, need, w.ptr);
+}
+
+// Runs one compute entry point: zeroes the results; checks the sizes, mem_kind, and for a non-empty raster every
+// argument's pointer and pitch, the shape limit of the kernels and the workspace; brings the device up, takes the
+// library's workspace if the caller gave none, stages the arguments, runs body(stream) and finishes the call.  An
+// empty raster returns OFL_OK once the sizes are checked.
+template <int N, class Limit, class Body>
+int run_call(CallArg (&a)[N], int64_t rows, int64_t cols, int mem_kind, void* stream,
+             std::initializer_list<Result> results, Limit shape_limit, Workspace w, Body body) {
+  int rc = check_call(a, rows, cols, mem_kind, results, shape_limit, w);
+  if (rc != OFL_OK) return rc == EMPTY_RASTER ? OFL_OK : rc;
+  const cudaStream_t st = static_cast<cudaStream_t>(stream);
+  rc = stage_in(a, mem_kind, st);
+  if (rc == OFL_OK) rc = body(st);
+  return finish_call(rc, a, mem_kind, st);
+}
 }  // namespace
 
 extern "C" {
@@ -250,94 +318,66 @@ size_t ofl_accumulation_workspace_bytes(int64_t rows, int64_t cols) { return acc
 
 int ofl_flow_direction_f32(const float* dem, int64_t rows, int64_t cols, int64_t ld_dem, double nodata, uint8_t* fdr,
                            int64_t ld_fdr, int mode, int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");
   OFL_REQUIRE(mode == OFL_DIR_MODE_TILE || mode == OFL_DIR_MODE_RASTER || mode == OFL_DIR_MODE_STRIP, OFL_ERR_INVALID,
               "unknown direction mode %d", mode);
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(dem != nullptr && fdr != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(ld_dem >= cols && ld_fdr >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int y_off = (mode == OFL_DIR_MODE_STRIP) ? 1 : 0;
   const int64_t in_rows = rows + 2 * y_off;
   const bool tile = mode == OFL_DIR_MODE_TILE;
   // host: the DEM goes up in bands; the codes come back band by band, or in TILE mode in one copy after the ring fill
   CallArg a[] = {{dem, in_rows, cols * 4, ld_dem * 4, COPY_NONE, 16},
                  {fdr, rows, cols, ld_fdr, tile ? COPY_OUT : COPY_NONE, 16}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = mem_kind == OFL_MEM_HOST
-             ? direction_from_host(dem, in_rows, rows, cols, ld_dem, nodata, y_off, a[0].d<float>(), a[0].ld(4),
-                                   a[1].d<uint8_t>(), a[1].ld(1), tile ? nullptr : fdr, ld_fdr, st)
-             : launch_direction(dem, in_rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, y_off, st);
-  if (rc == OFL_OK && tile) rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
-  return finish_call(rc, a, mem_kind, st);
+  const auto limit = [&](int64_t, int64_t) {  // a host DEM reaches the kernel in row bands
+    return direction_shape(mem_kind == OFL_MEM_DEVICE ? in_rows : 0, cols);
+  };
+  return run_call(a, rows, cols, mem_kind, stream, {}, limit, {}, [&](cudaStream_t st) {
+    int rc = mem_kind == OFL_MEM_HOST
+                 ? direction_from_host(dem, in_rows, rows, cols, ld_dem, nodata, y_off, a[0].d<float>(), a[0].ld(4),
+                                       a[1].d<uint8_t>(), a[1].ld(1), tile ? nullptr : fdr, ld_fdr, st)
+                 : launch_direction(dem, in_rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, y_off, st);
+    if (rc == OFL_OK && tile) rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
+    return rc;
+  });
 }
 
 int ofl_flow_direction_x64(const void* dem, int elem_kind, int64_t rows, int64_t cols, int64_t ld_dem, double nodata,
                            uint8_t* fdr, int64_t ld_fdr, int mode, int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");
   OFL_REQUIRE(elem_kind == OFL_ELEM_F64 || elem_kind == OFL_ELEM_I64 || elem_kind == OFL_ELEM_U64, OFL_ERR_INVALID,
               "unknown element kind %d", elem_kind);
   OFL_REQUIRE(mode == OFL_DIR_MODE_TILE || mode == OFL_DIR_MODE_RASTER || mode == OFL_DIR_MODE_STRIP, OFL_ERR_INVALID,
               "unknown direction mode %d", mode);
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(dem != nullptr && fdr != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(ld_dem >= cols && ld_fdr >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int y_off = (mode == OFL_DIR_MODE_STRIP) ? 1 : 0;
   const int64_t in_rows = rows + 2 * y_off;
   CallArg a[] = {{dem, in_rows, cols * 8, ld_dem * 8, COPY_IN, 8}, {fdr, rows, cols, ld_fdr, COPY_OUT, 16}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_direction_generic(a[0].dev, elem_kind, in_rows, cols, a[0].ld(8), nodata, a[1].d<uint8_t>(), rows,
-                                  a[1].ld(1), y_off, st);
-  if (rc == OFL_OK && mode == OFL_DIR_MODE_TILE)
-    rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {}, no_limit, {}, [&](cudaStream_t st) {
+    int rc = launch_direction_generic(a[0].dev, elem_kind, in_rows, cols, a[0].ld(8), nodata, a[1].d<uint8_t>(), rows,
+                                      a[1].ld(1), y_off, st);
+    if (rc == OFL_OK && mode == OFL_DIR_MODE_TILE)
+      rc = launch_fill_border(a[1].d<uint8_t>(), rows, cols, a[1].ld(1), OFL_DIR_NODATA, st);
+    return rc;
+  });
 }
 
 int ofl_fill_border_u8(uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int value, void* stream) {
-  OFL_REQUIRE(fdr != nullptr || rows * cols == 0, OFL_ERR_INVALID, "null raster pointer");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  return launch_fill_border(fdr, rows, cols, ld_fdr, value, static_cast<cudaStream_t>(stream));
+  CallArg a[] = {{fdr, rows, cols, ld_fdr}};
+  return run_call(a, rows, cols, OFL_MEM_DEVICE, stream, {}, no_limit, {},
+                  [&](cudaStream_t st) { return launch_fill_border(fdr, rows, cols, ld_fdr, value, st); });
 }
 
 // shared by ofl_flow_accumulation_u8 and ofl_flow_accumulation_seeded_u8
 static int accumulation_entry(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int64_t* fac, int64_t ld_fac,
                               const int64_t* perim_inflow, int64_t* perim_links, void* workspace, size_t workspace_bytes,
                               int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(fdr != nullptr && fac != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(ld_fdr >= cols && ld_fac >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const size_t need = accumulation_workspace_bytes(rows, cols);
-  if (workspace == nullptr) {
-    rc = scratch_get(SCRATCH_WORK, need, &workspace);
-    if (rc != OFL_OK) return rc;
-    workspace_bytes = need;
-  }
   const int64_t n_perim = perimeter_count(rows, cols);
   CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_OUT, 16},
                  {fdr, rows, cols, ld_fdr, COPY_IN, 16},
-                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1},
-                 {perim_inflow, 1, n_perim * 8, n_perim * 8, COPY_IN, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_accumulation(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<long long>(), a[0].ld(8),
-                             perim_links ? a[2].d<long long>() : nullptr, workspace, workspace_bytes, st, false, false,
-                             perim_inflow ? a[3].d<const long long>() : nullptr);
-  return finish_call(rc, a, mem_kind, st);
+                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1, true},
+                 {perim_inflow, 1, n_perim * 8, n_perim * 8, COPY_IN, 1, true}};
+  return run_call(a, rows, cols, mem_kind, stream, {}, accumulation_shape,
+                  {&workspace, &workspace_bytes, accumulation_workspace_bytes, "accumulation"}, [&](cudaStream_t st) {
+                    return launch_accumulation(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<long long>(),
+                                               a[0].ld(8), perim_links ? a[2].d<long long>() : nullptr, workspace, st,
+                                               false, false, perim_inflow ? a[3].d<const long long>() : nullptr);
+                  });
 }
 
 int ofl_flow_accumulation_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, int64_t* fac,
@@ -354,93 +394,75 @@ int ofl_flow_accumulation_seeded_u8(const uint8_t* fdr, int64_t rows, int64_t co
                             mem_kind, stream);
 }
 
+// Device rasters: the workspace is cleared on a second stream while the stencil runs.  Host rasters: the DEM goes up
+// and the codes come back in bands, overlapping; the counts follow the accumulation.
+static int routing_on_device(const float* dem, int64_t rows, int64_t cols, int64_t ld_dem, double nodata, uint8_t* fdr,
+                             int64_t ld_fdr, int64_t* fac, int64_t ld_fac, int64_t* perim_links, void* work,
+                             cudaStream_t st) {
+  int rc = pipe_streams();
+  if (rc != OFL_OK) return rc;
+  OFL_CUDA(cudaEventRecord(g_pipe.ev_in, st));
+  OFL_CUDA(cudaStreamWaitEvent(g_pipe.h2d, g_pipe.ev_in, 0));
+  rc = accumulation_prepare(rows, cols, work, g_pipe.h2d);
+  if (rc != OFL_OK) return rc;
+  OFL_CUDA(cudaEventRecord(g_pipe.ev_prep, g_pipe.h2d));
+  rc = launch_direction(dem, rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, 0, st);
+  if (rc != OFL_OK) return rc;
+  OFL_CUDA(cudaStreamWaitEvent(st, g_pipe.ev_prep, 0));
+  return launch_accumulation(fdr, rows, cols, ld_fdr, reinterpret_cast<long long*>(fac), ld_fac,
+                             reinterpret_cast<long long*>(perim_links), work, st, true, true);
+}
+
 int ofl_flow_routing_f32(const float* dem, int64_t rows, int64_t cols, int64_t ld_dem, double nodata, uint8_t* fdr,
                          int64_t ld_fdr, int64_t* fac, int64_t ld_fac, int64_t* perim_links, int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(dem != nullptr && fac != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(ld_dem >= cols && ld_fac >= cols && (fdr == nullptr || ld_fdr >= cols), OFL_ERR_INVALID,
-              "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* work = nullptr;
-  const size_t need = accumulation_workspace_bytes(rows, cols);
-  rc = scratch_get(SCRATCH_WORK, need, &work);
-  if (rc != OFL_OK) return rc;
-  if (mem_kind == OFL_MEM_DEVICE) {
-    OFL_REQUIRE(fdr != nullptr, OFL_ERR_INVALID, "device callers provide the code raster");
-    // the workspace is cleared on a second stream while the stencil runs
-    rc = pipe_streams();
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaEventRecord(g_pipe.ev_in, st));
-    OFL_CUDA(cudaStreamWaitEvent(g_pipe.h2d, g_pipe.ev_in, 0));
-    rc = accumulation_prepare(rows, cols, work, need, g_pipe.h2d);
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaEventRecord(g_pipe.ev_prep, g_pipe.h2d));
-    rc = launch_direction(dem, rows, cols, ld_dem, nodata, fdr, rows, ld_fdr, 0, st);
-    if (rc != OFL_OK) return rc;
-    OFL_CUDA(cudaStreamWaitEvent(st, g_pipe.ev_prep, 0));
-    return launch_accumulation(fdr, rows, cols, ld_fdr, reinterpret_cast<long long*>(fac), ld_fac,
-                               reinterpret_cast<long long*>(perim_links), work, need, st, true, true);
-  }
-  // the DEM goes up and the codes come back in bands, overlapping; the counts follow the accumulation
   const int64_t n_perim = perimeter_count(rows, cols);
   CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_OUT, 16},
                  {dem, rows, cols * 4, ld_dem * 4, COPY_NONE, 16},
-                 {fdr, rows, cols, ld_fdr, COPY_NONE, 16},
-                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = direction_from_host(dem, rows, rows, cols, ld_dem, nodata, 0, a[1].d<float>(), a[1].ld(4), a[2].d<uint8_t>(),
-                             a[2].ld(1), fdr, ld_fdr, st);
-  if (rc == OFL_OK)
-    rc = launch_accumulation(a[2].d<const uint8_t>(), rows, cols, a[2].ld(1), a[0].d<long long>(), a[0].ld(8),
-                             perim_links ? a[3].d<long long>() : nullptr, work, need, st, false, true);
-  return finish_call(rc, a, mem_kind, st);
+                 {fdr, rows, cols, ld_fdr, COPY_NONE, 16, mem_kind == OFL_MEM_HOST},
+                 {perim_links, 1, n_perim * 16, n_perim * 16, COPY_OUT, 1, true}};
+  void* work = nullptr;
+  size_t need = 0;
+  return run_call(a, rows, cols, mem_kind, stream, {}, accumulation_shape,
+                  {&work, &need, accumulation_workspace_bytes, "accumulation"}, [&](cudaStream_t st) {
+                    if (mem_kind == OFL_MEM_DEVICE)
+                      return routing_on_device(dem, rows, cols, ld_dem, nodata, fdr, ld_fdr, fac, ld_fac, perim_links,
+                                               work, st);
+                    int rc = direction_from_host(dem, rows, rows, cols, ld_dem, nodata, 0, a[1].d<float>(), a[1].ld(4),
+                                                 a[2].d<uint8_t>(), a[2].ld(1), fdr, ld_fdr, st);
+                    if (rc != OFL_OK) return rc;
+                    return launch_accumulation(a[2].d<const uint8_t>(), rows, cols, a[2].ld(1), a[0].d<long long>(),
+                                               a[0].ld(8), perim_links ? a[3].d<long long>() : nullptr, work, st,
+                                               false, true);
+                  });
 }
 
+// The checkers count violations in SCRATCH_MISC.
 int ofl_check_accumulation_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* fac,
                               int64_t ld_fac, int64_t* n_bad, int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_bad != nullptr, OFL_ERR_INVALID, "bad argument");
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  *n_bad = 0;
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(fdr != nullptr && fac != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* d_cnt = nullptr;
-  rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
-  if (rc != OFL_OK) return rc;
   CallArg a[] = {{fac, rows, cols * 8, ld_fac * 8, COPY_IN, 8}, {fdr, rows, cols, ld_fdr, COPY_IN, 16}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_check(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<const long long>(), a[0].ld(8),
-                      static_cast<unsigned long long*>(d_cnt), st);
-  if (rc == OFL_OK) rc = read_counter(n_bad, d_cnt, st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {{n_bad, 1, false}}, no_limit, {}, [&](cudaStream_t st) {
+    void* d_cnt = nullptr;
+    int rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
+    if (rc == OFL_OK)
+      rc = launch_check(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[0].d<const long long>(), a[0].ld(8),
+                        static_cast<unsigned long long*>(d_cnt), st);
+    return rc == OFL_OK ? read_counter(n_bad, d_cnt, st) : rc;
+  });
 }
 
 int ofl_strip_check_accumulation_u8(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr,
                                     const int64_t* fac, int64_t ld_fac, const int64_t* fac_above,
                                     const int64_t* fac_below, int64_t* n_bad, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_bad != nullptr, OFL_ERR_INVALID, "bad argument");
-  *n_bad = 0;
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(fdr_halo != nullptr && fac != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  void* d_cnt = nullptr;
-  rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
-  if (rc != OFL_OK) return rc;
-  rc = launch_check(fdr_halo, rows, cols, ld_fdr, reinterpret_cast<const long long*>(fac), ld_fac,
-                    static_cast<unsigned long long*>(d_cnt), st, 1, reinterpret_cast<const long long*>(fac_above),
-                    reinterpret_cast<const long long*>(fac_below));
-  if (rc != OFL_OK) return rc;
-  return read_counter(n_bad, d_cnt, st);
+  CallArg a[] = {{fdr_halo, rows + 2, cols, ld_fdr}, {fac, rows, cols * 8, ld_fac * 8}};
+  return run_call(a, rows, cols, OFL_MEM_DEVICE, stream, {{n_bad, 1, false}}, no_limit, {}, [&](cudaStream_t st) {
+    void* d_cnt = nullptr;
+    int rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
+    if (rc == OFL_OK)
+      rc = launch_check(fdr_halo, rows, cols, ld_fdr, reinterpret_cast<const long long*>(fac), ld_fac,
+                        static_cast<unsigned long long*>(d_cnt), st, 1, reinterpret_cast<const long long*>(fac_above),
+                        reinterpret_cast<const long long*>(fac_below));
+    return rc == OFL_OK ? read_counter(n_bad, d_cnt, st) : rc;
+  });
 }
 
 // ---------------------------------------------------------------- flat resolution (csrc/flats.cu)
@@ -448,103 +470,80 @@ size_t ofl_flats_workspace_bytes(int64_t rows, int64_t cols) {
   return (rows > 0 && cols > 0) ? flats_workspace_bytes(rows, cols) : 0;
 }
 
-#define OFL_FLATS_COMMON(...)                                                                                        \
-  OFL_REQUIRE(rows >= 0 && cols >= 0, OFL_ERR_INVALID, "negative raster size");                                       \
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind); \
-  if (rows == 0 || cols == 0) return OFL_OK;                                                                           \
-  OFL_REQUIRE(__VA_ARGS__, OFL_ERR_INVALID, "null raster pointer");                                                    \
-  int rc = ensure_init();                                                                                              \
-  if (rc != OFL_OK) return rc;                                                                                         \
-  cudaStream_t st = static_cast<cudaStream_t>(stream)
-
 int ofl_flat_edges_f32(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, uint8_t* edges, int64_t* n_low,
                        int64_t* n_high, int mem_kind, void* stream) {
-  if (n_low) *n_low = 0;
-  if (n_high) *n_high = 0;
-  OFL_FLATS_COMMON(dem && fdr && edges);
-  void* d_cnt = nullptr;
-  rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
-  if (rc != OFL_OK) return rc;
   CallArg a[] = {{dem, rows, cols * 4, cols * 4, COPY_IN, 1},
                  {fdr, rows, cols, cols, COPY_IN, 1},
                  {edges, rows, cols, cols, COPY_OUT, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_flat_edges(a[0].d<const float>(), a[1].d<const uint8_t>(), rows, cols, a[2].d<uint8_t>(), n_low,
-                           n_high, static_cast<unsigned*>(d_cnt), st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {{n_low, 1, true}, {n_high, 1, true}}, flats_shape, {},
+                  [&](cudaStream_t st) {
+                    void* d_cnt = nullptr;
+                    const int rc = scratch_get(SCRATCH_MISC, 256, &d_cnt);
+                    if (rc != OFL_OK) return rc;
+                    return launch_flat_edges(a[0].d<const float>(), a[1].d<const uint8_t>(), rows, cols,
+                                             a[2].d<uint8_t>(), n_low, n_high, static_cast<unsigned*>(d_cnt), st);
+                  });
 }
 
 // resolve (+ with `fix`, rewrite the codes in place): shared by ofl_resolve_flats_f32 and ofl_fix_flats_f32
-static int flats_run(const float* dem, const uint8_t* fdr, bool fix, int64_t rows, int64_t cols, int32_t* flat_mask,
-                     int32_t* labels, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
-                     cudaStream_t st) {
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || (flat_mask && labels), OFL_ERR_INVALID,
-              "device callers provide flat_mask and labels");
-  int rc;
-  if (!workspace) {
-    workspace_bytes = flats_workspace_bytes(rows, cols);
-    if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
-  }
+static int flats_entry(const float* dem, const uint8_t* fdr, bool fix, int64_t rows, int64_t cols, int32_t* flat_mask,
+                       int32_t* labels, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
+                       void* stream) {
+  const bool staged_only = fix && mem_kind == OFL_MEM_HOST;  // a host fix_flats caller need not see mask and labels
   CallArg a[] = {{dem, rows, cols * 4, cols * 4, COPY_IN, 1},
-                 {flat_mask, rows, cols * 4, cols * 4, COPY_OUT, 1},
-                 {labels, rows, cols * 4, cols * 4, COPY_OUT, 1},
+                 {flat_mask, rows, cols * 4, cols * 4, COPY_OUT, 1, staged_only},
+                 {labels, rows, cols * 4, cols * 4, COPY_OUT, 1, staged_only},
                  {fdr, rows, cols, cols, fix ? COPY_IN | COPY_OUT : COPY_IN, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_resolve_flats(a[0].d<const float>(), a[3].d<const uint8_t>(), rows, cols, a[1].d<int>(), a[2].d<int>(),
-                              info, workspace, workspace_bytes, st);
-  if (rc == OFL_OK && fix) rc = launch_masked_flow_dirs(a[1].d<int>(), a[2].d<int>(), a[3].d<uint8_t>(), rows, cols, st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {{info, 5, true}}, flats_shape,
+                  {&workspace, &workspace_bytes, flats_workspace_bytes, "flats"}, [&](cudaStream_t st) {
+                    int rc = launch_resolve_flats(a[0].d<const float>(), a[3].d<const uint8_t>(), rows, cols,
+                                                  a[1].d<int>(), a[2].d<int>(), info, workspace, st);
+                    if (rc == OFL_OK && fix)
+                      rc = launch_masked_flow_dirs(a[1].d<int>(), a[2].d<int>(), a[3].d<uint8_t>(), rows, cols, st);
+                    return rc;
+                  });
 }
 
 int ofl_resolve_flats_f32(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, int32_t* flat_mask,
                           int32_t* labels, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
                           void* stream) {
-  if (info) for (int k = 0; k < 5; ++k) info[k] = 0;
-  OFL_FLATS_COMMON(dem && fdr && flat_mask && labels);
-  return flats_run(dem, fdr, false, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
+  return flats_entry(dem, fdr, false, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, stream);
 }
 
 int ofl_fix_flats_f32(const float* dem, uint8_t* fdr, int64_t rows, int64_t cols, int32_t* flat_mask, int32_t* labels,
                       int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind, void* stream) {
-  if (info) for (int k = 0; k < 5; ++k) info[k] = 0;
-  OFL_FLATS_COMMON(dem && fdr);
-  return flats_run(dem, fdr, true, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, st);
+  return flats_entry(dem, fdr, true, rows, cols, flat_mask, labels, info, workspace, workspace_bytes, mem_kind, stream);
 }
 
 int ofl_d8_masked_flow_dirs_i32(const int32_t* flat_mask, const int32_t* labels, uint8_t* fdr, int64_t rows, int64_t cols,
                                 int mem_kind, void* stream) {
-  OFL_FLATS_COMMON(flat_mask && labels && fdr);
   CallArg a[] = {{flat_mask, rows, cols * 4, cols * 4, COPY_IN, 1},
                  {labels, rows, cols * 4, cols * 4, COPY_IN, 1},
                  {fdr, rows, cols, cols, COPY_IN | COPY_OUT, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK) rc = launch_masked_flow_dirs(a[0].d<const int>(), a[1].d<const int>(), a[2].d<uint8_t>(), rows, cols, st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {}, flats_shape, {}, [&](cudaStream_t st) {
+    return launch_masked_flow_dirs(a[0].d<const int>(), a[1].d<const int>(), a[2].d<uint8_t>(), rows, cols, st);
+  });
 }
 
 int ofl_flat_gradient_i32(const int32_t* labels, const uint8_t* fdr, int64_t rows, int64_t cols, const int32_t* seeds,
                           int64_t n_seeds, int towards, int32_t* flat_mask, int32_t* flat_height, int64_t n_heights,
                           void* workspace, size_t workspace_bytes, int mem_kind, void* stream) {
-  OFL_FLATS_COMMON(labels && fdr && flat_mask && (seeds || n_seeds == 0) && (flat_height || n_heights == 0));
-  const int64_t n = rows * cols;
-  OFL_REQUIRE(n_seeds >= 0 && n_heights >= 0 && n_seeds <= n && n_heights <= n, OFL_ERR_INVALID,
-              "seed / flat_height count out of range");
-  if (!workspace) {
-    workspace_bytes = flats_workspace_bytes(rows, cols);
-    if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
-  }
   CallArg a[] = {{labels, rows, cols * 4, cols * 4, COPY_IN, 1},
                  {flat_mask, rows, cols * 4, cols * 4, COPY_IN | COPY_OUT, 1},
                  {fdr, rows, cols, cols, COPY_IN, 1},
-                 {seeds, 1, n_seeds * 4, n_seeds * 4, COPY_IN, 1},
-                 {flat_height, 1, n_heights * 4, n_heights * 4, COPY_IN | COPY_OUT, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_flat_gradient(a[0].d<const int>(), a[2].d<const uint8_t>(), rows, cols, a[3].d<const int>(), n_seeds,
-                              towards, a[1].d<int>(), a[4].d<int>(), n_heights, workspace, workspace_bytes, st);
-  return finish_call(rc, a, mem_kind, st);
+                 {seeds, 1, n_seeds * 4, n_seeds * 4, COPY_IN, 1, n_seeds == 0},
+                 {flat_height, 1, n_heights * 4, n_heights * 4, COPY_IN | COPY_OUT, 1, n_heights == 0}};
+  const auto limit = [&](int64_t r, int64_t c) -> int {
+    OFL_REQUIRE(n_seeds >= 0 && n_seeds <= r * c && n_seeds < (1ll << 32) && n_heights >= 0 && n_heights <= r * c,
+                OFL_ERR_INVALID, "seed / flat_height count out of range");
+    return flats_shape(r, c);
+  };
+  return run_call(a, rows, cols, mem_kind, stream, {}, limit,
+                  {&workspace, &workspace_bytes, flats_workspace_bytes, "flats"}, [&](cudaStream_t st) {
+                    return launch_flat_gradient(a[0].d<const int>(), a[2].d<const uint8_t>(), rows, cols,
+                                                a[3].d<const int>(), n_seeds, towards, a[1].d<int>(), a[4].d<int>(),
+                                                n_heights, workspace, st);
+                  });
 }
 
 // ---------------------------------------------------------------- single-cell pit breaching (csrc/pits.cu)
@@ -555,22 +554,16 @@ size_t ofl_pits_workspace_bytes(int64_t rows, int64_t cols) {
 int ofl_breach_single_cell_pits_f32(float* chunk, int64_t rows, int64_t cols, int64_t ld_chunk, double nodata,
                                     int8_t* unsolved, int64_t* info, void* workspace, size_t workspace_bytes, int mem_kind,
                                     void* stream) {
-  if (info) info[0] = info[1] = info[2] = 0;
-  OFL_FLATS_COMMON(chunk && unsolved);
-  OFL_REQUIRE(ld_chunk >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  if (!workspace) {
-    workspace_bytes = pits_workspace_bytes(rows, cols);
-    if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
-  }
   CallArg a[] = {{chunk, rows, cols * 4, ld_chunk * 4, COPY_IN | COPY_OUT, 4},
                  {unsolved, rows, cols, cols, COPY_OUT, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_breach_pits(a[0].d<float>(), rows, cols, a[0].ld(4), nodata, a[1].d<int8_t>(), info, workspace,
-                            workspace_bytes, st);
-  return finish_call(rc, a, mem_kind, st);
+  return run_call(a, rows, cols, mem_kind, stream, {{info, 3, true}}, pits_shape,
+                  {&workspace, &workspace_bytes, pits_workspace_bytes, "pits"}, [&](cudaStream_t st) {
+                    return launch_breach_pits(a[0].d<float>(), rows, cols, a[0].ld(4), nodata, a[1].d<int8_t>(), info,
+                                              workspace, st);
+                  });
 }
 
+// ---------------------------------------------------------------- row strips (csrc/accumulation.cu), device pointers
 size_t ofl_strip_workspace_bytes(int64_t rows, int64_t cols) { return strip_workspace_bytes(rows, cols); }
 size_t ofl_strip_boundary_workspace_bytes(int n_strips, int64_t cols) {
   return strip_boundary_workspace_bytes(n_strips, cols);
@@ -578,23 +571,31 @@ size_t ofl_strip_boundary_workspace_bytes(int n_strips, int64_t cols) {
 
 size_t ofl_strip_record_bytes(int64_t cols) { return strip_record_bytes(cols); }
 
+// A strip is never empty, so its shape is checked first.  Device buffers the strip calls only pass on are listed with
+// an empty row: run_call checks their pointers.
 int ofl_strip_accum_local(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above,
                           int has_below, int64_t* fac, int64_t ld_fac, void* workspace, size_t workspace_bytes,
                           void* record, void* stream) {
-  OFL_REQUIRE(fdr_halo && fac && workspace && record, OFL_ERR_INVALID, "null pointer");
-  int rc = ensure_init();
+  CallArg a[] = {{fdr_halo, rows + 2, cols, ld_fdr}, {fac, rows, cols * 8, ld_fac * 8}, {workspace}, {record}};
+  const int rc = strip_shape(rows, cols, has_below);
   if (rc != OFL_OK) return rc;
-  return strip_accum_local(fdr_halo, rows, cols, ld_fdr, has_above, has_below, reinterpret_cast<long long*>(fac), ld_fac,
-                           workspace, workspace_bytes, record, static_cast<cudaStream_t>(stream));
+  return run_call(a, rows, cols, OFL_MEM_DEVICE, stream, {}, no_limit,
+                  {&workspace, &workspace_bytes, strip_workspace_bytes, "strip"}, [&](cudaStream_t st) {
+                    return strip_accum_local(fdr_halo, rows, cols, ld_fdr, has_above, has_below,
+                                             reinterpret_cast<long long*>(fac), ld_fac, workspace, record, st);
+                  });
 }
 
 int ofl_strip_boundary_solve(const void* records_all, int n_strips, int64_t cols, int64_t* J_all, void* workspace,
                              size_t workspace_bytes, void* stream) {
-  OFL_REQUIRE(records_all && J_all && workspace, OFL_ERR_INVALID, "null pointer");
-  int rc = ensure_init();
+  CallArg a[] = {{records_all}, {J_all}, {workspace}};
+  const int rc = boundary_shape(n_strips, cols);
   if (rc != OFL_OK) return rc;
-  return strip_boundary_solve(records_all, n_strips, cols, reinterpret_cast<long long*>(J_all), workspace,
-                              workspace_bytes, static_cast<cudaStream_t>(stream));
+  return run_call(a, n_strips, cols, OFL_MEM_DEVICE, stream, {}, no_limit,
+                  {&workspace, &workspace_bytes, strip_boundary_workspace_bytes, "boundary"}, [&](cudaStream_t st) {
+                    return strip_boundary_solve(records_all, n_strips, cols, reinterpret_cast<long long*>(J_all),
+                                                workspace, st);
+                  });
 }
 
 int ofl_strip_collect_flags(const void* strip_workspace, int64_t rows, int64_t cols, const void* boundary_workspace,
@@ -611,12 +612,15 @@ int ofl_strip_collect_flags(const void* strip_workspace, int64_t rows, int64_t c
 int ofl_strip_accum_final(const uint8_t* fdr_halo, int64_t rows, int64_t cols, int64_t ld_fdr, int has_above,
                           int has_below, const int64_t* J_mine, void* workspace, size_t workspace_bytes, int64_t* fac,
                           int64_t ld_fac, void* stream) {
-  OFL_REQUIRE(fdr_halo && fac && workspace && J_mine, OFL_ERR_INVALID, "null pointer");
-  int rc = ensure_init();
+  CallArg a[] = {{fdr_halo, rows + 2, cols, ld_fdr}, {fac, rows, cols * 8, ld_fac * 8}, {workspace}, {J_mine}};
+  const int rc = strip_shape(rows, cols, has_below);
   if (rc != OFL_OK) return rc;
-  return strip_accum_final(fdr_halo, rows, cols, ld_fdr, has_above, has_below, reinterpret_cast<const long long*>(J_mine),
-                           workspace, workspace_bytes, reinterpret_cast<long long*>(fac), ld_fac,
-                           static_cast<cudaStream_t>(stream));
+  return run_call(a, rows, cols, OFL_MEM_DEVICE, stream, {}, no_limit,
+                  {&workspace, &workspace_bytes, strip_workspace_bytes, "strip"}, [&](cudaStream_t st) {
+                    return strip_accum_final(fdr_halo, rows, cols, ld_fdr, has_above, has_below,
+                                             reinterpret_cast<const long long*>(J_mine), workspace,
+                                             reinterpret_cast<long long*>(fac), ld_fac, st);
+                  });
 }
 
 // ---------------------------------------------------------------- drainage basins (csrc/basins.cu)
@@ -625,63 +629,40 @@ size_t ofl_basins_workspace_bytes(int64_t rows, int64_t cols) { return basins_wo
 int ofl_label_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
                         int64_t n_pour, int64_t* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes,
                         int mem_kind, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_pour >= 0, OFL_ERR_INVALID, "negative raster size or pour-point count");
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(fdr != nullptr && labels != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(pour_points != nullptr || n_pour == 0, OFL_ERR_INVALID, "null pour-point list");
-  OFL_REQUIRE(ld_fdr >= cols && ld_labels >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (workspace == nullptr) {
-    workspace_bytes = basins_workspace_bytes(rows, cols);
-    if ((rc = scratch_get(SCRATCH_WORK, workspace_bytes, &workspace)) != OFL_OK) return rc;
-  }
+  OFL_REQUIRE(n_pour >= 0, OFL_ERR_INVALID, "negative pour-point count");
   CallArg a[] = {{labels, rows, cols * 8, ld_labels * 8, COPY_OUT, 16},
                  {fdr, rows, cols, ld_fdr, COPY_IN, 16},
-                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = launch_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(), n_pour,
-                       a[0].d<long long>(), a[0].ld(8), workspace, workspace_bytes, st);
-  return finish_call(rc, a, mem_kind, st);
+                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1, n_pour == 0}};
+  return run_call(a, rows, cols, mem_kind, stream, {}, basins_shape,
+                  {&workspace, &workspace_bytes, basins_workspace_bytes, "basins"}, [&](cudaStream_t st) {
+                    return launch_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(),
+                                         n_pour, a[0].d<long long>(), a[0].ld(8), workspace, st);
+                  });
 }
 
 int ofl_check_basins_u8(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const int64_t* pour_points,
                         int64_t n_pour, const int64_t* labels, int64_t ld_labels, int64_t* n_bad, int mem_kind,
                         void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0 && n_pour >= 0 && n_bad != nullptr, OFL_ERR_INVALID, "bad argument");
-  OFL_REQUIRE(mem_kind == OFL_MEM_HOST || mem_kind == OFL_MEM_DEVICE, OFL_ERR_INVALID, "unknown mem_kind %d", mem_kind);
-  *n_bad = 0;
-  if (rows == 0 || cols == 0) return OFL_OK;
-  OFL_REQUIRE(fdr != nullptr && labels != nullptr, OFL_ERR_INVALID, "null raster pointer");
-  OFL_REQUIRE(pour_points != nullptr || n_pour == 0, OFL_ERR_INVALID, "null pour-point list");
-  OFL_REQUIRE(ld_fdr >= cols && ld_labels >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  OFL_REQUIRE(n_pour >= 0, OFL_ERR_INVALID, "negative pour-point count");
   CallArg a[] = {{labels, rows, cols * 8, ld_labels * 8, COPY_IN, 8},
                  {fdr, rows, cols, ld_fdr, COPY_IN, 16},
-                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1}};
-  rc = stage_in(a, mem_kind, st);
-  if (rc == OFL_OK)
-    rc = check_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(), n_pour,
-                      a[0].d<const long long>(), a[0].ld(8), n_bad, st);
-  return finish_call(rc, a, mem_kind, st);
+                 {pour_points, 1, n_pour * 8, n_pour * 8, COPY_IN, 1, n_pour == 0}};
+  return run_call(a, rows, cols, mem_kind, stream, {{n_bad, 1, false}}, no_limit, {}, [&](cudaStream_t st) {
+    return check_basins(a[1].d<const uint8_t>(), rows, cols, a[1].ld(1), a[2].d<const long long>(), n_pour,
+                        a[0].d<const long long>(), a[0].ld(8), n_bad, st);
+  });
 }
 
 int ofl_synth_dem_f32(float* dem, int64_t rows, int64_t cols, int64_t ld_dem, int64_t row0, int64_t total_rows,
                       uint64_t seed, int kind, float relief, int holes_permille, float nodata, void* stream) {
-  OFL_REQUIRE(rows >= 0 && cols >= 0 && ld_dem >= cols, OFL_ERR_INVALID, "bad raster size");
-  OFL_REQUIRE(dem != nullptr || rows * cols == 0, OFL_ERR_INVALID, "null raster pointer");
+  OFL_REQUIRE(ld_dem >= cols, OFL_ERR_INVALID, "leading dimension smaller than cols");  // empty rasters included
   OFL_REQUIRE(kind >= 0 && kind <= 4, OFL_ERR_INVALID, "unknown synthetic DEM kind %d", kind);
   OFL_REQUIRE((kind != 3 && kind != 4) || total_rows / 2 * cols < 0xFD000000ll, OFL_ERR_INVALID,
               "serpentine DEM: the chain would run out of finite float32 values");
-  int rc = ensure_init();
-  if (rc != OFL_OK) return rc;
-  return launch_synth(dem, rows, cols, ld_dem, row0, total_rows, seed, kind, relief, holes_permille, nodata,
-                      static_cast<cudaStream_t>(stream));
+  CallArg a[] = {{dem, rows, cols * 4, ld_dem * 4}};
+  return run_call(a, rows, cols, OFL_MEM_DEVICE, stream, {}, no_limit, {}, [&](cudaStream_t st) {
+    return launch_synth(dem, rows, cols, ld_dem, row0, total_rows, seed, kind, relief, holes_permille, nodata, st);
+  });
 }
 
 }  // extern "C"

@@ -355,20 +355,24 @@ size_t basins_workspace_bytes(int64_t rows, int64_t cols) {
   return carve(nullptr, rows, cols).bytes;
 }
 
-int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
-                  long long* labels, int64_t ld_labels, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (rows <= 0 || cols <= 0) return OFL_OK;
+// 30-bit sides (BasinParams holds ints) and 32-bit perimeter node ids.
+int basins_shape(int64_t rows, int64_t cols) {
   OFL_REQUIRE(rows < (1ll << 30) && cols < (1ll << 30), OFL_ERR_INVALID, "bad raster size");
+  OFL_REQUIRE(tiles_along(rows) * tiles_along(cols) * SLOTS < (1ll << 31), OFL_ERR_INVALID,
+              "raster too large for 32-bit perimeter node ids");
+  return OFL_OK;
+}
+
+int launch_basins(const uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld_fdr, const long long* pour, int64_t n_pour,
+                  long long* labels, int64_t ld_labels, void* workspace, cudaStream_t st) {
+  if (rows <= 0 || cols <= 0) return OFL_OK;
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(fdr) & 15) == 0 && (ld_fdr % 16) == 0 && ld_fdr >= cols, OFL_ERR_ALIGNMENT,
               "fdr must be 16-byte aligned with ld_fdr %% 16 == 0 (ld_fdr=%lld)", (long long)ld_fdr);
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(labels) & 7) == 0 && ld_labels >= cols, OFL_ERR_ALIGNMENT,
               "labels must be 8-byte aligned");
   const int ntx = (int)tiles_along(cols), nty = (int)tiles_along(rows);
   const int64_t ntiles = (int64_t)ntx * nty, nodes = ntiles * SLOTS;
-  OFL_REQUIRE(nodes < (1ll << 31), OFL_ERR_INVALID, "raster too large for 32-bit perimeter node ids");
   const BasinLayout L = carve(workspace, rows, cols);
-  OFL_REQUIRE(workspace != nullptr && workspace_bytes >= L.bytes, OFL_ERR_WORKSPACE,
-              "basins workspace too small: need %zu bytes, have %zu", L.bytes, workspace_bytes);
   BasinParams p;
   p.fdr = fdr;
   p.ld_fdr = ld_fdr;

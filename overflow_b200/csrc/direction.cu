@@ -457,13 +457,17 @@ int launch_fill_border(uint8_t* fdr, int64_t rows, int64_t cols, int64_t ld, int
   return OFL_OK;
 }
 
+// The DEMs one launch takes (in_rows >= rows): 30-bit sides, DirParams holds ints.
+int direction_shape(int64_t in_rows, int64_t cols) {
+  OFL_REQUIRE(in_rows < (1ll << 30) && cols < (1ll << 30), OFL_ERR_INVALID, "raster dimension too large");
+  return OFL_OK;
+}
+
 // Device-pointer launcher.  `dem` has in_rows x cols floats; `fdr` has rows x cols codes;
 // input row of output row y is y + y_off (0 for raster mode, 1 for a strip with halo rows).
 int launch_direction(const float* dem, int64_t in_rows, int64_t cols, int64_t ld_dem, double nodata, uint8_t* fdr,
                      int64_t rows, int64_t ld_fdr, int y_off, cudaStream_t st) {
   if (rows <= 0 || cols <= 0) return OFL_OK;
-  OFL_REQUIRE(rows < (1ll << 30) && cols < (1ll << 30) && in_rows < (1ll << 30), OFL_ERR_INVALID,
-              "raster dimension too large");
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(dem) & 15) == 0 && (ld_dem % 4) == 0 && ld_dem >= cols,
               OFL_ERR_ALIGNMENT, "dem must be 16-byte aligned with ld_dem %% 4 == 0 (ld_dem=%lld)", (long long)ld_dem);
   OFL_REQUIRE((reinterpret_cast<uintptr_t>(fdr) & 3) == 0 && (ld_fdr % 4) == 0 && ld_fdr >= cols, OFL_ERR_ALIGNMENT,

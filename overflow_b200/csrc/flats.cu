@@ -1169,13 +1169,6 @@ FlatsWork flats_layout(void* base, int64_t rows, int64_t cols) {
   return w;
 }
 
-int carve(void* workspace, size_t workspace_bytes, int64_t rows, int64_t cols, FlatsWork* w) {
-  *w = flats_layout(workspace, rows, cols);
-  OFL_REQUIRE(workspace_bytes >= w->bytes, OFL_ERR_WORKSPACE, "flats workspace too small: %zu < %zu", workspace_bytes,
-              w->bytes);
-  return OFL_OK;
-}
-
 // One sweep from the seed list in w.q1 (count in cnt[CNT_SEEDS]): levels by tile relaxation, then mask values.
 // Asynchronous unless the caller wants the level count.
 int run_gradient(int rows, int cols, const int* labels, const uint8_t* fdr, int mode, bool open_ready, int* flat_mask,
@@ -1247,7 +1240,8 @@ int run_gradient(int rows, int cols, const int* labels, const uint8_t* fdr, int 
 
 size_t flats_workspace_bytes(int64_t rows, int64_t cols) { return flats_layout(nullptr, rows, cols).bytes; }
 
-static int check_shape(int64_t rows, int64_t cols) {
+// One tile of at most 2^32 cells: cell indices are unsigned 32-bit on the device.
+int flats_shape(int64_t rows, int64_t cols) {
   OFL_REQUIRE(rows > 0 && cols > 0 && rows < (1ll << 31) && cols < (1ll << 31) && rows * cols <= (1ll << 32), OFL_ERR_INVALID,
               "flat resolution works on one tile of at most 2^32 cells (got %lld x %lld)", (long long)rows,
               (long long)cols);
@@ -1257,11 +1251,9 @@ static int check_shape(int64_t rows, int64_t cols) {
 // edges[i]: bit 0 low edge, bit 1 high edge; counts -> host.  Dense rasters (ld == cols), device pointers.
 int launch_flat_edges(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, uint8_t* edges, int64_t* n_low,
                       int64_t* n_high, unsigned* cnt_dev, cudaStream_t st) {
-  int rc = check_shape(rows, cols);
-  if (rc != OFL_OK) return rc;
   PhaseScope ps(PHASE_FLATS, st);
   OFL_CUDA(cudaMemsetAsync(cnt_dev, 0, CNT_SLOTS * sizeof(unsigned), st));
-  rc = launch_edges_kernel(dem, fdr, rows, cols, edges, nullptr, nullptr, cnt_dev, st);
+  int rc = launch_edges_kernel(dem, fdr, rows, cols, edges, nullptr, nullptr, cnt_dev, st);
   if (rc != OFL_OK) return rc;
   unsigned* h = nullptr;
   rc = pinned_get(256, reinterpret_cast<void**>(&h));
@@ -1276,20 +1268,16 @@ int launch_flat_edges(const float* dem, const uint8_t* fdr, int64_t rows, int64_
 // resolve_flats (fix_flats.py:227-288).  All pointers device, dense.  info (host, nullable) receives
 // {low edges, high edges, labels, levels of the away sweep, levels of the towards sweep}.
 int launch_resolve_flats(const float* dem, const uint8_t* fdr, int64_t rows, int64_t cols, int* flat_mask, int* labels,
-                         int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  int rc = check_shape(rows, cols);
-  if (rc != OFL_OK) return rc;
+                         int64_t* info, void* workspace, cudaStream_t st) {
   const int64_t n = rows * cols;
-  FlatsWork w;
-  rc = carve(workspace, workspace_bytes, rows, cols, &w);
-  if (rc != OFL_OK) return rc;
+  const FlatsWork w = flats_layout(workspace, rows, cols);
   const unsigned nb = blocks_for(n, FL_THREADS), nbc = blocks_for(n, FL_CELLS_PER_CTA);
   OFL_CUDA(cudaMemsetAsync(w.cnt, 0, CNT_SLOTS * sizeof(unsigned), st));
   int* flat_height = reinterpret_cast<int*>(w.parent);  // lives where the forest was once the labels are known
   unsigned* minlow = w.q1;      // per-component smallest low edge, until the labels are known
   int* seedlabel = flat_mask;   // label of each component's first low edge, until the labels are known
   unsigned* h = nullptr;
-  rc = pinned_get(256, reinterpret_cast<void**>(&h));
+  int rc = pinned_get(256, reinterpret_cast<void**>(&h));
   if (rc != OFL_OK) return rc;
   int64_t lv_away = 0, lv_low = 0;
   {
@@ -1357,15 +1345,9 @@ int launch_resolve_flats(const float* dem, const uint8_t* fdr, int64_t rows, int
 // (cell indices, device).  flat_height has n_heights entries (device).
 int launch_flat_gradient(const int* labels, const uint8_t* fdr, int64_t rows, int64_t cols, const int* seeds,
                          int64_t n_seeds, int towards, int* flat_mask, int* flat_height, int64_t n_heights,
-                         void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  int rc = check_shape(rows, cols);
-  if (rc != OFL_OK) return rc;
+                         void* workspace, cudaStream_t st) {
   const int64_t n = rows * cols;
-  OFL_REQUIRE(n_seeds >= 0 && n_seeds <= n && n_seeds < (1ll << 32) && n_heights >= 0 && n_heights <= n, OFL_ERR_INVALID,
-              "seed / flat_height count out of range");
-  FlatsWork w;
-  rc = carve(workspace, workspace_bytes, rows, cols, &w);
-  if (rc != OFL_OK) return rc;
+  const FlatsWork w = flats_layout(workspace, rows, cols);
   PhaseScope ps(PHASE_FLATS, st);
   OFL_CUDA(cudaMemsetAsync(w.cnt, 0, CNT_SLOTS * sizeof(unsigned), st));
   const unsigned ns = (unsigned)n_seeds;
@@ -1374,7 +1356,7 @@ int launch_flat_gradient(const int* labels, const uint8_t* fdr, int64_t rows, in
   if (n_seeds) OFL_CUDA(cudaMemcpyAsync(w.q1, seeds, (size_t)n_seeds * sizeof(int), cudaMemcpyDeviceToDevice, st));
   int* acc = reinterpret_cast<int*>(w.parent);  // the sweep's own maxima; merged below so untouched labels keep the caller's value
   OFL_CUDA(cudaMemsetAsync(acc, 0, (size_t)n * sizeof(int), st));
-  rc = run_gradient((int)rows, (int)cols, labels, fdr, towards ? SWEEP_TOWARDS_NEGATED : SWEEP_AWAY, false, flat_mask,
+  const int rc = run_gradient((int)rows, (int)cols, labels, fdr, towards ? SWEEP_TOWARDS_NEGATED : SWEEP_AWAY, false, flat_mask,
                     flat_height, acc, w, nullptr, st);
   if (rc != OFL_OK) return rc;
   if (!towards && n_heights) {
@@ -1386,8 +1368,6 @@ int launch_flat_gradient(const int* labels, const uint8_t* fdr, int64_t rows, in
 
 int launch_masked_flow_dirs(const int* flat_mask, const int* labels, uint8_t* fdr, int64_t rows, int64_t cols,
                             cudaStream_t st) {
-  int rc = check_shape(rows, cols);
-  if (rc != OFL_OK) return rc;
   PhaseScope ps(PHASE_FLATS, st);
   const int aligned = (reinterpret_cast<uintptr_t>(fdr) & 3u) == 0;
   if (rows_vector_ok(rows, cols, 4) && aligned && (reinterpret_cast<uintptr_t>(flat_mask) & 15) == 0 &&

@@ -304,15 +304,19 @@ size_t pits_workspace_bytes(int64_t rows, int64_t cols) {
   return pits_layout(nullptr, rows, cols, a);
 }
 
+// One chunk of at most 2^32 cells: cell indices are unsigned 32-bit on the device.
+int pits_shape(int64_t rows, int64_t cols) {
+  OFL_REQUIRE(rows > 0 && cols > 0 && rows < (1ll << 31) && cols < (1ll << 31) && rows * cols <= (1ll << 32), OFL_ERR_INVALID,
+              "pit breaching works on one chunk of at most 2^32 cells (got %lld x %lld)", (long long)rows, (long long)cols);
+  return OFL_OK;
+}
+
 // chunk: device, rows x cols with leading dimension ld, breached in place.  unsolved: device int8, dense.
 // info (host, nullable): {pits found, pits left unsolved, rounds}.  Synchronises the stream (once, at the end).
 int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, double nodata, int8_t* unsolved,
-                       int64_t* info, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  OFL_REQUIRE(rows > 0 && cols > 0 && rows < (1ll << 31) && cols < (1ll << 31) && rows * cols <= (1ll << 32), OFL_ERR_INVALID,
-              "pit breaching works on one chunk of at most 2^32 cells (got %lld x %lld)", (long long)rows, (long long)cols);
+                       int64_t* info, void* workspace, cudaStream_t st) {
   PitsArgs a;
-  const size_t need = pits_layout(workspace, rows, cols, a);
-  OFL_REQUIRE(workspace_bytes >= need, OFL_ERR_WORKSPACE, "pits workspace too small");
+  pits_layout(workspace, rows, cols, a);
   a.chunk = chunk;
   a.rows = (int)rows;
   a.cols = (int)cols;
@@ -324,11 +328,11 @@ int launch_breach_pits(float* chunk, int64_t rows, int64_t cols, int64_t ld, dou
   OFL_CUDA(cudaMemsetAsync(a.cnt, 0, PC_SLOTS * sizeof(unsigned), st));
   const float nd_f = (float)nodata;
   const bool nd_exact = (double)nd_f == nodata;  // false for NaN and for values float32 cannot hold: nothing matches then
+  // the vector path's grid has a row of CTAs per PT / 32 chunk rows, at most 65535 of them
+  const dim3 grid((unsigned)((cols / 4 + 31) / 32), (unsigned)((rows + PT / 32 - 1) / (PT / 32)));
   const bool vec = cols % 4 == 0 && ld % 4 == 0 && (reinterpret_cast<uintptr_t>(chunk) & 15) == 0 &&
-                   (reinterpret_cast<uintptr_t>(unsolved) & 3) == 0 && !getenv("OFL_PITS_SCALAR");
+                   (reinterpret_cast<uintptr_t>(unsolved) & 3) == 0 && grid.y <= 65535u && !getenv("OFL_PITS_SCALAR");
   if (vec) {
-    const dim3 grid((unsigned)((cols / 4 + 31) / 32), (unsigned)((rows + PT / 32 - 1) / (PT / 32)));
-    OFL_REQUIRE(grid.y <= 65535u, OFL_ERR_INVALID, "chunk has too many rows for one launch");
     pits_detect4_kernel<<<grid, PT, 0, st>>>(chunk, (int)rows, (int)cols, ld, nd_f, nd_exact, unsolved, a.waiting, a.list_a,
                                              a.cnt);
   } else {

@@ -16,8 +16,8 @@ OFL_ERR_WORKSPACE = -6
 
 
 def test_failed_call_returns_with_no_copy_in_flight():
-    """A caller workspace one byte too small is refused after the 64 MB upload of the pinned codes has been queued:
-    the call waits for that upload before it returns, so the caller may free or reuse its buffers at once."""
+    """A caller workspace one byte too small is refused before the 64 MB upload of the pinned codes is queued, so
+    nothing the call started is in flight when it returns and the caller may free or reuse its buffers at once."""
     import torch
 
     rows = cols = 8192
@@ -33,6 +33,26 @@ def test_failed_call_returns_with_no_copy_in_flight():
                                       need - 1, _native.OFL_MEM_HOST, stream.cuda_stream)
     idle = stream.query()
     assert rc == OFL_ERR_WORKSPACE
+    assert idle
+
+
+def test_call_failing_after_its_upload_returns_with_no_copy_in_flight():
+    """A cyclic raster fails only once the 64 MB of pinned codes are on the device and the accumulation has run; the
+    call still waits for everything it started before it returns."""
+    import torch
+
+    rows = cols = 8192
+    _native.init(torch.cuda.current_device())
+    lib = _native.lib()
+    codes = torch.full((rows, cols), 8, dtype=torch.uint8).pin_memory()
+    codes[rows // 2, cols // 2], codes[rows // 2, cols // 2 + 1] = 0, 4  # two cells pointing at each other
+    fac = torch.empty((rows, cols), dtype=torch.int64).pin_memory()
+    stream = torch.cuda.Stream()
+    torch.cuda.synchronize()
+    rc = lib.ofl_flow_accumulation_u8(codes.data_ptr(), rows, cols, cols, fac.data_ptr(), cols, None, None, 0,
+                                      _native.OFL_MEM_HOST, stream.cuda_stream)
+    idle = stream.query()
+    assert rc == _native.OFL_ERR_CYCLE
     assert idle
 
 
