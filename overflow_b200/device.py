@@ -2,6 +2,9 @@
 
 PyTorch is only the owner of device memory and streams here; every kernel is in
 liboverflow_b200.  Calls are enqueued on torch's current stream.
+
+Every library call on torch tensors is made from this module, so it alone knows how a tensor meets the C ABI: the
+argument order, unit column stride, and the 16-byte base and row pitch the TMA tensor maps want (16 codes, 4 DEM cells).
 """
 import ctypes
 
@@ -10,9 +13,9 @@ import torch
 from . import _native
 
 
-def _stream(t=None):
+def _stream(t):
     """torch's current stream on the tensor's device (not on whatever device happens to be current)."""
-    return ctypes.c_void_p(torch.cuda.current_stream(t.device if t is not None else None).cuda_stream)
+    return ctypes.c_void_p(torch.cuda.current_stream(t.device).cuda_stream)
 
 
 def _init_for(t: torch.Tensor):
@@ -21,32 +24,64 @@ def _init_for(t: torch.Tensor):
     _native.init(t.device.index if t.device.index is not None else torch.cuda.current_device())
 
 
-def _pitched(rows, cols, dtype, device, align):
-    """rows x cols view of a buffer whose row pitch is a multiple of `align` elements (the library's TMA tensor
-    maps want 16-byte pitches; a dense tensor of odd width does not have one)."""
+# Codes and DEMs get 16-byte row pitches: the stencil and the accumulation read them through TMA tensor maps, which a
+# dense tensor of odd width does not satisfy.  Other rasters are dense.
+_PITCH = {torch.uint8: 16, torch.float32: 4}
+
+
+def pitched(rows, cols, dtype, device):
+    """rows x cols view of a new buffer with the row pitch the library wants for `dtype`."""
+    align = _PITCH.get(dtype, 1)
     return torch.empty((rows, (cols + align - 1) // align * align), dtype=dtype, device=device)[:, :cols]
 
 
-def _check_raster(name, t, dtype, shape, like, pitch_align=1):
-    """Raw pointers of `t` go straight into the C ABI: refuse anything it would mis-read."""
-    if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.dim() != 2 or tuple(t.shape) != tuple(shape):
-        raise ValueError(f"{name} must be a {dtype} tensor of shape {tuple(shape)}")
-    if t.device != like.device:
-        raise ValueError(f"{name} must live on {like.device}, not {t.device}")
-    if t.shape[1] > 1 and t.stride(1) != 1:
-        raise ValueError(f"{name} must have unit column stride")
-    if t.shape[0] > 1 and (t.stride(0) < t.shape[1] or t.stride(0) % pitch_align):
-        raise ValueError(f"{name}: row pitch {t.stride(0)} must be >= {t.shape[1]} and a multiple of {pitch_align}")
+def _input(name, t, dtype, repitch=False):
+    """`t`, a raster the call reads, checked, with the library initialised on its device.  With `repitch`, a raster
+    whose row pitch or base address does not meet the TMA contract comes back as a pitched copy.  A one-column
+    raster may have any column stride: it never addresses memory."""
+    if t.dtype != dtype or t.dim() != 2 or (t.shape[1] > 1 and t.stride(1) != 1):
+        raise ValueError(f"{name} must be a 2-D {dtype} tensor with unit column stride")
+    _init_for(t)
+    if repitch and t.numel() and (t.stride(0) % _PITCH[dtype] or t.data_ptr() % 16):
+        t = pitched(t.shape[0], t.shape[1], dtype, t.device).copy_(t)
     return t
 
 
-def _check_workspace(name, t, need, like):
+def _check_raster(name, t, dtype, shape, device, align=1, dense=False):
+    """Raw pointers of `t` go straight into the C ABI: refuse anything it would mis-read.  The row pitch must be a
+    multiple of `align` elements, or with `dense` equal to the width (calls that take packed rows)."""
+    if not isinstance(t, torch.Tensor) or t.dtype != dtype or t.dim() != 2 or tuple(t.shape) != tuple(shape):
+        raise ValueError(f"{name} must be a {dtype} tensor of shape {tuple(shape)}")
+    if t.device != device:
+        raise ValueError(f"{name} must live on {device}, not {t.device}")
+    if t.shape[1] > 1 and t.stride(1) != 1:
+        raise ValueError(f"{name} must have unit column stride")
+    pitch, width = t.stride(0), t.shape[1]
+    if t.shape[0] > 1 and (pitch < width or pitch % align or (dense and pitch != width)):
+        want = f"equal to {width}" if dense else f">= {width} and a multiple of {align}"
+        raise ValueError(f"{name}: row pitch {pitch} must be {want}")
+    return t
+
+
+def _output(name, t, dtype, shape, device, align=1, dense=False):
+    """The caller's raster `t` for the call to write, checked as _check_raster does; or, when it is None, a new one."""
+    if t is None:
+        return pitched(*shape, dtype, device)
+    return _check_raster(name, t, dtype, shape, device, align, dense)
+
+
+def _workspace(kind, rows, cols, device, t=None):
+    """The caller's workspace `t` for a rows x cols `kind` call, checked to hold ofl_<kind>_workspace_bytes(rows, cols)
+    bytes; or, when it is None, a new one of that size."""
+    need = int(getattr(_native.lib(), f"ofl_{kind}_workspace_bytes")(rows, cols))
+    if t is None:
+        return torch.empty((need,), dtype=torch.uint8, device=device)
     if not isinstance(t, torch.Tensor) or t.dtype != torch.uint8 or t.dim() != 1 or not t.is_contiguous():
-        raise ValueError(f"{name} must be a contiguous 1-D uint8 tensor")
-    if t.device != like.device:
-        raise ValueError(f"{name} must live on {like.device}, not {t.device}")
+        raise ValueError("workspace must be a contiguous 1-D uint8 tensor")
+    if t.device != device:
+        raise ValueError(f"workspace must live on {device}, not {t.device}")
     if t.numel() < need:
-        raise ValueError(f"{name} holds {t.numel()} bytes, {need} needed")
+        raise ValueError(f"workspace holds {t.numel()} bytes, {need} needed")
     return t
 
 
@@ -59,12 +94,7 @@ def synth_dem(rows, cols, *, row0=0, total_rows=None, seed=0, kind=0, relief=100
     (that is what a strip's halo row is at the raster top / bottom).  `out`: write into this tensor.
     """
     total_rows = rows if total_rows is None else total_rows
-    if out is None:
-        dem = _pitched(rows, cols, torch.float32, device, 4)
-    else:
-        if not out.is_cuda:
-            raise ValueError("expected a CUDA tensor (there is no CPU fallback)")
-        dem = _check_raster("out", out, torch.float32, (rows, cols), out)
+    dem = _output("out", out, torch.float32, (rows, cols), out.device if out is not None else device)
     _init_for(dem)
     _native.check(
         _native.lib().ofl_synth_dem_f32(
@@ -82,19 +112,12 @@ def flow_direction(dem: torch.Tensor, nodata_value: float, *, mode="raster", out
     mode "tile":   flow_direction_for_tile semantics (dem carries its ring; ring of the result is 9).
     mode "strip":  dem has 2 more rows than the result: halo rows above and below.
     """
-    if dem.dtype != torch.float32 or dem.dim() != 2 or dem.stride(1) != 1:
-        raise ValueError("dem must be a 2-D float32 tensor with unit column stride")
-    _init_for(dem)
+    dem = _input("dem", dem, torch.float32, repitch=True)
     m = {"tile": _native.OFL_DIR_MODE_TILE, "raster": _native.OFL_DIR_MODE_RASTER, "strip": _native.OFL_DIR_MODE_STRIP}[mode]
     rows, cols = dem.shape
     if m == _native.OFL_DIR_MODE_STRIP:
         rows -= 2
-    if dem.shape[0] and dem.shape[1] and (dem.stride(0) % 4 or dem.data_ptr() % 16):
-        dem = _pitched(dem.shape[0], cols, torch.float32, dem.device, 4).copy_(dem)  # dense odd widths: re-pitch (TMA)
-    if out is None:
-        out = _pitched(rows, cols, torch.uint8, dem.device, 16)  # flow_accumulation wants 16-byte pitches
-    else:
-        _check_raster("out", out, torch.uint8, (rows, cols), dem, 4)
+    out = _output("out", out, torch.uint8, (rows, cols), dem.device, 4)
     _native.check(
         _native.lib().ofl_flow_direction_f32(
             dem.data_ptr(), rows, cols, dem.stride(0), float(nodata_value), out.data_ptr(), out.stride(0), m,
@@ -105,8 +128,7 @@ def flow_direction(dem: torch.Tensor, nodata_value: float, *, mode="raster", out
 
 
 def accumulation_workspace(rows, cols, device="cuda") -> torch.Tensor:
-    n = int(_native.lib().ofl_accumulation_workspace_bytes(rows, cols))
-    return torch.empty((n,), dtype=torch.uint8, device=device)
+    return _workspace("accumulation", rows, cols, device)
 
 
 def flow_accumulation(fdr: torch.Tensor, *, out=None, workspace=None, with_links=False):
@@ -115,21 +137,10 @@ def flow_accumulation(fdr: torch.Tensor, *, out=None, workspace=None, with_links
     Returns fac, or (fac, perim_links[n,2]) in perimeter_indices order when with_links.
     Synchronises the stream (the perimeter-graph solve reports convergence to the host).
     """
-    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or fdr.stride(1) != 1:
-        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
-    _init_for(fdr)
+    fdr = _input("fdr", fdr, torch.uint8, repitch=True)
     rows, cols = fdr.shape
-    if rows and cols and (fdr.stride(0) % 16 or fdr.data_ptr() % 16):
-        fdr = _pitched(rows, cols, torch.uint8, fdr.device, 16).copy_(fdr)  # dense odd widths: re-pitch (TMA)
-    if out is None:
-        out = torch.empty((rows, cols), dtype=torch.int64, device=fdr.device)
-    else:
-        _check_raster("out", out, torch.int64, (rows, cols), fdr)
-    need = int(_native.lib().ofl_accumulation_workspace_bytes(rows, cols))
-    if workspace is None:
-        workspace = accumulation_workspace(rows, cols, fdr.device)
-    else:
-        _check_workspace("workspace", workspace, need, fdr)
+    out = _output("out", out, torch.int64, (rows, cols), fdr.device)
+    workspace = _workspace("accumulation", rows, cols, fdr.device, workspace)
     links = None
     if with_links:
         n = int(_native.lib().ofl_perimeter_count(rows, cols))
@@ -152,28 +163,19 @@ def flow_routing(dem: torch.Tensor, nodata_value: float, *, out_fdr=None, out_fa
     (fix_flats.py), accumulation -- with the codes resident on the device throughout.  The DEM must be free of
     pits then (the reference breaches them first): its d8_masked_flow_dirs points a pit at a neighbour, which can
     close a cycle, and a cyclic raster makes the accumulation raise OFL_ERR_CYCLE."""
-    if dem.dtype != torch.float32 or dem.dim() != 2 or dem.stride(1) != 1:
-        raise ValueError("dem must be a 2-D float32 tensor with unit column stride")
-    _init_for(dem)
-    rows, cols = dem.shape
     if resolve_flats:
+        _input("dem", dem, torch.float32)
         if not dem.is_contiguous():
             raise ValueError("resolve_flats needs a contiguous DEM")
-        if cols % 16:
+        if dem.shape[1] % 16:
             raise ValueError("resolve_flats needs a column count that is a multiple of 16 (dense codes, TMA pitch)")
         fdr = flow_direction(dem, nodata_value, out=out_fdr)
         fix_flats(dem, fdr)
         return fdr, flow_accumulation(fdr, out=out_fac)
-    if rows and cols and (dem.stride(0) % 4 or dem.data_ptr() % 16):
-        dem = _pitched(rows, cols, torch.float32, dem.device, 4).copy_(dem)  # dense odd widths: re-pitch (TMA)
-    if out_fdr is None:
-        out_fdr = _pitched(rows, cols, torch.uint8, dem.device, 16)
-    else:
-        _check_raster("out_fdr", out_fdr, torch.uint8, (rows, cols), dem, 16)
-    if out_fac is None:
-        out_fac = torch.empty((rows, cols), dtype=torch.int64, device=dem.device)
-    else:
-        _check_raster("out_fac", out_fac, torch.int64, (rows, cols), dem)
+    dem = _input("dem", dem, torch.float32, repitch=True)
+    rows, cols = dem.shape
+    out_fdr = _output("out_fdr", out_fdr, torch.uint8, (rows, cols), dem.device, 16)
+    out_fac = _output("out_fac", out_fac, torch.int64, (rows, cols), dem.device)
     _native.check(
         _native.lib().ofl_flow_routing_f32(
             dem.data_ptr(), rows, cols, dem.stride(0), float(nodata_value), out_fdr.data_ptr(), out_fdr.stride(0),
@@ -185,11 +187,9 @@ def flow_routing(dem: torch.Tensor, nodata_value: float, *, out_fdr=None, out_fa
 
 def check_accumulation(fdr: torch.Tensor, fac: torch.Tensor) -> int:
     """Number of cells violating the accumulation recurrence (0 proves fac exact on an acyclic raster)."""
-    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or (fdr.shape[1] > 1 and fdr.stride(1) != 1):
-        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
-    _init_for(fdr)
+    fdr = _input("fdr", fdr, torch.uint8)
     rows, cols = fdr.shape
-    _check_raster("fac", fac, torch.int64, (rows, cols), fdr)
+    _check_raster("fac", fac, torch.int64, (rows, cols), fdr.device)
     n_bad = ctypes.c_int64(0)
     _native.check(
         _native.lib().ofl_check_accumulation_u8(
@@ -201,8 +201,7 @@ def check_accumulation(fdr: torch.Tensor, fac: torch.Tensor) -> int:
 
 
 def basins_workspace(rows, cols, device="cuda") -> torch.Tensor:
-    n = int(_native.lib().ofl_basins_workspace_bytes(rows, cols))
-    return torch.empty((n,), dtype=torch.uint8, device=device)
+    return _workspace("basins", rows, cols, device)
 
 
 def _pour_indices(pour_points, fdr):
@@ -230,22 +229,11 @@ def label_basins(fdr: torch.Tensor, *, pour_points=None, out=None, workspace=Non
     """int64 basin labels of a uint8 CUDA flow-direction raster (overflow_b200.basins has the rules): the label of
     the outlet, or with pour points ((k, 2) of (row, col)) of the first pour point, that each cell's path reaches.
     Synchronises the stream (the call reports cycles and pour points outside the raster)."""
-    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or fdr.stride(1) != 1:
-        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
-    _init_for(fdr)
+    fdr = _input("fdr", fdr, torch.uint8, repitch=True)
     rows, cols = fdr.shape
     idx = _pour_indices(pour_points, fdr)
-    if rows and cols and (fdr.stride(0) % 16 or fdr.data_ptr() % 16):
-        fdr = _pitched(rows, cols, torch.uint8, fdr.device, 16).copy_(fdr)  # dense odd widths: re-pitch
-    if out is None:
-        out = torch.empty((rows, cols), dtype=torch.int64, device=fdr.device)
-    else:
-        _check_raster("out", out, torch.int64, (rows, cols), fdr)
-    need = int(_native.lib().ofl_basins_workspace_bytes(rows, cols))
-    if workspace is None:
-        workspace = basins_workspace(rows, cols, fdr.device)
-    else:
-        _check_workspace("workspace", workspace, need, fdr)
+    out = _output("out", out, torch.int64, (rows, cols), fdr.device)
+    workspace = _workspace("basins", rows, cols, fdr.device, workspace)
     _native.check(
         _native.lib().ofl_label_basins_u8(
             fdr.data_ptr(), rows, cols, fdr.stride(0), idx.data_ptr() if idx is not None else None,
@@ -258,11 +246,9 @@ def label_basins(fdr: torch.Tensor, *, pour_points=None, out=None, workspace=Non
 
 def check_basins(fdr: torch.Tensor, labels: torch.Tensor, pour_points=None) -> int:
     """Number of cells breaking the basin labelling rule (0 proves the labels exact on an acyclic raster)."""
-    if fdr.dtype != torch.uint8 or fdr.dim() != 2 or (fdr.shape[1] > 1 and fdr.stride(1) != 1):
-        raise ValueError("fdr must be a 2-D uint8 tensor with unit column stride")
-    _init_for(fdr)
+    fdr = _input("fdr", fdr, torch.uint8)
     rows, cols = fdr.shape
-    _check_raster("labels", labels, torch.int64, (rows, cols), fdr)
+    _check_raster("labels", labels, torch.int64, (rows, cols), fdr.device)
     idx = _pour_indices(pour_points, fdr)
     n_bad = ctypes.c_int64(0)
     _native.check(
@@ -276,88 +262,47 @@ def check_basins(fdr: torch.Tensor, labels: torch.Tensor, pour_points=None) -> i
 
 
 def flats_workspace(rows, cols, device="cuda") -> torch.Tensor:
-    n = int(_native.lib().ofl_flats_workspace_bytes(rows, cols))
-    return torch.empty((max(n, 256),), dtype=torch.uint8, device=device)
+    return _workspace("flats", rows, cols, device)
 
 
-def _flats_args(dem, fdr):
-    if dem.dtype != torch.float32 or dem.dim() != 2 or not dem.is_contiguous():
-        raise ValueError("dem must be a contiguous 2-D float32 tensor")
-    if fdr.dtype != torch.uint8 or fdr.shape != dem.shape or not fdr.is_contiguous():
-        raise ValueError("fdr must be a contiguous uint8 tensor of the DEM's shape")
-    _init_for(dem)
+def _flats_call(fix, dem, fdr, flat_mask, labels, workspace):
+    """ofl_fix_flats_f32 when `fix`, else ofl_resolve_flats_f32: (flat_mask, labels, info).  Both take packed rows:
+    every raster is dense."""
+    _input("dem", dem, torch.float32)
+    rows, cols = dem.shape
+    _check_raster("dem", dem, torch.float32, (rows, cols), dem.device, dense=True)
+    _check_raster("fdr", fdr, torch.uint8, (rows, cols), dem.device, dense=True)
+    flat_mask = _output("flat_mask", flat_mask, torch.int32, (rows, cols), dem.device, dense=True)
+    labels = _output("labels", labels, torch.int32, (rows, cols), dem.device, dense=True)
+    workspace = _workspace("flats", rows, cols, dem.device, workspace)
+    info = (ctypes.c_int64 * 5)()
+    fn = _native.lib().ofl_fix_flats_f32 if fix else _native.lib().ofl_resolve_flats_f32
+    _native.check(
+        fn(dem.data_ptr(), fdr.data_ptr(), rows, cols, flat_mask.data_ptr(), labels.data_ptr(), info,
+           workspace.data_ptr(), workspace.numel(), _native.OFL_MEM_DEVICE, _stream(dem))
+    )
+    return flat_mask, labels, [int(v) for v in info]
 
 
 def resolve_flats(dem: torch.Tensor, fdr: torch.Tensor, *, workspace=None):
     """(flat_mask int32, labels int32, info) of a float32 CUDA DEM and its uint8 codes (ofl_resolve_flats_f32).
     info = [low edges, high edges, labels, away levels, towards levels].  Synchronises the stream."""
-    _flats_args(dem, fdr)
-    rows, cols = dem.shape
-    flat_mask = torch.empty((rows, cols), dtype=torch.int32, device=dem.device)
-    labels = torch.empty((rows, cols), dtype=torch.int32, device=dem.device)
-    if workspace is None:
-        workspace = flats_workspace(rows, cols, dem.device)
-    else:
-        _check_workspace("workspace", workspace, int(_native.lib().ofl_flats_workspace_bytes(rows, cols)), dem)
-    info = (ctypes.c_int64 * 5)()
-    _native.check(
-        _native.lib().ofl_resolve_flats_f32(
-            dem.data_ptr(), fdr.data_ptr(), rows, cols, flat_mask.data_ptr(), labels.data_ptr(), info,
-            workspace.data_ptr(), workspace.numel(), _native.OFL_MEM_DEVICE, _stream(dem),
-        )
-    )
-    return flat_mask, labels, [int(v) for v in info]
+    return _flats_call(False, dem, fdr, None, None, workspace)
 
 
 def fix_flats(dem: torch.Tensor, fdr: torch.Tensor, *, workspace=None, flat_mask=None, labels=None):
     """Rewrite the code-8 cells of `fdr` in place (resolve_flats + d8_masked_flow_dirs, ofl_fix_flats_f32).
     Returns (fdr, info).  Synchronises the stream."""
-    _flats_args(dem, fdr)
-    rows, cols = dem.shape
-    if flat_mask is None:
-        flat_mask = torch.empty((rows, cols), dtype=torch.int32, device=dem.device)
-    elif not flat_mask.is_contiguous():
-        raise ValueError("flat_mask must be contiguous")
-    else:
-        _check_raster("flat_mask", flat_mask, torch.int32, (rows, cols), dem)
-    if labels is None:
-        labels = torch.empty((rows, cols), dtype=torch.int32, device=dem.device)
-    elif not labels.is_contiguous():
-        raise ValueError("labels must be contiguous")
-    else:
-        _check_raster("labels", labels, torch.int32, (rows, cols), dem)
-    if workspace is None:
-        workspace = flats_workspace(rows, cols, dem.device)
-    else:
-        _check_workspace("workspace", workspace, int(_native.lib().ofl_flats_workspace_bytes(rows, cols)), dem)
-    info = (ctypes.c_int64 * 5)()
-    _native.check(
-        _native.lib().ofl_fix_flats_f32(
-            dem.data_ptr(), fdr.data_ptr(), rows, cols, flat_mask.data_ptr(), labels.data_ptr(), info,
-            workspace.data_ptr(), workspace.numel(), _native.OFL_MEM_DEVICE, _stream(dem),
-        )
-    )
-    return fdr, [int(v) for v in info]
+    return fdr, _flats_call(True, dem, fdr, flat_mask, labels, workspace)[2]
 
 
 def breach_single_cell_pits(chunk: torch.Tensor, nodata_value: float, *, unsolved=None, workspace=None):
     """Breach the single-cell pits of a float32 CUDA chunk in place (ofl_breach_single_cell_pits_f32).
     Returns (unsolved int8 tensor, [pits found, pits left unsolved, rounds]).  Synchronises the stream."""
-    if chunk.dtype != torch.float32 or chunk.dim() != 2 or chunk.stride(1) != 1:
-        raise ValueError("chunk must be a 2-D float32 tensor with unit column stride")
-    _init_for(chunk)
+    chunk = _input("chunk", chunk, torch.float32)
     rows, cols = chunk.shape
-    nbytes = int(_native.lib().ofl_pits_workspace_bytes(rows, cols))
-    if unsolved is None:
-        unsolved = torch.empty((rows, cols), dtype=torch.int8, device=chunk.device)
-    elif not unsolved.is_contiguous():
-        raise ValueError("unsolved must be contiguous")
-    else:
-        _check_raster("unsolved", unsolved, torch.int8, (rows, cols), chunk)
-    if workspace is None:
-        workspace = torch.empty((max(nbytes, 256),), dtype=torch.uint8, device=chunk.device)
-    else:
-        _check_workspace("workspace", workspace, nbytes, chunk)
+    unsolved = _output("unsolved", unsolved, torch.int8, (rows, cols), chunk.device, dense=True)
+    workspace = _workspace("pits", rows, cols, chunk.device, workspace)
     info = (ctypes.c_int64 * 3)()
     _native.check(
         _native.lib().ofl_breach_single_cell_pits_f32(
@@ -366,3 +311,66 @@ def breach_single_cell_pits(chunk: torch.Tensor, nodata_value: float, *, unsolve
         )
     )
     return unsolved, [int(v) for v in info]
+
+
+# ---------------------------------------------------------------- row strips (strips.py)
+# These calls run several times per multi-GPU step and only enqueue work, so they make no Python checks: the library
+# checks their sizes, pointers, pitches and workspaces before it touches the device.  `fdr_halo` is a strip's codes
+# with one halo row above and below; `record` is its boundary record block (strips.record_bytes).
+def strip_workspace(rows, cols, device="cuda") -> torch.Tensor:
+    return _workspace("strip", rows, cols, device)
+
+
+def strip_boundary_workspace(n_strips, cols, device="cuda") -> torch.Tensor:
+    return _workspace("strip_boundary", n_strips, cols, device)
+
+
+def strip_accum_local(fdr_halo, has_above, has_below, fac, workspace, record):
+    """Strip-local counts into `fac` and the strip's boundary record into `record` (ofl_strip_accum_local)."""
+    _init_for(fac)
+    rows, cols = fac.shape
+    _native.check(_native.lib().ofl_strip_accum_local(
+        fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), int(has_above), int(has_below), fac.data_ptr(),
+        fac.stride(0), workspace.data_ptr(), workspace.numel(), record.data_ptr(), _stream(fac)))
+
+
+def strip_boundary_solve(records_all, cols, J_all, workspace):
+    """Inflow J_all [n_strips, 2, cols] of every strip's boundary cells from the gathered records
+    [n_strips, record bytes] (ofl_strip_boundary_solve)."""
+    _init_for(J_all)
+    _native.check(_native.lib().ofl_strip_boundary_solve(
+        records_all.data_ptr(), records_all.shape[0], cols, J_all.data_ptr(), workspace.data_ptr(), workspace.numel(),
+        _stream(J_all)))
+
+
+def strip_accum_final(fdr_halo, has_above, has_below, J_mine, workspace, fac):
+    """The strip's final counts into `fac`: its inflow J_mine [2, cols] pushed down the strip (ofl_strip_accum_final)."""
+    _init_for(fac)
+    rows, cols = fac.shape
+    _native.check(_native.lib().ofl_strip_accum_final(
+        fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), int(has_above), int(has_below), J_mine.data_ptr(),
+        workspace.data_ptr(), workspace.numel(), fac.data_ptr(), fac.stride(0), _stream(fac)))
+
+
+def strip_collect_flags(workspace, rows, cols, boundary_workspace, n_strips, out):
+    """Error flags of the strip calls since the last strip_accum_local (and of the boundary solve) into the int32[4]
+    tensor `out`; either workspace may be None.  Stream-ordered, no synchronisation (ofl_strip_collect_flags)."""
+    _init_for(out)
+    _native.check(_native.lib().ofl_strip_collect_flags(
+        workspace.data_ptr() if workspace is not None else None, rows, cols,
+        boundary_workspace.data_ptr() if boundary_workspace is not None else None, n_strips, out.data_ptr(),
+        _stream(out)))
+
+
+def strip_check_accumulation(fdr_halo, fac, fac_above, fac_below) -> int:
+    """Cells of the strip violating the accumulation recurrence, its first and last rows checked against the
+    neighbouring strips' boundary counts fac_above / fac_below (None at the raster's edge); synchronises the stream
+    (ofl_strip_check_accumulation_u8)."""
+    _init_for(fac)
+    rows, cols = fac.shape
+    n_bad = ctypes.c_int64(0)
+    _native.check(_native.lib().ofl_strip_check_accumulation_u8(
+        fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), fac.data_ptr(), fac.stride(0),
+        fac_above.data_ptr() if fac_above is not None else None,
+        fac_below.data_ptr() if fac_below is not None else None, ctypes.byref(n_bad), _stream(fac)))
+    return int(n_bad.value)

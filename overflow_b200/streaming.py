@@ -20,7 +20,6 @@ code before it can finish a single count); rasters beyond device memory take
 25 ms next to tens of seconds of I/O -- splitting it per band would buy nothing).
 PyTorch owns device memory, pinned memory and streams here; every kernel is in liboverflow_b200.
 """
-import ctypes
 import queue
 import threading
 import time
@@ -30,10 +29,6 @@ import numpy as np
 from . import _native
 from .constants import FLOW_ACCUMULATION_NODATA, FLOW_DIRECTION_NODATA
 from .flow_accumulation import as_codes
-
-
-def _round_up(v, a):
-    return (v + a - 1) // a * a
 
 
 def _get(q, check):
@@ -181,10 +176,10 @@ def _stream(input_path, dem_in, flow_direction_path, flow_accumulation_path, ban
             s_up, s_down = torch.cuda.Stream(device), torch.cuda.Stream(device)
             if dem_in:
                 # the DEM carries one nodata row above and below (what util/raster.py:67 pads)
-                dem_halo = torch.empty((rows + 2, _round_up(cols, 4)), dtype=torch.float32, device=device)[:, :cols]
+                dem_halo = dev.pitched(rows + 2, cols, torch.float32, device)
                 dem_halo[0].fill_(float(np.float32(nodata)))
                 dem_halo[-1].fill_(float(np.float32(nodata)))
-            fdr = torch.empty((rows, _round_up(cols, 16)), dtype=torch.uint8, device=device)[:, :cols]
+            fdr = dev.pitched(rows, cols, torch.uint8, device)
             s_up.wait_stream(s_comp)  # the new blocks may still be in use by work queued on s_comp
             in_ring = _Ring(torch, ring, (band_rows, cols), up_dtype)
             code_ring = _Ring(torch, ring, (band_rows + 1, cols), torch.uint8) if fdr_band is not None else None
@@ -221,7 +216,6 @@ def _stream(input_path, dem_in, flow_direction_path, flow_accumulation_path, ban
             for b in range(len(bands)):
                 reader.submit(read_job(b))
 
-            lib = _native.lib()
             done = 0  # output rows whose codes exist
             for _ in range(len(bands)):
                 b, slot = _get(filled, check)
@@ -242,10 +236,8 @@ def _stream(input_path, dem_in, flow_direction_path, flow_accumulation_path, ban
                     s_comp.wait_event(e1)
                     d0, d1 = ev_t(), ev_t()
                     d0.record(s_comp)
-                    _native.check(lib.ofl_flow_direction_f32(
-                        dem_halo[done].data_ptr(), end - done, cols, dem_halo.stride(0), float(nodata),
-                        fdr[done:end].data_ptr(), fdr.stride(0), _native.OFL_DIR_MODE_STRIP, _native.OFL_MEM_DEVICE,
-                        ctypes.c_void_p(s_comp.cuda_stream)))
+                    with torch.cuda.stream(s_comp):  # the slices are pitched already: no copy
+                        dev.flow_direction(dem_halo[done : end + 2], nodata, mode="strip", out=fdr[done:end])
                     d1.record(s_comp)
                     dir_events.append((d0, d1))
                     if fdr_band is not None:

@@ -20,12 +20,10 @@ The compute lives behind a small engine interface so the host-side exchange logi
 CPU (gloo) with a stand-in engine; the shipped engine (CudaStripEngine) is the C ABI and has no
 CPU fallback.
 """
-import ctypes
-
 import numpy as np
 import torch
 
-from . import _native
+from . import _native, device as dev
 from .flow_accumulation import as_codes
 
 TILE = 64  # strips must start on multiples of the accumulation tile side
@@ -70,70 +68,44 @@ def record_views(rec, cols):
 
 
 class CudaStripEngine:
-    """The product engine: every method is a liboverflow_b200 call on torch CUDA tensors.  The strip calls only
-    enqueue work on torch's current stream; `flags` hands out their error flags."""
+    """The product engine: every method is a liboverflow_b200 call on torch CUDA tensors (device.py).  The strip calls
+    only enqueue work on torch's current stream; `flags` hands out their error flags."""
 
     def __init__(self, device):
         self.device = torch.device(device)
         if self.device.type != "cuda":
             raise ValueError("CudaStripEngine needs a CUDA device (there is no CPU fallback)")
-        _native.init(self.device.index if self.device.index is not None else torch.cuda.current_device())
-
-    def _stream(self):
-        return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def empty(self, shape, dtype):
         return torch.empty(shape, dtype=dtype, device=self.device)
 
     def strip_workspace(self, rows, cols):
-        return self.empty((int(_native.lib().ofl_strip_workspace_bytes(rows, cols)),), torch.uint8)
+        return dev.strip_workspace(rows, cols, self.device)
 
     def boundary_workspace(self, n_strips, cols):
-        return self.empty((int(_native.lib().ofl_strip_boundary_workspace_bytes(n_strips, cols)),), torch.uint8)
+        return dev.strip_boundary_workspace(n_strips, cols, self.device)
 
     def synth_dem(self, out, row0, total_rows, seed, kind, holes_permille, nodata, relief=1000.0):
-        rows, cols = out.shape
-        _native.check(_native.lib().ofl_synth_dem_f32(out.data_ptr(), rows, cols, out.stride(0), row0, total_rows, seed,
-                                                      kind, relief, holes_permille, nodata, self._stream()))
+        dev.synth_dem(*out.shape, row0=row0, total_rows=total_rows, seed=seed, kind=kind, relief=relief,
+                      holes_permille=holes_permille, nodata=nodata, out=out)
 
     def direction(self, dem_halo, nodata, fdr_out):
-        rows, cols = fdr_out.shape
-        _native.check(_native.lib().ofl_flow_direction_f32(
-            dem_halo.data_ptr(), rows, cols, dem_halo.stride(0), float(nodata), fdr_out.data_ptr(), fdr_out.stride(0),
-            _native.OFL_DIR_MODE_STRIP, _native.OFL_MEM_DEVICE, self._stream()))
+        dev.flow_direction(dem_halo, nodata, mode="strip", out=fdr_out)
 
     def accum_local(self, fdr_halo, has_above, has_below, fac, ws, rec):
-        rows, cols = fac.shape
-        _native.check(_native.lib().ofl_strip_accum_local(
-            fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), int(has_above), int(has_below), fac.data_ptr(),
-            fac.stride(0), ws.data_ptr(), ws.numel(), rec.data_ptr(), self._stream()))
+        dev.strip_accum_local(fdr_halo, has_above, has_below, fac, ws, rec)
 
     def boundary_solve(self, rec_all, cols, J_all, ws):
-        _native.check(_native.lib().ofl_strip_boundary_solve(
-            rec_all.data_ptr(), rec_all.shape[0], cols, J_all.data_ptr(), ws.data_ptr(), ws.numel(), self._stream()))
+        dev.strip_boundary_solve(rec_all, cols, J_all, ws)
 
     def accum_final(self, fdr_halo, has_above, has_below, J_mine, ws, fac):
-        rows, cols = fac.shape
-        _native.check(_native.lib().ofl_strip_accum_final(
-            fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), int(has_above), int(has_below), J_mine.data_ptr(),
-            ws.data_ptr(), ws.numel(), fac.data_ptr(), fac.stride(0), self._stream()))
+        dev.strip_accum_final(fdr_halo, has_above, has_below, J_mine, ws, fac)
 
     def flags(self, ws, rows, cols, bws, n_strips, out):
-        """Error flags of the strip calls since the last accum_local (and of the boundary solve) into the int32[4]
-        device tensor `out`; stream-ordered, no synchronisation."""
-        _native.check(_native.lib().ofl_strip_collect_flags(
-            ws.data_ptr() if ws is not None else None, rows, cols, bws.data_ptr() if bws is not None else None,
-            n_strips, out.data_ptr(), self._stream()))
+        dev.strip_collect_flags(ws, rows, cols, bws, n_strips, out)
 
     def check(self, fdr_halo, fac, fac_above, fac_below):
-        """Cells of the strip violating the accumulation recurrence (ofl_strip_check_accumulation_u8)."""
-        rows, cols = fac.shape
-        n_bad = ctypes.c_int64(0)
-        _native.check(_native.lib().ofl_strip_check_accumulation_u8(
-            fdr_halo.data_ptr(), rows, cols, fdr_halo.stride(0), fac.data_ptr(), fac.stride(0),
-            fac_above.data_ptr() if fac_above is not None else None,
-            fac_below.data_ptr() if fac_below is not None else None, ctypes.byref(n_bad), self._stream()))
-        return int(n_bad.value)
+        return dev.strip_check_accumulation(fdr_halo, fac, fac_above, fac_below)
 
 
 def raise_for_flags(flags):

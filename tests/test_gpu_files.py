@@ -107,7 +107,10 @@ def test_flow_routing_files_equal_the_two_step_outputs(tmp_path):
 # ---- the band pipeline of streaming.py (SURVEY 8f rank 1): the oracle's codes and counts, and those of the whole-raster
 # host call (what the file drivers computed before Float32 DEMs streamed), for any band height
 @pytest.mark.parametrize("band_rows", [1, 7, 64, 100, 5000])
-def test_streamed_routing_equals_oracle_and_whole_raster(tmp_path, band_rows):
+def test_streamed_routing_equals_oracle_and_whole_raster(tmp_path, band_rows, monkeypatch):
+    import torch
+
+    from overflow_b200 import device as dev
     from overflow_b200.flow_routing import flow_routing_for_raster
     from overflow_b200.streaming import stream_routing
 
@@ -117,8 +120,17 @@ def test_streamed_routing_equals_oracle_and_whole_raster(tmp_path, band_rows):
     ds.GetRasterBand(1).WriteArray(dem)
     ds.GetRasterBand(1).SetNoDataValue(synth.NODATA)
     ds.FlushCache()
+    allocs, pitched = [], dev.pitched
+
+    def spy(rows, cols, dtype, device):  # sees every pitched buffer, the re-pitch copies of device.py's calls included
+        allocs.append((rows, cols, dtype))
+        return pitched(rows, cols, dtype, device)
+
+    monkeypatch.setattr(dev, "pitched", spy)
     rep = stream_routing(src, str(tmp_path / "fdr_s.tif"), str(tmp_path / "fac_s.tif"), band_rows=band_rows)
     assert rep["rows"] == 333 and rep["bands"] == -(-333 // min(band_rows, 333)) and rep["wall_s"] > 0
+    # the device DEM with its halo rows and the codes; no band of the stencil was copied to meet the TMA contract
+    assert allocs == [(335, 257, torch.float32), (333, 257, torch.uint8)]
     whole = flow_routing_for_raster(dem, synth.NODATA)
     want_fdr = oracle.flow_direction_for_tile(synth.pad_nodata(dem), synth.NODATA)[1:-1, 1:-1]
     want_fac = oracle.flow_accumulation(np.ascontiguousarray(want_fdr))
